@@ -3,6 +3,7 @@
 fraction of the HBM roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload tiles256|stamps32|frame|ngc|sat]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 4 — a synthetic 2048x2048 crowded field split into 64
 256x256 subdivisions, each solved for the 5 beta initialisations of the reference's application script
@@ -62,7 +63,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-clocks", action="store_true", help="experiments: do not sample clocks during the timed region")
     ap.add_argument("--cpu-sample", type=int, default=8)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def make_workload(args, rank):
@@ -86,7 +93,10 @@ def make_workload(args, rank):
         return w, kw, name, True
     if args.workload in ("ngc", "sat"):
         # the two SGP-dec simulations the reference bundles (simulated_test/data/*.mat), read from the committed fixtures
-        fx = np.load(os.path.join(ROOT, "tests", "golden", "fixtures.npz"))
+        spec = importlib.util.spec_from_file_location("_bsgp_golden_store", os.path.join(ROOT, "tests", "golden", "golden_store.py"))
+        store = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(store)
+        fx = store.load("fixtures")
         gn, psf, bg = fx[args.workload + "/gn"].astype(np.float64), fx[args.workload + "/psf"].astype(np.float64), float(fx[args.workload + "/bkg"])
         if args.workload == "ngc":
             w = dict(gn=gn[None], bkg=np.array([bg]), psf=psf, flux=None, beta0=np.array([1.0]), divergence="kl")
@@ -286,6 +296,32 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(res, out_dir):
+    """--dump-outputs: the arrays the last timed step returned (solve_batch_sharded), one float32 / float64 .npy per field, so
+    that two builds can be compared output for output on the same seeded inputs.  Integer fields are written as float64
+    (exact).  "times" (device clock stamps of every iteration) is left out: it differs from run to run by nature.  The
+    restored images "x" get what the 64 MB budget leaves; when they do not fit, a fixed seeded sample of whole images is
+    written (of image rows when not even one image fits), and "x_index" holds the sampled batch indices (row indices
+    b * ny + y for rows)."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.cpu().numpy() for k, v in res.items() if k != "times"}
+    out = {k: (v if v.dtype in (np.float32, np.float64) else v.astype(np.float64)) for k, v in host.items() if k != "x"}
+    x = host["x"]
+    room = DUMP_LIMIT_BYTES - 4096 - sum(v.nbytes for v in out.values())        # 4096: the .npy headers
+    units = x if x[0].nbytes + 8 <= room else x.reshape(-1, x.shape[-1])
+    keep = min(len(units), room // (units[0].nbytes + 8))
+    if keep < len(units):
+        idx = np.sort(np.random.default_rng(0).choice(len(units), keep, replace=False))
+        out["x_index"] = idx.astype(np.float64)
+        units = units[idx]
+    out["x"] = units
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def hbm_peak():
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(peaks_path):
@@ -293,10 +329,11 @@ def hbm_peak():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
-def measure(args, ctx, workload, steps, warmup, with_cpu, sharded=True, with_clocks=True):
+def measure(args, ctx, workload, steps, warmup, with_cpu, sharded=True, with_clocks=True, dump_dir=None):
     """One workload through the product: `value` with inputs resident in HBM (sharded over the ranks of ctx, gather inside
     the timed region), `e2e` from page-locked host memory, roofline of the solve kernel from CUDA events inside the timed
-    region.  Returns the JSON-able dict (rank 0) or None."""
+    region.  dump_dir: rank 0 writes the outputs of the last timed step there (dump_outputs).  Returns the JSON-able dict
+    (rank 0) or None."""
     import torch
     import torch.distributed as dist
     bs, dev, rank, local_rank, world = ctx["bs"], ctx["dev"], ctx["rank"], ctx["local_rank"], ctx["world"]
@@ -435,6 +472,8 @@ def measure(args, ctx, workload, steps, warmup, with_cpu, sharded=True, with_clo
     ms, ms_e2e = float(ms.item()), float(ms_e2e.item())
     if rank != 0:
         return None
+    if dump_dir:
+        dump_outputs(res, dump_dir)
     images = B * steps
     value = images / (ms * 1e-3)
     peak, peak_src = hbm_peak()
@@ -552,7 +591,8 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     ctx = dict(bs=bs, dev=dev, rank=rank, local_rank=local_rank, world=world)
-    line = measure(args, ctx, args.workload, args.steps, args.warmup, with_cpu=not args.no_cpu_baseline, with_clocks=not args.no_clocks)
+    line = measure(args, ctx, args.workload, args.steps, args.warmup, with_cpu=not args.no_cpu_baseline, with_clocks=not args.no_clocks,
+                   dump_dir=args.dump_outputs)
     if args.workload == "tiles256" and not args.no_extra:
         extra = {}
         if world == 1:

@@ -17,12 +17,14 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def fixtures():
-    return np.load(os.path.join(HERE, "golden", "fixtures.npz"))
+    import golden_store
+    return golden_store.load("fixtures")
 
 
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(HERE, "golden", "golden_ref.npz"))
+    import golden_store
+    return golden_store.load("golden_ref")
 
 
 def case_inputs(name, fixtures, golden):

@@ -1,12 +1,12 @@
 """Generate the committed golden vectors by running the UNMODIFIED reference in this container.
 
-    cd /root/repo && python tests/golden/make_golden.py
+    python tests/golden/make_golden.py        (from the repository root)
 
-Writes tests/golden/fixtures.npz (inputs) and tests/golden/golden_ref.npz (reference outputs plus the
-oracle's controller trace).  For every case the oracle (oracle/sgp_oracle.py) is run on the same
-inputs and must agree BIT FOR BIT with the reference (image, iteration count, objective trace) —
-that is the oracle's pin; the script aborts otherwise.  /root/reference does not exist on the GPU
-box, so tests only ever read the two .npz files.
+Writes the golden archives "fixtures" (inputs) and "golden_ref" (reference outputs plus the oracle's
+controller trace) as tests/golden/<name>.<part>.npz (golden_store.py).  For every case the oracle
+(oracle/sgp_oracle.py) is run on the same inputs and must agree BIT FOR BIT with the reference (image,
+iteration count, objective trace) — that is the oracle's pin; the script aborts otherwise.  The tests
+never need the reference: they only read the committed archives.
 """
 import contextlib
 import io
@@ -24,6 +24,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.join(ROOT, "beta-sgp_b200"))
 
+import golden_store  # noqa: E402
 import reference_loader  # noqa: E402
 from cases import CASES, N_CUTOUTS31, N_STAMPS, N_TILES  # noqa: E402
 import synth  # noqa: E402
@@ -58,6 +59,8 @@ def build_inputs():
 
 
 def main():
+    from threadpoolctl import threadpool_limits
+    threadpool_limits(limits=golden_store.BLAS_THREADS, user_api="blas")
     ref_sgp, ref_proj = reference_loader.load()
     data = build_inputs()
     fixtures, golden = {}, {}
@@ -141,10 +144,9 @@ def main():
     golden["betadiv/value_1p5"] = np.asarray(ref_sgp.betaDiv(y1, x1, 1.5))
     golden["betadiv/deriv_1p7"] = np.asarray(ref_sgp.betaDivDeriv(y1, x1, 1.7))
 
-    np.savez_compressed(os.path.join(HERE, "fixtures.npz"), **fixtures)
-    np.savez_compressed(os.path.join(HERE, "golden_ref.npz"), **golden)
-    for f in ("fixtures.npz", "golden_ref.npz"):
-        print(f, os.path.getsize(os.path.join(HERE, f)) / 1e6, "MB")
+    for name, arrays in (("fixtures", fixtures), ("golden_ref", golden)):
+        for path in golden_store.save(name, arrays):
+            print(os.path.basename(path), os.path.getsize(path) / 1e6, "MB")
 
 
 if __name__ == "__main__":

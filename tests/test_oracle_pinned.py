@@ -5,10 +5,22 @@ fail the suite spuriously."""
 import numpy as np
 import pytest
 
+import golden_store
 from cases import CASES
 from oracle import sgp_oracle as orc
 
 FAST = [n for n in CASES if not n.endswith("_332")]
+
+
+@pytest.fixture(autouse=True, scope="module")
+def golden_blas_threads():
+    """np.dot (the reference's, hence the oracle's) runs on OpenBLAS, whose ddot splits vectors of more than 10 000 elements
+    over its threads: the thread count fixes the summation order, and the long runs below amplify that last-bit difference
+    to 1e-3 within a few hundred iterations.  make_golden.py ran with golden_store.BLAS_THREADS OpenBLAS threads; a machine
+    with another core count reproduces its vectors only with the same count."""
+    from threadpoolctl import threadpool_limits
+    with threadpool_limits(limits=golden_store.BLAS_THREADS, user_api="blas"):
+        yield
 
 
 @pytest.mark.parametrize("name", FAST)

@@ -6,7 +6,8 @@ import numpy as np
 import beta_sgp_b200 as bs
 from cases import CASES
 from conftest import case_inputs
-fx = np.load(os.path.join(ROOT, "tests/golden/fixtures.npz")); gd = np.load(os.path.join(ROOT, "tests/golden/golden_ref.npz"))
+import golden_store
+fx = golden_store.load("fixtures"); gd = golden_store.load("golden_ref")
 
 def conv_check(shape, G=0):
     rng = np.random.default_rng(1)

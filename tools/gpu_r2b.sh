@@ -40,7 +40,8 @@ import sys, os, numpy as np
 sys.path.insert(0, os.getcwd()); sys.path.insert(0, "tests"); sys.path.insert(0, "tests/golden")
 import beta_sgp_b200 as bs
 from conftest import case_inputs
-fx = np.load("tests/golden/fixtures.npz"); gd = np.load("tests/golden/golden_ref.npz")
+import golden_store
+fx = golden_store.load("fixtures"); gd = golden_store.load("golden_ref")
 for name in ("ngc_kl_27", "ngc_beta_p1_27", "sat_kl_40", "ngc_beta_p1_stop3", "stamp00", "stamp05", "tile00", "tile07", "cutout31_02"):
     gn, psf, bkg, div, kw = case_inputs(name, fx, gd)
     kw = dict(kw); flux = kw.pop("flux", None); b0 = kw.pop("betaParam", 1.005)
