@@ -73,6 +73,7 @@ template <typename T> struct ImgState {
     int tw_split;                    // the shared-memory tables are two-level (long transforms)
     ConvGeom geom;
     int nslab, bkg_img, init_recon, has_cap, pflag, want_err, stop2;
+    int x_ones;                      // the projection's X is 1, not clip(x): initial projection, first iteration from x = 0
     int masked, reg[4];              // zero-padded operator: valid window [reg0, reg1) x [reg2, reg3) of the FFT grid
     T bkg_raw_s, scaling, bkg_s, null_fill, x_const, cap, xlo, xhi;
     T div_a, div_at;                 // output divisors of A / A^T (zero-padded operator; 1 otherwise)
@@ -82,7 +83,7 @@ struct R2 { double a, b; };
 struct R3 { double a, b, c; };
 struct R7 { double v[7]; };
 
-enum { F_PENDING = 1, F_XONES = 2, F_FIRST = 4 };
+enum { F_FIRST = 4 };
 
 // divergence constants for the current beta (sgp.py:452-458)
 template <typename T> struct DivK {
@@ -283,28 +284,31 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE double ph_init(Ctx ctx, 
     return sum;
 }
 
-// initial projection, step 1: pflag 0 -> x = max(x, 0); pflag 1 -> c = x, X = 1
+// initial projection, step 1: pflag 0 -> x = max(x, 0); pflag 1 -> c = x (x_ones: X = 1)
 template <typename T, class Ctx> BSGP_NOINLINE void ph_proj_init_load(Ctx ctx, const ImgState<T>* S) {
     ctx.sync();
-    T* x = S->x; T* cbuf = S->d; T* Xbuf = S->t1; const bool pflag = S->pflag != 0;
+    T* x = S->x; T* cbuf = S->d; const bool pflag = S->pflag != 0;
     auto fetch = [&](int i) { In1<T> r; r.a = ld2(x, i); return r; };
     auto body = [&](int i, const In1<T>& in) {
-        if (pflag) { st2(cbuf, i, in.a); st2(Xbuf, i, mk2((T)1, (T)1)); }
+        if (pflag) st2(cbuf, i, in.a);
         else st2(x, i, mk2((in.a.x < (T)0) ? (T)0 : in.a.x, (in.a.y < (T)0) ? (T)0 : in.a.y));
     };
     pair_loop<4>(ctx, S->nslab, fetch, body);
 }
 
-// r(lambda) + b = sum_i x_i(lambda) over the slab                       flux_conserve_proj.py:22-25
+// r(lambda) + b = sum_i x_i(lambda) over the slab; X = clip(x) is recomputed from x     flux_conserve_proj.py:22-25
 template <typename T, bool MK, class Ctx> BSGP_NOINLINE double ph_proj_eval(Ctx ctx, const ImgState<T>* S, T lam) {
     ctx.sync();
-    const T* cbuf = S->d; const T* Xbuf = S->t1; const bool has_cap = S->has_cap != 0; const T cap = S->cap;
+    const T* cbuf = S->d; const T* x = S->x; const bool has_cap = S->has_cap != 0; const T cap = S->cap;
+    const T xlo = S->xlo, xhi = S->xhi;
+    const bool ones = S->x_ones != 0;
     const Region R = region_of<MK>(ctx, S);
     double s = 0.0;
-    auto fetch = [&](int i) { In2<T> r; r.a = ld2(cbuf, i); r.b = ld2(Xbuf, i); return r; };
+    auto fetch = [&](int i) { In2<T> r; r.a = ld2(cbuf, i); r.b = ones ? mk2((T)0, (T)0) : ld2(x, i); return r; };
+    auto X = [&](T xv) { return ones ? (T)1 : clip_bounds(xv, xlo, xhi); };
     auto body = [&](int i, const In2<T>& in) {
-        if (inside<MK>(R, i)) s += (double)proj_point(in.a.x, in.b.x, lam, has_cap, cap);
-        if (inside<MK>(R, i + 1)) s += (double)proj_point(in.a.y, in.b.y, lam, has_cap, cap);
+        if (inside<MK>(R, i)) s += (double)proj_point(in.a.x, X(in.b.x), lam, has_cap, cap);
+        if (inside<MK>(R, i + 1)) s += (double)proj_point(in.a.y, X(in.b.y), lam, has_cap, cap);
     };
     pair_loop<BSGP_U_PE>(ctx, S->nslab, fetch, body);
     return s;
@@ -438,35 +442,30 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE R2 ph_ri_bounds(Ctx ctx,
 // -------------------------------------------------------------------------------------------------
 // iteration phases (sgp.py:302-425 / 748-882)
 // -------------------------------------------------------------------------------------------------
-// proj_type 1: (pending x update,) X = clip(x), c = (x - alpha X g) / X           sgp.py:311-316
+// proj_type 1: X = clip(x), c = (x - alpha X g) / X                              sgp.py:311-316
+// X is not stored: ph_proj_eval and ph_rf_dir recompute it from x.
 // Also returns the slab sums of x(lambda) for lambda = 0, +1, -1: the root-find always starts with lambda = 0 and
 // then tries +1 or -1 (flux_conserve_proj.py:7,22,33,58), so its first two evaluations need no pass of their own.
-template <typename T, bool MK, class Ctx> BSGP_NOINLINE R3 ph_trial_point(Ctx ctx, const ImgState<T>* S, T al, T lam_pending, int flags) {
+template <typename T, bool MK, class Ctx> BSGP_NOINLINE R3 ph_trial_point(Ctx ctx, const ImgState<T>* S, T al) {
     ctx.sync();
-    T* x = S->x; const T* gr = S->g; T* cbuf = S->d; T* Xbuf = S->t1;
+    const T* x = S->x; const T* gr = S->g; T* cbuf = S->d;
     const T xlo = S->xlo, xhi = S->xhi, cap = S->cap;
-    const bool has_cap = S->has_cap != 0;
-    const bool pending = (flags & F_PENDING) != 0, ones = (flags & F_XONES) != 0;
+    const bool has_cap = S->has_cap != 0, ones = S->x_ones != 0;
     const Region R = region_of<MK>(ctx, S);
     double s0 = 0.0, sp = 0.0, sm = 0.0;
-    auto fetch = [&](int i) { In3<T> r; r.a = ld2(x, i); r.b = ld2(gr, i); r.c = pending ? ld2(cbuf, i) : mk2((T)0, (T)0); return r; };
-    auto one = [&](bool m, T xv, T gv, T dv, T& xo, T& co, T& Xo) {
-        if (!m) { xo = (T)0; co = (T)0; Xo = (T)1; return; }
-        if (pending) xv = nadd(xv, nmul(lam_pending, dv));
+    auto fetch = [&](int i) { In2<T> r; r.a = ld2(x, i); r.b = ld2(gr, i); return r; };
+    auto one = [&](bool m, T xv, T gv) -> T {
+        if (!m) return (T)0;
         const T X = ones ? (T)1 : clip_bounds(xv, xlo, xhi);
         const T y = nsub(xv, nmul(al, nmul(X, gv)));
-        xo = xv; co = nmul(y, ndiv((T)1, X)); Xo = X;
+        const T co = nmul(y, ndiv((T)1, X));
         s0 += (double)proj_point(co, X, (T)0, has_cap, cap);
         sp += (double)proj_point(co, X, (T)1, has_cap, cap);
         sm += (double)proj_point(co, X, (T)-1, has_cap, cap);
+        return co;
     };
-    auto body = [&](int i, const In3<T>& in) {
-        V2<T> xo, co, Xo;
-        one(inside<MK>(R, i), in.a.x, in.b.x, in.c.x, xo.x, co.x, Xo.x);
-        one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y, xo.y, co.y, Xo.y);
-        if (pending) st2(x, i, xo);
-        st2(cbuf, i, co);
-        st2(Xbuf, i, Xo);
+    auto body = [&](int i, const In2<T>& in) {
+        st2(cbuf, i, mk2(one(inside<MK>(R, i), in.a.x, in.b.x), one(inside<MK>(R, i + 1), in.a.y, in.b.y)));
     };
     pair_loop<BSGP_U_TP>(ctx, S->nslab, fetch, body);
     R3 r; r.a = s0; r.b = sp; r.c = sm;
@@ -474,41 +473,30 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE R3 ph_trial_point(Ctx ct
 }
 
 // producer of A(d): d = y - x with y the projected trial point; returns the slab part of gd = d.g   sgp.py:311-321
-template <typename T, bool MK, class Ctx> BSGP_NOINLINE double ph_rf_dir(Ctx ctx, const ImgState<T>* S, T al, T lam_proj, T lam_pending, int flags) {
+template <typename T, bool MK, class Ctx> BSGP_NOINLINE double ph_rf_dir(Ctx ctx, const ImgState<T>* S, T al, T lam_proj) {
     ctx.sync();
-    T* x = S->x; const T* gr = S->g; T* dbuf = S->d; const T* Xbuf = S->t1;
+    const T* x = S->x; const T* gr = S->g; T* dbuf = S->d;
     const T xlo = S->xlo, xhi = S->xhi, cap = S->cap;
-    const bool has_cap = S->has_cap != 0, pflag = S->pflag != 0;
-    const bool pending = (flags & F_PENDING) != 0, ones = (flags & F_XONES) != 0;
+    const bool has_cap = S->has_cap != 0, pflag = S->pflag != 0, ones = S->x_ones != 0;
     const Region R = region_of<MK>(ctx, S);
     double gd = 0.0;
-    auto pf = [&](int i) {
-        In4<T> r; r.a = ld2(x, i); r.b = ld2(gr, i);
-        r.c = (pflag || pending) ? ld2(dbuf, i) : mk2((T)0, (T)0);
-        r.d = pflag ? ld2(Xbuf, i) : mk2((T)0, (T)0);
-        return r;
-    };
-    auto one = [&](bool m, T xv, T gv, T cv, T Xv, T& xo) -> T {
-        if (!m) { xo = (T)0; return (T)0; }
+    auto pf = [&](int i) { In3<T> r; r.a = ld2(x, i); r.b = ld2(gr, i); r.c = pflag ? ld2(dbuf, i) : mk2((T)0, (T)0); return r; };
+    auto one = [&](bool m, T xv, T gv, T cv) -> T {
+        if (!m) return (T)0;
+        const T X = ones ? (T)1 : clip_bounds(xv, xlo, xhi);
         T y;
         if (pflag) {
-            y = proj_point(cv, Xv, lam_proj, has_cap, cap);
+            y = proj_point(cv, X, lam_proj, has_cap, cap);
         } else {
-            if (pending) xv = nadd(xv, nmul(lam_pending, cv));
-            const T X = ones ? (T)1 : clip_bounds(xv, xlo, xhi);
             y = nsub(xv, nmul(al, nmul(X, gv)));
             y = (y < (T)0) ? (T)0 : y;
         }
-        xo = xv;
         const T d = nsub(y, xv);
         gd += (double)nmul(d, gv);
         return d;
     };
-    auto pe = [&](int i, const In4<T>& in) -> V2<T> {
-        V2<T> xo, d;
-        d.x = one(inside<MK>(R, i), in.a.x, in.b.x, in.c.x, in.d.x, xo.x);
-        d.y = one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y, in.d.y, xo.y);
-        if (!pflag && pending) st2(x, i, xo);
+    auto pe = [&](int i, const In3<T>& in) -> V2<T> {
+        const V2<T> d = mk2(one(inside<MK>(R, i), in.a.x, in.b.x, in.c.x), one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y));
         st2(dbuf, i, d);
         return d;
     };
@@ -604,8 +592,10 @@ template <typename T, bool MK, int KIND, class Ctx> BSGP_NOINLINE R3 ph_trial_k(
 }
 
 // consumer of A^T(.): new gradient, y_k, Barzilai-Borwein sums, stop-rule / error sums   sgp.py:343-365, 394-402
+// The next iterate x + lam*d goes into the d array (d is dead after this pass); the controller swaps the x and d
+// pointers when the loop continues, so x keeps the previous iterate when it stops.
 template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, const ImgState<T>* S, T lam, int kind) {
-    const T* t1 = S->t1; T* gr = S->g; const T* dbuf = S->d; const T* x = S->x; const T* truth = S->truth;
+    const T* t1 = S->t1; T* gr = S->g; T* dbuf = S->d; const T* x = S->x; const T* truth = S->truth;
     const T xlo = S->xlo, xhi = S->xhi, scaling = S->scaling, div = S->div_at;
     const bool want_err = S->want_err != 0, stop2 = S->stop2 != 0;
     const Region R = region_of<MK>(ctx, S);
@@ -616,8 +606,8 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, con
         In5<T> r; r.a = ld2(t1, i); r.b = ld2(gr, i); r.c = ld2(dbuf, i); r.d = ld2(x, i);
         r.e = want_err ? ld2(truth, i) : mk2((T)0, (T)0); return r;
     };
-    auto one = [&](bool m, T p1, T gold, T dv, T xv, T tr, T w) -> T {
-        if (!m) return (T)0;
+    auto one = [&](bool m, T p1, T gold, T dv, T xv, T tr, T w, T& xo) -> T {
+        if (!m) { xo = (T)0; return (T)0; }
         if (MK) w = ndiv(w, div);
         const T gnew = (kind == 0) ? nsub((T)1, w) : nsub(p1, w);
         const T yk = nsub(gnew, gold);
@@ -632,13 +622,15 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, con
         bb[3] += (double)yk2 * (double)yk2;
         if (stop2) { bb[4] += (double)sk * (double)sk; bb[5] += (double)xn * (double)xn; }
         if (want_err) { const T e = nsub(xn, ndiv(tr, scaling)); bb[6] += (double)nmul(e, e); }
+        xo = xn;
         return gnew;
     };
     auto ca = [&](int i, const In5<T>& in, V2<T> w) {
-        V2<T> gnew;
-        gnew.x = one(inside<MK>(R, i), in.a.x, in.b.x, in.c.x, in.d.x, in.e.x, w.x);
-        gnew.y = one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y, in.d.y, in.e.y, w.y);
+        V2<T> gnew, xn;
+        gnew.x = one(inside<MK>(R, i), in.a.x, in.b.x, in.c.x, in.d.x, in.e.x, w.x, xn.x);
+        gnew.y = one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y, in.d.y, in.e.y, w.y, xn.y);
         st2(gr, i, gnew);
+        st2(dbuf, i, xn);
     };
     conv_rows_inverse<1, MK>(ctx, S->geom, S->ws_off, S->twx, S->twx_off, S->tw_split, S->ppx_off, S->spec, cf, ca);
     R7 r;
@@ -680,9 +672,9 @@ template <typename T> struct CtlState {
     double pre[3];                                   // sums of x(lambda) at lambda = 0, +1, -1 delivered by ph_trial_point
     double alpha_hist[kMaxMem], f_hist[kMaxMem];     // Valpha / Fold (sgp.py:214-215)
     DivK<T> dk;
-    T al, lam_pending, lam_proj;
-    int status, total_evals, total_trials, iter, trials, evals, flags;
-    int have_pre, s1_valid, X_is_ones, keep_going, pending;
+    T al, lam_proj;
+    int status, total_evals, total_trials, iter, trials, evals;
+    int have_pre, s1_valid, keep_going;
 };
 
 // all-reduce of K doubles as a real function (the execution context travels by value, its parity comes back)
@@ -787,6 +779,17 @@ template <typename T> BSGP_NOINLINE double ctl_finish_iteration(const bsgp_param
     return stop_val;
 }
 
+// x <- x + lam*d: ph_ri_bb has stored the new iterate in the d array, so the x and d arrays swap roles.  When the loop stops
+// nothing is swapped and x still holds the previous iterate, which is what the reference returns (sgp.py:424-425).  Only
+// thread 0 of each CTA writes S: every thread read it before the all-reduce that followed ph_ri_bb, and the next phase
+// opens with a barrier.  A real function: a thread-index test in the controller's loop costs it registers across every
+// phase call.
+template <typename T, class Ctx> BSGP_NOINLINE void ctl_accept_step(Ctx ctx, ImgState<T>* S, int keep_going) {
+    if (ctx.tid != 0) return;
+    S->x_ones = 0;
+    if (keep_going) { T* t = S->x; S->x = S->d; S->d = t; }
+}
+
 template <typename T, bool MK, class Ctx>
 BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* const* buf, cplx<T>* tf, cplx<T>* tf_adj, int img) {
     const bsgp_params& P = a.p;
@@ -818,6 +821,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
             S->tf_at = P.adjoint_second_psf ? tf_adj : tf;
             S->nslab = nslab; S->bkg_img = bkg_img; S->init_recon = P.init_recon; S->has_cap = P.has_sat != 0;
             S->pflag = pflag; S->want_err = want_err; S->stop2 = (P.stop_criterion == 2);
+            S->x_ones = 1;                                                  // the initial projection: c = x, X = 1
             S->bkg_raw_s = bkg_raw_s;
             S->masked = masked; S->reg[0] = P.region[0]; S->reg[1] = P.region[1]; S->reg[2] = P.region[2]; S->reg[3] = P.region[3];
             S->div_a = masked ? (T)P.div_a : (T)1; S->div_at = masked ? (T)P.div_at : (T)1;
@@ -946,13 +950,9 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         for (int k = 0; k < MA; ++k) W->alpha_hist[k] = P.alpha_max;
         for (int k = 0; k < M; ++k) W->f_hist[k] = -1e30;
     }
-    W->X_is_ones = (P.init_recon == 0);
+    if (ctx.tid == 0) S->x_ones = (P.init_recon == 0);                 // X = 1 in the first iteration from a zero start
     W->iter = 1;
     W->keep_going = (W->status == BSGP_ST_OK);
-    // The accepted step x <- x + lam*d is applied lazily at the start of the NEXT iteration, so when
-    // the loop stops x still holds the previous iterate, which is what the reference returns (:424-425).
-    W->pending = 0;
-    W->lam_pending = (T)0;
 
     while (W->keep_going) {
         // history shift (:306-308)
@@ -966,19 +966,16 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
 
         // ---- trial point y = x - alpha X g, projection (:311-318)
         W->al = (T)W->alpha;
-        W->flags = (W->pending ? F_PENDING : 0) | (W->X_is_ones ? F_XONES : 0);
         W->evals = 0;
         W->lam_proj = (T)0;
         if (pflag) {
             {
-                const R3 t = ph_trial_point<T, MK>(ctx, S, W->al, W->lam_pending, W->flags);
+                const R3 t = ph_trial_point<T, MK>(ctx, S, W->al);
                 double pre[3] = {t.a, t.b, t.c};
                 allreduce_fn<0, 3>(ctx, pre);
                 W->pre[0] = pre[0]; W->pre[1] = pre[1]; W->pre[2] = pre[2];
                 W->have_pre = 1;
             }
-            W->pending = 0;
-            W->flags &= ~F_PENDING;
             const RfOut rf = rootfind_call<T, MK>(ctx, S, W, P.max_projs);
             ctx.parity = rf.parity;
             const ProjResult pr = rf.pr;
@@ -991,8 +988,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         // ---- d = y - x, gd = d.g, d_tf = A(d) with the first line-search trial fused (:318-334)
         {
             double sums[4];   // [0..2] objective terms, [3] gd
-            sums[3] = ph_rf_dir<T, MK>(ctx, S, W->al, W->lam_proj, W->lam_pending, W->flags);
-            W->pending = 0;
+            sums[3] = ph_rf_dir<T, MK>(ctx, S, W->al, W->lam_proj);
             conv_middle<T, MK>(ctx, S, S->tf, CONV_TF);
             {
                 const R3 o = BSGP_DISPATCH_KIND(W->dk, ph_ri_trial_k, ctx, S, W->dk);
@@ -1029,12 +1025,11 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         }
         W->total_trials += W->trials;
 
-        // ---- accept: x_tf, new gradient through A^T, BB sums (:337-347, 355-365, 402); x itself is updated lazily
+        // ---- accept: x_tf, new gradient through A^T, BB sums (:337-347, 355-365, 402); the new x goes into the d array
         ph_rf_grad<T, MK>(ctx, S, W->dk.kind, (T)W->lam, 0);
         conv_middle<T, MK>(ctx, S, S->tf_at, mode_at);
         R7 bbr = ph_ri_bb<T, MK>(ctx, S, (T)W->lam, W->dk.kind);
         allreduce_fn<0, 7>(ctx, bbr.v);
-        W->X_is_ones = 0;
 
         // ---- Barzilai-Borwein steps, lr schedule, bookkeeping and stop rules (:366-425)
         const double stop_val = ctl_finish_iteration<T>(&a.p, W, bbr);
@@ -1051,7 +1046,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
             if (a.tr_evals) a.tr_evals[o] = W->evals;
             if (want_err && iter <= P.maxit + 1) a.err[(size_t)img * (P.maxit + 2) + iter] = sqrt(bbr.v[6] / W->truth_sq);   // :394-396
         }
-        if (W->keep_going) { W->pending = 1; W->lam_pending = (T)W->lam; }       // else: the previous iterate is returned (:424-425)
+        ctl_accept_step<T>(ctx, S, W->keep_going);
     }
 
     // ------------------------------------------------------------------ epilogue (:427-438)
