@@ -100,25 +100,21 @@ def lib():
     L.bsgp_plan_configure.argtypes = [vp, ip, ip]
     L.bsgp_set_psf.argtypes = [vp, vp, ip, vp]
     L.bsgp_set_psf_host.argtypes = [vp, vp, ip]
-    if hasattr(L, "bsgp_set_psf_adjoint"):            # absent only in older builds loaded through BSGP_LIB for A/B runs
-        L.bsgp_set_psf_adjoint.argtypes = [vp, vp, ip, vp]
-        L.bsgp_set_psf_adjoint_host.argtypes = [vp, vp, ip]
+    L.bsgp_set_psf_adjoint.argtypes = [vp, vp, ip, vp]
+    L.bsgp_set_psf_adjoint_host.argtypes = [vp, vp, ip]
     L.bsgp_solve_batch.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
     L.bsgp_solve_batch_host.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs)]
-    if hasattr(L, "bsgp_solve_batch_pinned"):
-        L.bsgp_solve_batch_pinned.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
+    L.bsgp_solve_batch_pinned.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
     L.bsgp_apply_psf.argtypes = [vp, vp, vp, ip, ip, vp]
     L.bsgp_apply_psf_host.argtypes = [vp, vp, vp, ip, ip]
     L.bsgp_project_df.argtypes = [vp, vp, vp, ip, ip, dp, dp, dp, dp, ip, ip, ip, vp, vp, vp, ip, vp]
     L.bsgp_project_df_host.argtypes = [vp, vp, vp, ip, ip, dp, dp, dp, dp, ip, ip, ip, vp, vp, vp, ip]
     L.bsgp_beta_div_host.argtypes = [vp, vp, C.c_longlong, dp, vp, vp, ip]
     L.bsgp_beta_grad_terms_host.argtypes = [vp, vp, C.c_longlong, dp, vp, vp, ip]
-    if hasattr(L, "bsgp_tile_boxes"):
-        L.bsgp_tile_boxes.argtypes = [ip, ip, ip, ip, dp, dp, vp, ip, C.POINTER(ip)]
-        L.bsgp_extract_tiles.argtypes = [vp, ip, ip, ip, vp, ip, ip, ip, vp, ip, vp]
-        L.bsgp_assemble_tiles.argtypes = [vp, vp, ip, ip, ip, ip, ip, vp, ip, ip, ip, vp]
-    if hasattr(L, "bsgp_psf_model_eval"):
-        L.bsgp_psf_model_eval.argtypes = [vp, ip, ip, ip, ip, ip, ip, ip, vp, ip, vp]
+    L.bsgp_tile_boxes.argtypes = [ip, ip, ip, ip, dp, dp, vp, ip, C.POINTER(ip)]
+    L.bsgp_extract_tiles.argtypes = [vp, ip, ip, ip, vp, ip, ip, ip, vp, ip, vp]
+    L.bsgp_assemble_tiles.argtypes = [vp, vp, ip, ip, ip, ip, ip, vp, ip, ip, ip, vp]
+    L.bsgp_psf_model_eval.argtypes = [vp, ip, ip, ip, ip, ip, ip, ip, vp, ip, vp]
     L.bsgp_device_count.restype = ip
     L.bsgp_launch_count.restype = C.c_longlong
     L.bsgp_last_error_string.restype = C.c_char_p

@@ -462,10 +462,6 @@ template <typename T> static int plan_setup_frame(bsgp_plan* p) {
         const int want = p->g.lg_col_tile > 2 ? p->g.lg_col_tile : 2;
         if (want < p->g.lg_cp) p->g.lg_cp = want;
     }
-    if (const char* e = getenv("BSGP_FRAME_LGCP")) {      // tuning experiments: log2 of the panel width
-        const int v = atoi(e);
-        if (v >= 0 && v <= ilog2(p->g.cols_per_cta)) p->g.lg_cp = v;
-    }
     SmemPlan sp;
     size_t off = up128(sizeof(SharedCtl));
     sp.off_state = (unsigned)off; off = up128(off + sizeof(ImgState<T>));
@@ -533,13 +529,7 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
     if (threads <= 0) threads = small_slab ? (p->small_try ? 128 : 256) : 128;
     if (threads != 256 && threads != 512 && threads != 128) return fail(BSGP_E_ARG, "threads must be 128, 256 or 512");
     int minb = threads >= 512 ? 1 : (threads >= 256 ? (small_slab ? 2 : 1) : (small_slab ? 3 : 4));
-    if (const char* e = getenv("BSGP_MINB")) {             // tuning experiments: CTAs per SM
-        const int v = atoi(e);
-        if (threads == 256 && (v == 1 || v == 2)) minb = v;
-        if (threads == 128 && (v == 3 || v == 4)) minb = v;
-    }
     size_t ws_limit = (minb >= 4 ? 38 : 76) * 1024;
-    if (const char* e = getenv("BSGP_WS_KB")) { const int v = atoi(e); if (v >= 8 && v <= 200) ws_limit = (size_t)v * 1024; }
     // short sides that are not a power of two: dense DFT of the image's own length on the first slots of the grid (bsgp_wrap.h)
     const int dny = p->ny != p->img_ny ? dense_len(p->img_ny) : 0, dnx = p->nx != p->img_nx ? dense_len(p->img_nx) : 0;
     bool ok = make_geom(p->ny, p->nx, G, sizeof(cplx<T>), ws_limit, &p->g, &p->ws_bytes, dny, dnx);
@@ -971,8 +961,10 @@ int bsgp_set_psf_adjoint_host(bsgp_plan* p, const void* psf_host, int n_psf) {
     return rc;
 }
 
-// argument checks + launch; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0
-static int solve_checked(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
+// Argument checks of every solve entry point.  The host entry points run them on the caller's pointers before they size
+// anything from batch or prm->maxit (the device copies they stage are present exactly where the caller's arrays are),
+// and they can read the queue order: the kernel indexes the images with it, so every entry must lie in 0..batch-1.
+static int check_solve(const bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, bool host) {
     if (!p || !prm || !in || !out) return fail(BSGP_E_ARG, "NULL argument");
     if (batch < 1) return fail(BSGP_E_ARG, "batch must be >= 1");
     int rc = check_params(prm);
@@ -994,11 +986,17 @@ static int solve_checked(bsgp_plan* p, const bsgp_params* prm, int batch, const 
             return fail(BSGP_E_ARG, "region {%d, %d, %d, %d} does not fit the %dx%d grid", r[0], r[1], r[2], r[3], p->ny, p->nx);
         if (!(prm->div_a > 0.0) || !(prm->div_at > 0.0)) return fail(BSGP_E_ARG, "div_a / div_at must be positive when a region is set");
     }
+    if (host && in->order) for (int i = 0; i < batch; ++i) if (in->order[i] < 0 || in->order[i] >= batch) return fail(BSGP_E_ARG, "inputs.order is not a permutation of 0..batch-1");
+    return BSGP_OK;
+}
+
+// launch on device arrays that passed check_solve; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0
+static int solve_launch(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
     if (!p->embedded && (misaligned(in->gn) || misaligned(out->x) || misaligned(in->x0) || misaligned(in->obj) || (in->bkg_is_image && misaligned(in->bkg))))
         return fail(BSGP_E_ARG, "image pointers must be 16-byte aligned (vector loads)");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
-    rc = plan_enter(p, st);
+    int rc = plan_enter(p, st);
     if (rc) return rc;
     rc = p->dtype == BSGP_F64 ? solve_t<double>(p, prm, batch, in, out, st, ready) : solve_t<float>(p, prm, batch, in, out, st, ready);
     if (rc) return rc;
@@ -1006,7 +1004,8 @@ static int solve_checked(bsgp_plan* p, const bsgp_params* prm, int batch, const 
 }
 
 int bsgp_solve_batch(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
-    return solve_checked(p, prm, batch, in, out, stream, nullptr);
+    const int rc = check_solve(p, prm, batch, in, out, false);
+    return rc ? rc : solve_launch(p, prm, batch, in, out, stream, nullptr);
 }
 
 // host staging helpers -----------------------------------------------------------------------
@@ -1031,37 +1030,76 @@ struct DevBuf {
         return BSGP_OK;
     }
 };
-
-int bsgp_solve_batch_host(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
-    if (!p || !prm || !in || !out) return fail(BSGP_E_ARG, "NULL argument");
-    CU(cudaSetDevice(p->device));
-    const size_t img = (size_t)p->img_ny * p->img_nx * p->elem, B = (size_t)batch, tr = (size_t)(prm->maxit + 1);
-    DevBuf gn, bkg, flux, beta0, x0, obj, order, x, iters, status, discr, times, stopv, err, bfin, pe, lt, sc, ta, tl, tb, tt, te;
-    int rc;
 #define TRY(e) do { rc = (e); if (rc) return rc; } while (0)
-    TRY(gn.up(in->gn, B * img));
-    TRY(bkg.up(in->bkg, in->bkg_is_image ? B * img : B * p->elem));
-    TRY(flux.up(in->flux, B * 8)); TRY(beta0.up(in->beta0, B * 8)); TRY(x0.up(in->x0, B * img)); TRY(obj.up(in->obj, B * img));
-    TRY(order.up(in->order, B * 4));
-    TRY(x.alloc(true, B * img)); TRY(iters.alloc(true, B * 4)); TRY(status.alloc(true, B * 4));
-    TRY(discr.alloc(true, B * tr * 8)); TRY(times.alloc(true, B * tr * 8));
-    TRY(stopv.alloc(out->stop_value, B * tr * 8)); TRY(err.alloc(out->err, B * (tr + 1) * 8)); TRY(bfin.alloc(out->beta_final, B * 8));
-    TRY(pe.alloc(out->proj_evals, B * 4)); TRY(lt.alloc(out->ls_trials, B * 4)); TRY(sc.alloc(out->scalars, B * BSGP_NSCALARS * 8));
-    TRY(ta.alloc(out->trace_alpha, B * tr * 8)); TRY(tl.alloc(out->trace_lambda, B * tr * 8)); TRY(tb.alloc(out->trace_beta, B * tr * 8));
-    TRY(tt.alloc(out->trace_trials, B * tr * 4)); TRY(te.alloc(out->trace_evals, B * tr * 4));
-    bsgp_inputs di = {gn.d, bkg.d, in->bkg_is_image, (const double*)flux.d, (const double*)beta0.d, x0.d, obj.d, (const int*)order.d};
-    bsgp_outputs dout = {x.d, (int*)iters.d, (int*)status.d, (double*)discr.d, (double*)times.d, (double*)stopv.d, (double*)err.d,
-                         (double*)bfin.d, (int*)pe.d, (int*)lt.d, (double*)sc.d, (double*)ta.d, (double*)tl.d, (double*)tb.d,
-                         (int*)tt.d, (int*)te.d};
-    TRY(bsgp_solve_batch(p, prm, batch, &di, &dout, nullptr));
+
+// The host I/O of one solve, laid out in one device staging area: the caller's pointer of every array (nullptr: absent),
+// its size for this batch and its offset in the area, inputs first, then the outputs, which are zero-filled before the
+// launch and copied back after it.  The restored images are staged too, unless the kernel stores them straight into
+// host memory through `x_mapped`.
+struct HostIO {
+    enum Slot { GN, BKG, X0, OBJ, FLUX, BETA0, ORDER,                 // inputs, the image-shaped ones first
+                X, ITERS, STATUS, DISCR, TIMES, STOP_VALUE, ERR, BETA_FINAL, PROJ_EVALS, LS_TRIALS, SCALARS,
+                TRACE_ALPHA, TRACE_LAMBDA, TRACE_BETA, TRACE_TRIALS, TRACE_EVALS, NSLOT };
+    const void* host[NSLOT];              // nullptr: not staged
+    size_t bytes[NSLOT], off[NSLOT];
+    size_t out_begin = 0, size = 0;       // the outputs occupy [out_begin, size)
+    size_t img;                           // bytes of one image
+    int bkg_is_image;
+    void* x_mapped;
+
+    HostIO(const bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* x_mapped_)
+        : img((size_t)p->img_ny * p->img_nx * p->elem), bkg_is_image(in->bkg_is_image), x_mapped(x_mapped_) {
+        const size_t B = (size_t)batch, tr = (size_t)prm->maxit + 1, imgs = B * img, it8 = B * tr * 8, it4 = B * tr * 4;
+        const void* const h[NSLOT] = {in->gn, in->bkg, in->x0, in->obj, in->flux, in->beta0, in->order,
+                                      x_mapped ? nullptr : out->x, out->iters, out->status, out->discr, out->times, out->stop_value,
+                                      out->err, out->beta_final, out->proj_evals, out->ls_trials, out->scalars,
+                                      out->trace_alpha, out->trace_lambda, out->trace_beta, out->trace_trials, out->trace_evals};
+        const size_t n[NSLOT] = {imgs, bkg_is_image ? imgs : B * p->elem, imgs, imgs, B * 8, B * 8, B * 4,
+                                 imgs, B * 4, B * 4, it8, it8, it8,
+                                 B * (tr + 1) * 8, B * 8, B * 4, B * 4, B * BSGP_NSCALARS * 8,
+                                 it8, it8, it8, it4, it4};
+        for (int k = 0; k < NSLOT; ++k) {
+            if (k == X) out_begin = size;
+            host[k] = h[k]; bytes[k] = n[k]; off[k] = size;
+            if (h[k]) size = (size + n[k] + 255) & ~(size_t)255;
+        }
+    }
+    bool image(int k) const { return k <= OBJ && (k != BKG || bkg_is_image); }
+    // the solve on the staging area at `base`
+    int launch(bsgp_plan* p, const bsgp_params* prm, int batch, char* base, void* stream, const int* ready) const {
+        auto dev = [&](int k) -> void* { return host[k] ? base + off[k] : nullptr; };
+        const bsgp_inputs in = {dev(GN), dev(BKG), bkg_is_image, (const double*)dev(FLUX), (const double*)dev(BETA0), dev(X0), dev(OBJ),
+                                (const int*)dev(ORDER)};
+        const bsgp_outputs out = {x_mapped ? x_mapped : dev(X), (int*)dev(ITERS), (int*)dev(STATUS), (double*)dev(DISCR), (double*)dev(TIMES),
+                                  (double*)dev(STOP_VALUE), (double*)dev(ERR), (double*)dev(BETA_FINAL), (int*)dev(PROJ_EVALS),
+                                  (int*)dev(LS_TRIALS), (double*)dev(SCALARS), (double*)dev(TRACE_ALPHA), (double*)dev(TRACE_LAMBDA),
+                                  (double*)dev(TRACE_BETA), (int*)dev(TRACE_TRIALS), (int*)dev(TRACE_EVALS)};
+        return solve_launch(p, prm, batch, &in, &out, stream, ready);
+    }
+    // the staged outputs to the caller's arrays, queued on `st`
+    int copy_back(const char* base, cudaStream_t st) const {
+        for (int k = X; k < NSLOT; ++k)
+            if (host[k]) CU(cudaMemcpyAsync(const_cast<void*>(host[k]), base + off[k], bytes[k], cudaMemcpyDeviceToHost, st));
+        return BSGP_OK;
+    }
+};
+
+// pageable host arrays: one staging allocation per call, freed before returning
+int bsgp_solve_batch_host(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
+    int rc;
+    TRY(check_solve(p, prm, batch, in, out, true));
+    CU(cudaSetDevice(p->device));
+    const HostIO io(p, prm, batch, in, out, nullptr);
+    DevBuf area;
+    TRY(area.alloc(true, io.size));
+    char* base = (char*)area.d;
+    for (int k = 0; k < HostIO::X; ++k)
+        if (io.host[k]) CU(cudaMemcpy(base + io.off[k], io.host[k], io.bytes[k], cudaMemcpyHostToDevice));
+    TRY(io.launch(p, prm, batch, base, nullptr, nullptr));
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess) return fail(BSGP_E_CUDA, "solve kernel failed: %s", cudaGetErrorString(e));
-    TRY(x.down(out->x, B * img)); TRY(iters.down(out->iters, B * 4)); TRY(status.down(out->status, B * 4));
-    TRY(discr.down(out->discr, B * tr * 8)); TRY(times.down(out->times, B * tr * 8)); TRY(stopv.down(out->stop_value, B * tr * 8));
-    TRY(err.down(out->err, B * (tr + 1) * 8)); TRY(bfin.down(out->beta_final, B * 8)); TRY(pe.down(out->proj_evals, B * 4));
-    TRY(lt.down(out->ls_trials, B * 4)); TRY(sc.down(out->scalars, B * BSGP_NSCALARS * 8)); TRY(ta.down(out->trace_alpha, B * tr * 8));
-    TRY(tl.down(out->trace_lambda, B * tr * 8)); TRY(tb.down(out->trace_beta, B * tr * 8)); TRY(tt.down(out->trace_trials, B * tr * 4));
-    TRY(te.down(out->trace_evals, B * tr * 4));
+    TRY(io.copy_back(base, nullptr));
+    CU(cudaStreamSynchronize(nullptr));
     return BSGP_OK;
 }
 
@@ -1085,41 +1123,19 @@ static bool page_locked(const void* h) {
 }
 
 int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
-    if (!p || !prm || !in || !out) return fail(BSGP_E_ARG, "NULL argument");
-    if (batch < 1) return fail(BSGP_E_ARG, "batch must be >= 1");
-    if (!in->gn || !in->bkg || !out->x || !out->iters || !out->status || !out->discr || !out->times) return fail(BSGP_E_ARG, "required pointer is NULL");
+    int rc;
+    TRY(check_solve(p, prm, batch, in, out, true));
     CU(cudaSetDevice(p->device));
     if (!page_locked(in->gn) || !page_locked(out->x) || !page_locked(in->x0) || !page_locked(in->obj) || (in->bkg_is_image && !page_locked(in->bkg)))
         return fail(BSGP_E_ARG, "bsgp_solve_batch_pinned needs page-locked image buffers (cudaHostAlloc / cudaHostRegister / torch pin_memory)");
-    if (in->order) for (int i = 0; i < batch; ++i) if (in->order[i] < 0 || in->order[i] >= batch) return fail(BSGP_E_ARG, "inputs.order is not a permutation of 0..batch-1");
-    int pin_mode = 0;                                             // experiments: 1 = stage x on the device and copy it back at the end, 2 = upload everything before the flags
-    if (const char* e = getenv("BSGP_PIN_MODE")) pin_mode = atoi(e);
     void* x_mapped = nullptr;
     CU(cudaHostGetDevicePointer(&x_mapped, out->x, 0));
+    const HostIO io(p, prm, batch, in, out, x_mapped);
+    const size_t img = io.img, B = (size_t)batch;
     // images in the caller's own shape: a plan whose grid differs from it (sides that are not a power of two) moves them
     // to and from the grid on the device (solve_t), which needs all of them resident first, like frame mode
-    const size_t img = (size_t)p->img_ny * p->img_nx * p->elem, B = (size_t)batch, tr = (size_t)(prm->maxit + 1);
     const bool resident_first = p->frame || p->embedded;
-    // ---- carve the staging arena
-    size_t off = 0;
-    auto carve = [&](bool want, size_t bytes) -> size_t { if (!want) return (size_t)-1; const size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_gn = carve(true, B * img), o_bkg = carve(true, in->bkg_is_image ? B * img : B * p->elem);
-    const size_t o_x0 = carve(in->x0 != nullptr, B * img), o_obj = carve(in->obj != nullptr, B * img);
-    const size_t o_flux = carve(in->flux != nullptr, B * 8), o_b0 = carve(in->beta0 != nullptr, B * 8), o_ord = carve(in->order != nullptr, B * 4);
-    const size_t o_xs = carve((pin_mode & 1) != 0, B * img);
-    const size_t o_small = off;                                   // everything from here on is zero-filled output
-    const size_t o_it = carve(true, B * 4), o_st = carve(true, B * 4), o_di = carve(true, B * tr * 8), o_ti = carve(true, B * tr * 8);
-    const size_t o_sv = carve(out->stop_value != nullptr, B * tr * 8), o_er = carve(out->err != nullptr, B * (tr + 1) * 8);
-    const size_t o_bf = carve(out->beta_final != nullptr, B * 8), o_pe = carve(out->proj_evals != nullptr, B * 4), o_lt = carve(out->ls_trials != nullptr, B * 4);
-    const size_t o_sc = carve(out->scalars != nullptr, B * BSGP_NSCALARS * 8);
-    const size_t o_ta = carve(out->trace_alpha != nullptr, B * tr * 8), o_tl = carve(out->trace_lambda != nullptr, B * tr * 8), o_tb = carve(out->trace_beta != nullptr, B * tr * 8);
-    const size_t o_tt = carve(out->trace_trials != nullptr, B * tr * 4), o_te = carve(out->trace_evals != nullptr, B * tr * 4);
-    if (off > p->stage_cap) {
-        CU(cudaDeviceSynchronize());
-        cudaFree(p->stage); p->stage = nullptr; p->stage_cap = 0;
-        CU(cudaMalloc(&p->stage, off));
-        p->stage_cap = off;
-    }
+    TRY(grow(&p->stage, &p->stage_cap, io.size));
     if (batch > p->ready_cap) {
         CU(cudaDeviceSynchronize());
         cudaFree(p->ready); cudaFreeHost(p->ones_host); p->ready = nullptr; p->ones_host = nullptr; p->ready_cap = 0;
@@ -1134,79 +1150,55 @@ int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, con
         for (cudaEvent_t* e : {&p->ev_fork, &p->ev_flags, &p->ev_copy, &p->ev_run}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
     }
     char* S = (char*)p->stage;
-    auto at = [&](size_t o) -> void* { return o == (size_t)-1 ? nullptr : (void*)(S + o); };
     cudaStream_t user = (cudaStream_t)stream, sc = p->s_copy, sr = p->s_run;
     // ---- fork from the caller's stream (the PSF spectra may still be in flight there)
     CU(cudaEventRecord(p->ev_fork, user));
     CU(cudaStreamWaitEvent(sc, p->ev_fork, 0));
     CU(cudaStreamWaitEvent(sr, p->ev_fork, 0));
     // ---- run stream: small inputs, cleared outputs and flags, then the kernel
-    if (!in->bkg_is_image) CU(cudaMemcpyAsync(at(o_bkg), in->bkg, B * p->elem, cudaMemcpyHostToDevice, sr));
-    if (in->flux) CU(cudaMemcpyAsync(at(o_flux), in->flux, B * 8, cudaMemcpyHostToDevice, sr));
-    if (in->beta0) CU(cudaMemcpyAsync(at(o_b0), in->beta0, B * 8, cudaMemcpyHostToDevice, sr));
-    if (in->order) CU(cudaMemcpyAsync(at(o_ord), in->order, B * 4, cudaMemcpyHostToDevice, sr));
-    CU(cudaMemsetAsync(S + o_small, 0, off - o_small, sr));
+    for (int k = 0; k < HostIO::X; ++k)
+        if (io.host[k] && !io.image(k)) CU(cudaMemcpyAsync(S + io.off[k], io.host[k], io.bytes[k], cudaMemcpyHostToDevice, sr));
+    CU(cudaMemsetAsync(S + io.out_begin, 0, io.size - io.out_begin, sr));
     CU(cudaMemsetAsync(p->ready, 0, B * sizeof(int), sr));
     CU(cudaEventRecord(p->ev_flags, sr));
     CU(cudaStreamWaitEvent(sc, p->ev_flags, 0));                   // no flag may be raised before the flags are cleared
-    bsgp_inputs di = {at(o_gn), at(o_bkg), in->bkg_is_image, (const double*)at(o_flux), (const double*)at(o_b0), at(o_x0), at(o_obj), (const int*)at(o_ord)};
-    bsgp_outputs dout = {(pin_mode & 1) ? at(o_xs) : x_mapped, (int*)at(o_it), (int*)at(o_st), (double*)at(o_di), (double*)at(o_ti), (double*)at(o_sv), (double*)at(o_er),
-                         (double*)at(o_bf), (int*)at(o_pe), (int*)at(o_lt), (double*)at(o_sc), (double*)at(o_ta), (double*)at(o_tl), (double*)at(o_tb),
-                         (int*)at(o_tt), (int*)at(o_te)};
-    const bool per_item = !p->frame && (img >= 65536 || in->order == nullptr) && !(pin_mode & 2);
-    auto upload_all = [&]() -> int {
-        CU(cudaMemcpyAsync(at(o_gn), in->gn, B * img, cudaMemcpyHostToDevice, sc));
-        if (in->bkg_is_image) CU(cudaMemcpyAsync(at(o_bkg), in->bkg, B * img, cudaMemcpyHostToDevice, sc));
-        if (in->x0) CU(cudaMemcpyAsync(at(o_x0), in->x0, B * img, cudaMemcpyHostToDevice, sc));
-        if (in->obj) CU(cudaMemcpyAsync(at(o_obj), in->obj, B * img, cudaMemcpyHostToDevice, sc));
+    // ---- copy stream: items [first, first + n) of every image-shaped input, then the flags that hand them to the kernel
+    auto upload = [&](size_t first, size_t n) -> int {
+        for (int k = 0; k < HostIO::X; ++k)
+            if (io.host[k] && io.image(k))
+                CU(cudaMemcpyAsync(S + io.off[k] + first * img, (const char*)io.host[k] + first * img, n * img, cudaMemcpyHostToDevice, sc));
         return BSGP_OK;
     };
-    int rc;
-    if (resident_first) {                                          // no per-item hand-over: everything resident first
-        rc = upload_all(); if (rc) return rc;
-        CU(cudaEventRecord(p->ev_copy, sc));
-        CU(cudaStreamWaitEvent(sr, p->ev_copy, 0));
-    }
-    // ---- copy stream: images in queue order, flags behind them
+    const bool per_item = !p->frame && (img >= 65536 || in->order == nullptr);
     auto feed = [&]() -> int {
-        if (!per_item) {
-            rc = upload_all(); if (rc) return rc;
+        if (resident_first) {                                      // no per-item hand-over: everything resident first
+            TRY(upload(0, B));
+            CU(cudaEventRecord(p->ev_copy, sc));
+            CU(cudaStreamWaitEvent(sr, p->ev_copy, 0));
+        } else if (!per_item) {
+            TRY(upload(0, B));
             CU(cudaMemcpyAsync(p->ready, p->ones_host, B * sizeof(int), cudaMemcpyHostToDevice, sc));
         } else {
-            // consecutive queue items that are also consecutive in memory travel as one copy of <= ~1 MB per array
+            // images in queue order, flags behind them; consecutive queue items that are also consecutive in memory
+            // travel as one copy of <= ~1 MB per array
             const size_t max_run = img >= ((size_t)1 << 20) ? 1 : (((size_t)1 << 20) / img);
-            int i0 = 0;
-            while (i0 < batch) {
+            for (int i0 = 0, n = 0; i0 < batch; i0 += n) {
                 const int first = in->order ? in->order[i0] : i0;
-                int n = 1;
-                while (i0 + n < batch && (size_t)n < max_run && (in->order ? in->order[i0 + n] : i0 + n) == first + n) ++n;
-                const size_t o = (size_t)first * img, nb = (size_t)n * img;
-                CU(cudaMemcpyAsync((char*)at(o_gn) + o, (const char*)in->gn + o, nb, cudaMemcpyHostToDevice, sc));
-                if (in->bkg_is_image) CU(cudaMemcpyAsync((char*)at(o_bkg) + o, (const char*)in->bkg + o, nb, cudaMemcpyHostToDevice, sc));
-                if (in->x0) CU(cudaMemcpyAsync((char*)at(o_x0) + o, (const char*)in->x0 + o, nb, cudaMemcpyHostToDevice, sc));
-                if (in->obj) CU(cudaMemcpyAsync((char*)at(o_obj) + o, (const char*)in->obj + o, nb, cudaMemcpyHostToDevice, sc));
+                for (n = 1; i0 + n < batch && (size_t)n < max_run && (in->order ? in->order[i0 + n] : i0 + n) == first + n;) ++n;
+                TRY(upload((size_t)first, (size_t)n));
                 CU(cudaMemcpyAsync(p->ready + i0, p->ones_host, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, sc));
-                i0 += n;
             }
         }
         return BSGP_OK;
     };
-    if (!resident_first) {
-        rc = feed();
-        if (rc) { cudaGetLastError(); cudaStreamSynchronize(sc); cudaStreamSynchronize(sr); return rc; }
-    }
+    rc = feed();
+    if (rc) { cudaGetLastError(); cudaStreamSynchronize(sc); cudaStreamSynchronize(sr); return rc; }
     // ---- run stream: the kernel.  Launched AFTER the copies are queued, so that a launch made synchronous by a tool
     // (ncu, compute-sanitizer, CUDA_LAUNCH_BLOCKING) cannot wait for flags that nobody has been asked to raise yet.
-    rc = solve_checked(p, prm, batch, &di, &dout, sr, resident_first ? nullptr : p->ready);
+    rc = io.launch(p, prm, batch, S, sr, resident_first ? nullptr : p->ready);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sr); return rc; }
     // ---- small outputs behind the kernel
-    auto down = [&](void* h, size_t o, size_t bytes) -> int { if (h && o != (size_t)-1) CU(cudaMemcpyAsync(h, S + o, bytes, cudaMemcpyDeviceToHost, sr)); return BSGP_OK; };
-    if (pin_mode & 1) TRY(down(out->x, o_xs, B * img));
-    TRY(down(out->iters, o_it, B * 4)); TRY(down(out->status, o_st, B * 4)); TRY(down(out->discr, o_di, B * tr * 8)); TRY(down(out->times, o_ti, B * tr * 8));
-    TRY(down(out->stop_value, o_sv, B * tr * 8)); TRY(down(out->err, o_er, B * (tr + 1) * 8)); TRY(down(out->beta_final, o_bf, B * 8));
-    TRY(down(out->proj_evals, o_pe, B * 4)); TRY(down(out->ls_trials, o_lt, B * 4)); TRY(down(out->scalars, o_sc, B * BSGP_NSCALARS * 8));
-    TRY(down(out->trace_alpha, o_ta, B * tr * 8)); TRY(down(out->trace_lambda, o_tl, B * tr * 8)); TRY(down(out->trace_beta, o_tb, B * tr * 8));
-    TRY(down(out->trace_trials, o_tt, B * tr * 4)); TRY(down(out->trace_evals, o_te, B * tr * 4));
+    TRY(io.copy_back(S, sr));
     // ---- join: the caller's stream continues after both private streams; results are complete when this returns
     CU(cudaEventRecord(p->ev_copy, sc));
     CU(cudaEventRecord(p->ev_run, sr));

@@ -10,6 +10,7 @@ application_sgp_star_stamps.py:56-105 and application_sgp_subdivisions.py:83-107
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 from dataclasses import dataclass
 
@@ -37,7 +38,7 @@ class Plan:
         check(lib().bsgp_plan_create(self.ny, self.nx, _DT[self.dtype], self.device, C.byref(self._h)))
         if cluster_size or threads:
             check(lib().bsgp_plan_configure(self._h, int(cluster_size), int(threads)))
-        self._psf_key = None
+        self._psf_keepalive = {}
 
     @property
     def handle(self):
@@ -66,31 +67,25 @@ class Plan:
 
     def set_psf(self, psf):
         """psf: numpy [ny,nx] / [n,ny,nx] or a CUDA tensor of the same shapes."""
-        if _is_tensor(psf):
-            t, n = self._image_tensor(psf, "psf")
-            check(lib().bsgp_set_psf(self._h, t.data_ptr(), n, _stream_ptr()))
-            self._psf_keepalive = t
-            return n
-        a = np.ascontiguousarray(psf, dtype=_NP[self.dtype])
-        n = 1 if a.ndim == 2 else a.shape[0]
-        if a.shape[-2:] != (self.ny, self.nx):
-            raise ValueError(f"PSF shape {a.shape[-2:]} must equal the image shape {(self.ny, self.nx)} "
-                             "(the reference's numpy A/AT closure has the same requirement, sgp.py:108-120)")
-        check(lib().bsgp_set_psf_host(self._h, a.ctypes.data, n))
-        return n
+        return self._set_psf(psf, adjoint=False)
 
     def set_psf_adjoint(self, psf):
         """Second kernel, used for A^T by the zero-padded operator (sgp.py:157); numpy or CUDA tensor, [ny,nx] / [n,ny,nx]."""
+        return self._set_psf(psf, adjoint=True)
+
+    def _set_psf(self, psf, adjoint):
+        L, name = lib(), "adjoint psf" if adjoint else "psf"
         if _is_tensor(psf):
-            t, n = self._image_tensor(psf, "adjoint psf")
-            check(lib().bsgp_set_psf_adjoint(self._h, t.data_ptr(), n, _stream_ptr()))
-            self._psf_adj_keepalive = t
+            t, n = self._image_tensor(psf, name)
+            check((L.bsgp_set_psf_adjoint if adjoint else L.bsgp_set_psf)(self._h, t.data_ptr(), n, _stream_ptr()))
+            self._psf_keepalive[adjoint] = t            # read by the library on the stream, after this call returns
             return n
         a = np.ascontiguousarray(psf, dtype=_NP[self.dtype])
         n = 1 if a.ndim == 2 else a.shape[0]
         if a.shape[-2:] != (self.ny, self.nx):
-            raise ValueError("adjoint kernel must be embedded in the plan's grid")
-        check(lib().bsgp_set_psf_adjoint_host(self._h, a.ctypes.data, n))
+            raise ValueError(f"{name} shape {a.shape[-2:]} must equal the image shape {(self.ny, self.nx)} "
+                             "(the reference's numpy A/AT closure has the same requirement, sgp.py:108-120)")
+        check((L.bsgp_set_psf_adjoint_host if adjoint else L.bsgp_set_psf_host)(self._h, a.ctypes.data, n))
         return n
 
     def apply_psf(self, x, adjoint=False):
@@ -213,8 +208,13 @@ class PaddedGeometry:
         self.region = (self.rows.start, self.rows.stop, self.cols.start, self.cols.stop)
 
     def embed(self, a, dtype):
-        """[B,ny,nx] -> [B,P,P], zeros in the padding."""
-        out = np.zeros(a.shape[:-2] + (self.P, self.P), dtype=dtype)
+        """[B,ny,nx] -> [B,P,P] of `dtype`, zeros in the padding: numpy in, numpy out; a tensor in, a tensor on its device out."""
+        shape = tuple(a.shape[:-2]) + (self.P, self.P)
+        if _is_tensor(a):
+            import torch
+            out = torch.zeros(shape, dtype=dtype, device=a.device)
+        else:
+            out = np.zeros(shape, dtype=dtype)
         out[..., self.rows, self.cols] = a
         return out
 
@@ -233,6 +233,94 @@ def _params(divergence, kw, has_flux):
     if unknown:
         raise TypeError(f"unexpected keyword argument(s): {sorted(unknown)}")
     return _capi.make_params(DIV_KL if divergence == "kl" else DIV_BETA, has_flux=has_flux, **kw)
+
+
+# The solve's outputs besides the restored images, in the order of struct bsgp_outputs: (field, shape for B images and
+# T = MAXIT + 1, dtype, present only with).  The trace_* arrays come back as BatchResult.trace under _TRACE_KEYS.
+_OUTPUTS = (
+    ("iters", lambda B, T: (B,), np.int32, None),
+    ("status", lambda B, T: (B,), np.int32, None),
+    ("discr", lambda B, T: (B, T), np.float64, None),
+    ("times", lambda B, T: (B, T), np.float64, None),
+    ("stop_value", lambda B, T: (B, T), np.float64, None),
+    ("err", lambda B, T: (B, T + 1), np.float64, "errflag"),
+    ("beta_final", lambda B, T: (B,), np.float64, None),
+    ("proj_evals", lambda B, T: (B,), np.int32, None),
+    ("ls_trials", lambda B, T: (B,), np.int32, None),
+    ("scalars", lambda B, T: (B, _capi.NSCALARS), np.float64, None),
+    ("trace_alpha", lambda B, T: (B, T), np.float64, "trace"),
+    ("trace_lambda", lambda B, T: (B, T), np.float64, "trace"),
+    ("trace_beta", lambda B, T: (B, T), np.float64, "trace"),
+    ("trace_trials", lambda B, T: (B, T), np.int32, "trace"),
+    ("trace_evals", lambda B, T: (B, T), np.int32, "trace"),
+)
+_TRACE_KEYS = {"trace_alpha": "alpha", "trace_lambda": "lam", "trace_beta": "beta", "trace_trials": "trials", "trace_evals": "evals"}
+
+
+def _ptr(a):
+    return None if a is None else (a.data_ptr() if _is_tensor(a) else a.ctypes.data)
+
+
+def _ndim(a):
+    return a.dim() if _is_tensor(a) else np.ndim(a)
+
+
+def _torch_dtype(dt):
+    import torch
+    return {np.dtype(np.float64): torch.float64, np.dtype(np.float32): torch.float32, np.dtype(np.int32): torch.int32}[np.dtype(dt)]
+
+
+def _host_vector(a, B, dtype):
+    """A scalar or [B] array -> contiguous numpy [B] of `dtype` (the numpy and pinned routes)."""
+    return np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=dtype).reshape(-1), (B,)))
+
+
+def _plan_for(plan, gn, dtype, device, same_device=False):
+    """The caller's plan, or the cached one for gn; it must fit gn's shape and dtype (and device, for device tensors)."""
+    if gn.ndim != 3:
+        raise ValueError("gn must be [batch, ny, nx]")
+    _, ny, nx = gn.shape
+    plan = plan or get_plan(ny, nx, dtype, device)
+    if (plan.ny, plan.nx, plan.dtype) != (ny, nx, dtype) or (same_device and plan.device != device):
+        raise ValueError(f"plan is for {plan.ny}x{plan.nx} {plan.dtype} images on cuda:{plan.device}, gn is {ny}x{nx} {dtype}")
+    return plan
+
+
+class _Args:
+    """The arguments of one solve, normalised the same way on every route: the parameters, the PSF on the plan, bkg (an
+    image stack, or one value per image), flux and betaParam per image, x0 / obj, and the outputs of _OUTPUTS.  The route
+    supplies `psf_arg` (the PSF as it hands it to the plan), `image(a, name)` (a [B,ny,nx] array converted and checked),
+    `vector(a, B, dtype)` (a scalar or [B] array as a contiguous [B] array of a numpy dtype) and `alloc(shape, dtype)`."""
+
+    def __init__(self, gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, *, psf_arg, image,
+                 vector, alloc):
+        B = self.B = gn.shape[0]
+        self.params = p = _params(divergence, kw, flux is not None)
+        if not psf_is_set and plan.set_psf(psf_arg(psf)) not in (1, B):
+            raise ValueError("psf must be one image or one per batch entry")
+        self.gn, self.bkg_img, self.trace = gn, int(_ndim(bkg) == 3), trace
+        self.bkg = image(bkg, "bkg") if self.bkg_img else vector(bkg, B, _NP[plan.dtype])
+        self.flux = None if flux is None else vector(flux, B, np.float64)
+        self.beta0 = vector(betaParam, B, np.float64)
+        self.x0 = None if x0 is None else image(x0, "x0")
+        self.obj = None if obj is None else image(obj, "obj")
+        if p.init_recon == 1 and self.x0 is None:
+            raise ValueError("init_recon=1 needs x0 (the sgp()/sgp_betaDiv() wrappers draw it with seed 42)")
+        present = {None: True, "errflag": bool(p.errflag), "trace": bool(trace)}
+        self.out = {f: alloc(shape(B, p.maxit + 1), dt) if present[when] else None for f, shape, dt, when in _OUTPUTS}
+
+    def structs(self, x, order):
+        """_capi.Inputs / _capi.Outputs for restored images `x` and the work-queue order (None: natural order).  The
+        structs hold raw addresses, so the order is kept here, with the other arrays, for as long as the arguments live."""
+        self.order = order
+        ci = _capi.Inputs(_ptr(self.gn), _ptr(self.bkg), self.bkg_img, _ptr(self.flux), _ptr(self.beta0), _ptr(self.x0),
+                          _ptr(self.obj), _ptr(order))
+        return ci, _capi.Outputs(_ptr(x), *(_ptr(a) for a in self.out.values()))
+
+    def result(self, x):
+        out = dict(self.out)
+        trace = {key: out.pop(f) for f, key in _TRACE_KEYS.items()}
+        return BatchResult(x=x, trace=trace if self.trace else None, **out)
 
 
 def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=None, obj=None, dtype="float64",
@@ -265,57 +353,7 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
     if _is_tensor(gn):                                    # pageable CPU tensor: the plain host path
         gn = gn.numpy()
         psf, bkg, flux, betaParam, x0, obj = (a.numpy() if _is_tensor(a) and not a.is_cuda else a for a in (psf, bkg, flux, betaParam, x0, obj))
-    npdt = _NP[dtype]
-    gn = np.ascontiguousarray(gn, dtype=npdt)
-    if gn.ndim != 3:
-        raise ValueError("gn must be [batch, ny, nx]")
-    B, ny, nx = gn.shape
-    p = _params(divergence, kw, flux is not None)
-    plan = plan or get_plan(ny, nx, dtype, device)
-    if not psf_is_set:
-        n_psf = plan.set_psf(psf)
-        if n_psf not in (1, B):
-            raise ValueError("psf must be one image or one per batch entry")
-    bkg = np.asarray(bkg, dtype=npdt)
-    if bkg.ndim == 3:
-        bkg_img, bkg_a = 1, np.ascontiguousarray(bkg)
-        if bkg_a.shape != gn.shape:
-            raise ValueError("bkg image stack must have the shape of gn")
-    else:
-        bkg_img, bkg_a = 0, np.ascontiguousarray(np.broadcast_to(bkg.reshape(-1), (B,)).astype(npdt))
-    fl = None if flux is None else np.ascontiguousarray(np.broadcast_to(np.asarray(flux, dtype=np.float64).reshape(-1), (B,)))
-    b0 = np.ascontiguousarray(np.broadcast_to(np.asarray(betaParam, dtype=np.float64).reshape(-1), (B,)))
-    x0a = None if x0 is None else np.ascontiguousarray(x0, dtype=npdt)
-    obja = None if obj is None else np.ascontiguousarray(obj, dtype=npdt)
-    for name, a in (("x0", x0a), ("obj", obja)):
-        if a is not None and a.shape != gn.shape:
-            raise ValueError(f"{name} has shape {a.shape}; expected the shape of gn {gn.shape}")
-    if (plan.ny, plan.nx) != (ny, nx) or plan.dtype != dtype:
-        raise ValueError(f"plan is for {plan.ny}x{plan.nx} {plan.dtype} images, gn is {ny}x{nx} {dtype}")
-    if p.init_recon == 1 and x0a is None:
-        raise ValueError("init_recon=1 needs x0 (the sgp()/sgp_betaDiv() wrappers draw it with seed 42)")
-    T = p.maxit + 1
-    out = dict(x=np.empty((B, ny, nx), npdt), iters=np.zeros(B, np.int32), status=np.zeros(B, np.int32),
-               discr=np.zeros((B, T)), times=np.zeros((B, T)), stop_value=np.zeros((B, T)),
-               err=np.zeros((B, T + 1)) if p.errflag else None, beta_final=np.zeros(B), proj_evals=np.zeros(B, np.int32),
-               ls_trials=np.zeros(B, np.int32), scalars=np.zeros((B, _capi.NSCALARS)))
-    tr = None
-    if trace:
-        tr = dict(alpha=np.zeros((B, T)), lam=np.zeros((B, T)), beta=np.zeros((B, T)), trials=np.zeros((B, T), np.int32),
-                  evals=np.zeros((B, T), np.int32))
-
-    def ptr(a):
-        return None if a is None else a.ctypes.data
-
-    order = _queue_order(divergence, b0)
-    ci = _capi.Inputs(ptr(gn), ptr(bkg_a), bkg_img, ptr(fl), ptr(b0), ptr(x0a), ptr(obja), ptr(order))
-    co = _capi.Outputs(ptr(out["x"]), ptr(out["iters"]), ptr(out["status"]), ptr(out["discr"]), ptr(out["times"]),
-                       ptr(out["stop_value"]), ptr(out["err"]), ptr(out["beta_final"]), ptr(out["proj_evals"]),
-                       ptr(out["ls_trials"]), ptr(out["scalars"]),
-                       ptr(tr["alpha"]) if tr else None, ptr(tr["lam"]) if tr else None, ptr(tr["beta"]) if tr else None,
-                       ptr(tr["trials"]) if tr else None, ptr(tr["evals"]) if tr else None)
-    check(lib().bsgp_solve_batch_host(plan.handle, C.byref(p), B, C.byref(ci), C.byref(co)))
-    return BatchResult(trace=tr, **out)
+    return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, kw)
 
 
 def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, kw):
@@ -341,36 +379,43 @@ def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtyp
     big, div_a = geo.kernel(psf_h, npdt)
     bigt, div_at = geo.kernel(np.conj(np.swapaxes(psf_h, -1, -2)), npdt)          # psf.conj().T, sgp.py:157
     extra = dict(region=geo.region, div_a=div_a, div_at=div_at, adjoint_second_psf=True)
-    if on_dev:
-        import torch
-        with torch.cuda.device(gn.device):
-            if plan.set_psf(torch.as_tensor(big, device=gn.device)) not in (1, B) or \
-                    plan.set_psf_adjoint(torch.as_tensor(bigt, device=gn.device)) not in (1, B):
-                raise ValueError("psf must be one kernel or one per batch entry")
-
-            def emb(t):
-                out = torch.zeros(t.shape[:-2] + (geo.P, geo.P), dtype=gn.dtype, device=gn.device)
-                out[..., geo.rows, geo.cols] = t
-                return out
-
-            bkg_p = emb(bkg) if (_is_tensor(bkg) and bkg.dim() == 3) else bkg
-            res = _solve_batch_device(emb(gn), None, bkg_p, divergence, flux, betaParam, None if x0 is None else emb(x0),
-                                      None if obj is None else emb(obj), trace, plan, True, dict(kw, **extra))
-            res.x = res.x[:, geo.rows, geo.cols].contiguous()
-        return res
-    if plan.set_psf(big) not in (1, B) or plan.set_psf_adjoint(bigt) not in (1, B):
-        raise ValueError("psf must be one kernel or one per batch entry")
-    bkg = np.asarray(bkg, dtype=npdt)
-    bkg_p = geo.embed(bkg, npdt) if bkg.ndim == 3 else bkg
-    res = solve_batch(geo.embed(gn, npdt), None, bkg_p, divergence=divergence, flux=flux, betaParam=betaParam,
-                      x0=None if x0 is None else geo.embed(np.asarray(x0, dtype=npdt), npdt),
-                      obj=None if obj is None else geo.embed(np.asarray(obj, dtype=npdt), npdt), dtype=dtype, device=device,
-                      trace=trace, plan=plan, psf_is_set=True, **extra, **kw)
-    res.x = np.ascontiguousarray(res.x[:, geo.rows, geo.cols])
+    dt = gn.dtype if on_dev else npdt
+    with torch.cuda.device(gn.device) if on_dev else contextlib.nullcontext():
+        if on_dev:
+            big, bigt = torch.as_tensor(big, device=gn.device), torch.as_tensor(bigt, device=gn.device)
+        if plan.set_psf(big) not in (1, B) or plan.set_psf_adjoint(bigt) not in (1, B):
+            raise ValueError("psf must be one kernel or one per batch entry")
+        res = solve_batch(geo.embed(gn, dt), None, geo.embed(bkg, dt) if _ndim(bkg) == 3 else bkg, divergence=divergence,
+                          flux=flux, betaParam=betaParam, x0=None if x0 is None else geo.embed(x0, dt),
+                          obj=None if obj is None else geo.embed(obj, dt), dtype=dtype, device=device, trace=trace, plan=plan,
+                          psf_is_set=True, **extra, **kw)
+    x = res.x[:, geo.rows, geo.cols]
+    res.x = x.contiguous() if on_dev else np.ascontiguousarray(x)
     return res
 
 
+def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, kw):
+    """numpy arrays -> numpy arrays; one call of bsgp_solve_batch_host."""
+    npdt = _NP[dtype]
+    gn = np.ascontiguousarray(gn, dtype=npdt)
+    plan = _plan_for(plan, gn, dtype, device)
+
+    def image(a, name):
+        a = np.ascontiguousarray(a, dtype=npdt)
+        if a.shape != gn.shape:
+            raise ValueError(f"{name} has shape {a.shape}; expected the shape of gn {gn.shape}")
+        return a
+
+    args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw,
+                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros)
+    x = np.empty(gn.shape, npdt)
+    ci, co = args.structs(x, _queue_order(divergence, args.beta0))
+    check(lib().bsgp_solve_batch_host(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co)))
+    return args.result(x)
+
+
 def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw):
+    """CUDA tensors -> CUDA tensors, asynchronous on the current stream: no host synchronisation, no host copies."""
     import torch
     if not gn.is_cuda:
         raise BsgpError("tensor inputs must live on a CUDA device (there is no CPU path)")
@@ -378,72 +423,38 @@ def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trac
     if gn.dtype not in (torch.float64, torch.float32):
         raise ValueError("gn must be float64 or float32")
     dtype = {torch.float64: "float64", torch.float32: "float32"}[gn.dtype]
-    if gn.dim() != 3:
-        raise ValueError("gn must be [batch, ny, nx]")
+    plan = _plan_for(plan, gn, dtype, dev.index or 0, same_device=True)
     gn = gn.contiguous()
-    B, ny, nx = gn.shape
-    p = _params(divergence, kw, flux is not None)
-    plan = plan or get_plan(ny, nx, dtype, dev.index or 0)
-    if (plan.ny, plan.nx) != (ny, nx) or plan.dtype != dtype or plan.device != (dev.index or 0):
-        raise ValueError(f"plan is for {plan.ny}x{plan.nx} {plan.dtype} images on cuda:{plan.device}, gn is {ny}x{nx} {dtype} on {dev}")
 
-    def image_stack(t, name):
+    def image(t, name):
         """[B,ny,nx] tensor of gn's dtype on gn's device (raw pointers go to the library: a short or foreign array would be read out of bounds)"""
-        if t is None:
-            return None
         if not _is_tensor(t):
             t = torch.as_tensor(np.ascontiguousarray(t), device=dev)
-        if t.device != dev or tuple(t.shape) != (B, ny, nx):
-            raise ValueError(f"{name} must have the shape {(B, ny, nx)} of gn and live on {dev}; got {tuple(t.shape)} on {t.device}")
+        if t.device != dev or tuple(t.shape) != tuple(gn.shape):
+            raise ValueError(f"{name} must have the shape {tuple(gn.shape)} of gn and live on {dev}; got {tuple(t.shape)} on {t.device}")
         return t.to(gn.dtype).contiguous()
 
+    def vector(a, B, dt):
+        t = (a if _is_tensor(a) else torch.as_tensor(np.asarray(a, dtype=np.float64), device=dev)).to(_torch_dtype(dt))
+        if t.device != dev:
+            raise ValueError(f"bkg, flux and betaParam must live on gn's device {dev}; got {t.device}")
+        return t.reshape(-1).expand(B).contiguous()
+
+    def psf_arg(a):
+        return a if _is_tensor(a) else torch.as_tensor(np.ascontiguousarray(a), dtype=gn.dtype, device=dev)
+
     with torch.cuda.device(dev):
-        if not psf_is_set:
-            n_psf = plan.set_psf(psf if _is_tensor(psf) else torch.as_tensor(np.ascontiguousarray(psf), dtype=gn.dtype, device=dev))
-            if n_psf not in (1, B):
-                raise ValueError("psf must be one image or one per batch entry")
-        if _is_tensor(bkg) and bkg.dim() == 3:
-            bkg_img, bkg_t = 1, image_stack(bkg, "bkg")
-        else:
-            bkg_img = 0
-            bkg_t = (bkg if _is_tensor(bkg) else torch.as_tensor(np.asarray(bkg, dtype=np.float64), device=dev)).to(gn.dtype).reshape(-1).expand(B).contiguous()
-        f64 = dict(dtype=torch.float64, device=dev)
-        fl = None if flux is None else (flux if _is_tensor(flux) else torch.as_tensor(np.asarray(flux, dtype=np.float64), device=dev)).to(torch.float64).reshape(-1).expand(B).contiguous()
-        b0 = (betaParam if _is_tensor(betaParam) else torch.as_tensor(np.asarray(betaParam, dtype=np.float64), device=dev)).to(torch.float64).reshape(-1).expand(B).contiguous()
-        x0t, objt = image_stack(x0, "x0"), image_stack(obj, "obj")
-        if p.init_recon == 1 and x0t is None:
-            raise ValueError("init_recon=1 needs x0 (the sgp()/sgp_betaDiv() wrappers draw it with seed 42)")
-        for name, t in (("bkg", bkg_t), ("flux", fl), ("betaParam", b0)):
-            if t is not None and t.device != dev:
-                raise ValueError(f"{name} lives on {t.device}, gn on {dev}")
-        T = p.maxit + 1
-        i32 = dict(dtype=torch.int32, device=dev)
-        out = dict(x=torch.empty_like(gn), iters=torch.zeros(B, **i32), status=torch.zeros(B, **i32),
-                   discr=torch.zeros(B, T, **f64), times=torch.zeros(B, T, **f64), stop_value=torch.zeros(B, T, **f64),
-                   err=torch.zeros(B, T + 1, **f64) if p.errflag else None, beta_final=torch.zeros(B, **f64),
-                   proj_evals=torch.zeros(B, **i32), ls_trials=torch.zeros(B, **i32),
-                   scalars=torch.zeros(B, _capi.NSCALARS, **f64))
-        tr = None
-        if trace:
-            tr = dict(alpha=torch.zeros(B, T, **f64), lam=torch.zeros(B, T, **f64), beta=torch.zeros(B, T, **f64),
-                      trials=torch.zeros(B, T, **i32), evals=torch.zeros(B, T, **i32))
-
-        def ptr(t):
-            return None if t is None else t.data_ptr()
-
+        args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
+                     image=image, vector=vector, alloc=lambda shape, dt: torch.zeros(shape, dtype=_torch_dtype(dt), device=dev))
+        x = torch.empty_like(gn)
         order = None
-        if divergence == "beta" and B > 1:
+        if divergence == "beta" and args.B > 1:
             # longest expected solve first (see _queue_order); computed on the device, no host sync
-            order = torch.argsort((b0 - 1.0).abs(), stable=True).to(torch.int32)
-        ci = _capi.Inputs(ptr(gn), ptr(bkg_t), bkg_img, ptr(fl), ptr(b0), ptr(x0t), ptr(objt), ptr(order))
-        co = _capi.Outputs(ptr(out["x"]), ptr(out["iters"]), ptr(out["status"]), ptr(out["discr"]), ptr(out["times"]),
-                           ptr(out["stop_value"]), ptr(out["err"]), ptr(out["beta_final"]), ptr(out["proj_evals"]),
-                           ptr(out["ls_trials"]), ptr(out["scalars"]),
-                           ptr(tr["alpha"]) if tr else None, ptr(tr["lam"]) if tr else None, ptr(tr["beta"]) if tr else None,
-                           ptr(tr["trials"]) if tr else None, ptr(tr["evals"]) if tr else None)
-        check(lib().bsgp_solve_batch(plan.handle, C.byref(p), B, C.byref(ci), C.byref(co), _stream_ptr()))
-        res = BatchResult(trace=tr, **out)
-        res._keepalive = (gn, bkg_t, fl, b0, x0t, objt, order)
+            order = torch.argsort((args.beta0 - 1.0).abs(), stable=True).to(torch.int32)
+        ci, co = args.structs(x, order)
+        check(lib().bsgp_solve_batch(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co), _stream_ptr()))
+        res = args.result(x)
+        res._keepalive = (gn, args.bkg, args.flux, args.beta0, args.x0, args.obj, args.order)
     return res
 
 
@@ -452,77 +463,37 @@ def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, devi
     are in host memory).  `device` selects the GPU.  Image-shaped arguments (bkg stack, x0, obj) must be pinned too."""
     import torch
     dtype = {torch.float64: "float64", torch.float32: "float32"}[gn.dtype]
-    npdt = _NP[dtype]
     gn = gn.contiguous()
-    if gn.dim() != 3:
-        raise ValueError("gn must be [batch, ny, nx]")
-    B, ny, nx = gn.shape
-    p = _params(divergence, kw, flux is not None)
-    plan = plan or get_plan(ny, nx, dtype, device)
-    if (plan.ny, plan.nx) != (ny, nx) or plan.dtype != dtype:
-        raise ValueError(f"plan is for {plan.ny}x{plan.nx} {plan.dtype} images, gn is {ny}x{nx} {dtype}")
+    plan = _plan_for(plan, gn, dtype, device)
+
+    def pinned(t, name):
+        if not (_is_tensor(t) and not t.is_cuda and t.is_pinned() and t.dtype == gn.dtype and tuple(t.shape) == tuple(gn.shape)):
+            raise ValueError(f"{name} must be a pinned CPU tensor of the shape and dtype of gn")
+        return t.contiguous()
+
+    def psf_arg(a):
+        return (a if _is_tensor(a) else torch.as_tensor(np.ascontiguousarray(a))).to(device=f"cuda:{plan.device}", dtype=gn.dtype, non_blocking=True)
+
+    # the small outputs are page-locked as well (torch's caching host allocator makes repeated calls cheap), handed
+    # back as numpy views: the copies behind the kernel run at full PCIe speed and never block on a staging buffer
+    def hbuf(shape, dt):
+        return torch.empty(shape, dtype=_torch_dtype(dt), pin_memory=True).numpy()
+
     with torch.cuda.device(plan.device):
-        if not psf_is_set:
-            psf_t = psf if _is_tensor(psf) else torch.as_tensor(np.ascontiguousarray(psf))
-            n_psf = plan.set_psf(psf_t.to(device=f"cuda:{plan.device}", dtype=gn.dtype, non_blocking=True))
-            if n_psf not in (1, B):
-                raise ValueError("psf must be one image or one per batch entry")
-
-        def pinned_image(t, name):
-            if t is None:
-                return None
-            if not (_is_tensor(t) and not t.is_cuda and t.is_pinned() and t.dtype == gn.dtype and tuple(t.shape) == tuple(gn.shape)):
-                raise ValueError(f"{name} must be a pinned CPU tensor of the shape and dtype of gn")
-            return t.contiguous()
-
-        if _is_tensor(bkg) and bkg.dim() == 3:
-            bkg_img, bkg_t = 1, pinned_image(bkg, "bkg")
-            bkg_ptr = bkg_t.data_ptr()
-        else:
-            bkg_img, bkg_t = 0, np.ascontiguousarray(np.broadcast_to(np.asarray(bkg, dtype=npdt).reshape(-1), (B,)).astype(npdt))
-            bkg_ptr = bkg_t.ctypes.data
-
-        def small(a):
-            return None if a is None else np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=np.float64).reshape(-1), (B,)))
-
-        fl, b0 = small(flux), small(betaParam)
-        x0t, objt = pinned_image(x0, "x0"), pinned_image(obj, "obj")
-        if p.init_recon == 1 and x0t is None:
-            raise ValueError("init_recon=1 needs x0 (the sgp()/sgp_betaDiv() wrappers draw it with seed 42)")
-        T = p.maxit + 1
+        args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
+                     image=pinned, vector=_host_vector, alloc=hbuf)
         if x_out is None:
-            x = torch.empty((B, ny, nx), dtype=gn.dtype, pin_memory=True)
+            x = torch.empty(tuple(gn.shape), dtype=gn.dtype, pin_memory=True)
         else:
             x = x_out
-            if not (_is_tensor(x) and not x.is_cuda and x.is_pinned() and x.dtype == gn.dtype and tuple(x.shape) == (B, ny, nx) and x.is_contiguous()):
+            if not (_is_tensor(x) and not x.is_cuda and x.is_pinned() and x.dtype == gn.dtype and x.shape == gn.shape and x.is_contiguous()):
                 raise ValueError("x_out must be a contiguous pinned CPU tensor of the shape and dtype of gn")
-
-        # the small outputs are page-locked as well (torch's caching host allocator makes repeated calls cheap), handed
-        # back as numpy views: the copies behind the kernel run at full PCIe speed and never block on a staging buffer
-        def hbuf(shape, dt=np.float64):
-            return torch.empty(shape, dtype=torch.float64 if dt is np.float64 else torch.int32, pin_memory=True).numpy()
-
-        out = dict(iters=hbuf(B, np.int32), status=hbuf(B, np.int32), discr=hbuf((B, T)), times=hbuf((B, T)),
-                   stop_value=hbuf((B, T)), err=hbuf((B, T + 1)) if p.errflag else None, beta_final=hbuf(B),
-                   proj_evals=hbuf(B, np.int32), ls_trials=hbuf(B, np.int32), scalars=hbuf((B, _capi.NSCALARS)))
-        tr = None
-        if trace:
-            tr = dict(alpha=hbuf((B, T)), lam=hbuf((B, T)), beta=hbuf((B, T)), trials=hbuf((B, T), np.int32), evals=hbuf((B, T), np.int32))
-
-        def ptr(a):
-            return None if a is None else (a.data_ptr() if _is_tensor(a) else a.ctypes.data)
-
-        order = _queue_order(divergence, b0)
-        ci = _capi.Inputs(gn.data_ptr(), bkg_ptr, bkg_img, ptr(fl), ptr(b0), ptr(x0t), ptr(objt), ptr(order))
-        co = _capi.Outputs(x.data_ptr(), ptr(out["iters"]), ptr(out["status"]), ptr(out["discr"]), ptr(out["times"]),
-                           ptr(out["stop_value"]), ptr(out["err"]), ptr(out["beta_final"]), ptr(out["proj_evals"]),
-                           ptr(out["ls_trials"]), ptr(out["scalars"]),
-                           ptr(tr["alpha"]) if tr else None, ptr(tr["lam"]) if tr else None, ptr(tr["beta"]) if tr else None,
-                           ptr(tr["trials"]) if tr else None, ptr(tr["evals"]) if tr else None)
-        check(lib().bsgp_solve_batch_pinned(plan.handle, C.byref(p), B, C.byref(ci), C.byref(co), _stream_ptr()))
-    for i in np.nonzero(out["status"] == _capi.ST_INPUT_TIMEOUT)[0]:      # skipped images: defined (zero) pixels, status says why
+        ci, co = args.structs(x, _queue_order(divergence, args.beta0))
+        check(lib().bsgp_solve_batch_pinned(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co), _stream_ptr()))
+    res = args.result(x)
+    for i in np.nonzero(res.status == _capi.ST_INPUT_TIMEOUT)[0]:      # skipped images: defined (zero) pixels, status says why
         x[int(i)].zero_()
-    return BatchResult(x=x, trace=tr, **out)
+    return res
 
 
 def project_batch(b, c, dia, sat_cap=None, lambda_=0.0, dlambda_=1.0, tol_lam=1e-11, max_projs=1000, biter=0, siter=0, device=0):

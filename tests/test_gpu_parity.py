@@ -674,6 +674,37 @@ def test_pipelined_pinned_path_matches_numpy_path(bs, fixtures, golden):
     assert np.array_equal(pa.x, pb.x)
 
 
+def test_host_entry_rejects_queue_order_out_of_range(bs):
+    """bsgp_solve_batch_host checks the caller's queue order before it stages anything: the kernel indexes the images with
+    it, so an entry outside 0..batch-1 is BSGP_E_ARG and no kernel runs.  A permutation runs."""
+    import ctypes as C
+    capi, L = bs._capi, bs._capi.lib()
+    B, n = 4, 32
+    gn = np.random.default_rng(0).poisson(100.0, (B, n, n)).astype(np.float64)
+    psf = bs.synth.moffat_psf(n, n, 2.0)
+    plan = bs.Plan(n, n)
+    plan.set_psf(psf / psf.sum())
+    prm = capi.make_params(capi.DIV_KL, MAXIT=3, verbose=False)
+    bkg = np.full(B, 10.0)
+    x, iters, status, discr, times = np.zeros_like(gn), np.zeros(B, np.int32), np.zeros(B, np.int32), np.zeros((B, 4)), np.zeros((B, 4))
+    co = capi.Outputs(x.ctypes.data, iters.ctypes.data, status.ctypes.data, discr.ctypes.data, times.ctypes.data)
+
+    def solve(order):
+        o = np.array(order, np.int32)
+        ci = capi.Inputs(gn.ctypes.data, bkg.ctypes.data, 0, None, None, None, None, o.ctypes.data)
+        return L.bsgp_solve_batch_host(plan.handle, C.byref(prm), B, C.byref(ci), C.byref(co))
+
+    for order in ([0, 1, 2, B], [3, 2, -1, 0], [0, 1, 2, 1 << 30]):
+        n0 = L.bsgp_launch_count()
+        assert solve(order) == 1                                      # BSGP_E_ARG
+        assert L.bsgp_launch_count() == n0 and b"order" in L.bsgp_last_error_string()
+    assert not x.any() and not iters.any()
+    assert solve([3, 2, 1, 0]) == 0 and np.all(status == 0)
+    r = bs.solve_batch(gn, psf / psf.sum(), bkg, divergence="kl", MAXIT=3, verbose=False, plan=plan)     # natural order
+    assert np.array_equal(r.x, x) and np.array_equal(r.iters, iters) and np.array_equal(r.discr, discr)
+    plan.close()
+
+
 def test_tiling_extract_assemble_and_frame_restoration(bs, fixtures, golden):
     """SURVEY §8(f) rank 3: tiles cut on the device equal numpy slices of the reference's boxes (bit-exact); re-assembly is
     the documented cross-fade (checked against a numpy restatement; identity on consistent tiles); a frame made of four

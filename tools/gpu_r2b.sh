@@ -1,5 +1,5 @@
 #!/bin/bash
-# round 2, second GPU session: parity suite, the new bench (with the workloads key), width probe with 2 CTAs x 256 threads
+# round 2, second GPU session: parity suite, the new bench (with the workloads key), fp32 errors against the golden images
 mkdir -p gpurun_out
 python -m pytest tests -m gpu -q -x > gpurun_out/pytest_gpu_r2b.log 2>&1; echo "pytest rc=$?" | tee -a gpurun_out/pytest_gpu_r2b.log
 tail -8 gpurun_out/pytest_gpu_r2b.log
@@ -12,27 +12,6 @@ print("main", round(d["value"],1), "e2e", round(d["e2e"]["value"],1), "frac", ro
 for k, v in d.get("workloads", {}).items():
     if "error" in v: print(k, v); continue
     print(k, "value", round(v["value"],2), "ms/step", round(v["ms_per_step"],3), "ms/it(longest)", round(v["ms_per_iteration_longest_solve"],4), "frac", round(v["roofline"]["frac"],3), "e2e", round(v["e2e"]["value"],2), "cpu", v.get("cpu_baseline",{}).get("value"), "cfg", v["cluster_size"], v["threads"])
-PY
-BSGP_MINB=2 timeout 300 python - <<PY
-import sys, os, json, numpy as np, torch
-sys.path.insert(0, os.getcwd())
-import beta_sgp_b200 as bs
-dev = torch.device("cuda", 0)
-w = bs.synth.field_tiles(size=2048, tile=256, seed=2024, n_beta=5); kw = dict(bs.synth.TILE_KWARGS)
-order = np.argsort(np.abs(w["beta0"] - 1.0), kind="stable")
-for (G, th) in ((0, 256), (16, 256)):
-    plan = bs.Plan(256, 256, "float64", 0, cluster_size=G, threads=th); info = plan.info()
-    for B in (8, 20, 40, 80, 160):
-        idx = np.sort(order[:: max(1, len(order) // B)][:B])
-        t = {k: torch.as_tensor(np.ascontiguousarray(w[k][idx] if k != "psf" else w[k]), device=dev) for k in ("gn", "psf", "bkg", "flux", "beta0")}
-        plan.set_psf(t["psf"])
-        for rep in range(3):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            r = bs.solve_batch(t["gn"], None, t["bkg"], divergence="beta", flux=t["flux"], betaParam=t["beta0"], plan=plan, psf_is_set=True, **kw)
-            e1.record(); torch.cuda.synchronize()
-        print("MINB=2", json.dumps(dict(G=info["cluster_size"], threads=info["threads"], slots=info["num_clusters"], B=B, ms=round(e0.elapsed_time(e1), 3), max_it=int(r.iters.max()))), flush=True)
-    plan.close()
 PY
 python - <<PY
 # fp32 mode: actual errors against the fp64 golden images
