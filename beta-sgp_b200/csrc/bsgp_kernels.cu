@@ -523,8 +523,11 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
     // B200, 320 solves of 256x256: 1 x 512 threads 112 ms, 2 x 256 threads 94 ms, 4 x 128 threads 87 ms).
     //   big slabs   : 4 CTAs x 128 threads, 38 KB FFT workspace, per-image state in L2 / HBM
     //   small slabs : (stamps) 2 CTAs x 256 threads, everything resident in shared memory
+    // The small-slab launch shapes compile DeviceCtxSmall, whose all-reduce (allreduce_sum8) sums over ONE CTA: a cluster of
+    // several CTAs takes the large-slab shapes whatever its slab size (with DeviceCtxSmall its CTAs would each see their
+    // own partial sums, take different control paths and never meet at the next cluster barrier).
     const size_t nslab = npix / G;
-    const bool small_slab = nslab * sizeof(T) <= 16384;
+    const bool small_slab = G == 1 && nslab * sizeof(T) <= 16384;
     int threads = p->want_threads;
     if (threads <= 0) threads = small_slab ? (p->small_try ? 128 : 256) : 128;
     if (threads != 256 && threads != 512 && threads != 128) return fail(BSGP_E_ARG, "threads must be 128, 256 or 512");

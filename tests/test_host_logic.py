@@ -93,6 +93,43 @@ def test_emulated_cluster_convolution(ny, nx, G, ws):
             assert np.abs(y - ref).max() <= 5e-15 * np.abs(ref).max()
 
 
+def _tile_split(ny, nx, G, ws, elem):
+    """(row tile pairs, column tile) of make_geom (csrc/bsgp_plan.h) for complex elements of `elem` bytes."""
+    def plen(n):
+        return n + (n >> 3)                               # the last radix stage is 8 for every side >= 16
+    rtp, ct = ny // G // 2, nx // 2 // G
+    while rtp > 1 and rtp * plen(nx) * elem > ws:
+        rtp >>= 1
+    while ct > 1 and ct * (plen(ny) | 1) * elem > ws:
+        ct >>= 1
+    return rtp, ct
+
+
+@pytest.mark.parametrize("ny,nx,G,ws", [(32, 32, 1, 1 << 20), (32, 32, 2, 1 << 20), (64, 64, 4, 1 << 20), (256, 256, 8, 72 * 1024),
+                                        (256, 256, 16, 72 * 1024), (128, 512, 8, 40 * 1024), (512, 128, 2, 72 * 1024), (64, 32, 2, 4096),
+                                        (256, 256, 2, 36 * 1024)])
+def test_emulated_cluster_convolution_f32(ny, nx, G, ws):
+    """The fp32 sibling of test_emulated_cluster_convolution: make_geom sizes the tiles with sizeof(cplx<float>), so fp32
+    runs row / column tile partitions that fp64 never runs (the last case: 16 row-tile pairs and 8 columns per tile in fp32
+    against 8 and 4 in fp64).  Against numpy in fp64 on the same fp32 values, within 2^-23 * log2(ny * nx) of the
+    largest value (the bar of the device's fp32 operator, tests/test_gpu_variants.py)."""
+    if (ny, nx, G, ws) == (256, 256, 2, 36 * 1024):
+        assert _tile_split(ny, nx, G, ws, 8) != _tile_split(ny, nx, G, ws, 16)
+    L = eh.lib()
+    F = C.POINTER(C.c_float)
+    L.emul_conv_f32.argtypes = [C.c_int] * 3 + [C.c_longlong, F, F, C.c_int, F]
+    rng = np.random.default_rng(ny * 1000 + nx + G)
+    x = rng.normal(size=(ny, nx)).astype(np.float32)
+    psf = rng.random((ny, nx))
+    psf = (psf / psf.sum()).astype(np.float32)
+    tf = np.fft.fftn(np.fft.fftshift(psf.astype(np.float64)))
+    for adjoint in (0, 1):
+        y = np.zeros((ny, nx), np.float32)
+        assert L.emul_conv_f32(ny, nx, G, ws, x.ctypes.data_as(F), psf.ctypes.data_as(F), adjoint, y.ctypes.data_as(F)) == 0
+        ref = np.real(np.fft.ifftn((np.conj(tf) if adjoint else tf) * np.fft.fftn(x.astype(np.float64))))
+        assert np.abs(y - ref).max() <= 2.0 ** -23 * np.log2(ny * nx) * np.abs(ref).max()
+
+
 def test_emulated_projection_known_answers(golden):
     for i in range(12):
         k = f"proj{i:02d}"
