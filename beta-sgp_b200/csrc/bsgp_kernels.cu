@@ -48,24 +48,23 @@ template <typename T> struct ConvArgs {
 
 // mode CONV_MAKE_TF: tf[p] = fftn(fftshift(psf[p])) in workspace order (sgp.py:109); otherwise
 // out[i] = A(in[i]) or A^T(in[i]) (sgp.py:111-120).  Dynamic shared memory: [SharedCtl][ConvGeom][position table][workspace].
-template <typename T>
-__global__ void __launch_bounds__(512, 1) bsgp_conv_kernel(const ConvArgs<T> a, const unsigned off_geom, const unsigned off_ppx, const unsigned off_ws) {
+// `cluster_id` selects this cluster's exchange buffer; next() hands out the items.
+template <typename T, class Ctx, class Next>
+__device__ __forceinline__ void conv_items(Ctx& ctx, const ConvArgs<T>& a, const unsigned off_geom, const unsigned off_ppx, const unsigned off_ws,
+                                           const int cluster_id, Next next) {
     unsigned char* smem = dyn_smem();
-    DeviceCtx ctx = make_ctx(reinterpret_cast<SharedCtl*>(smem), a.g.G);
     ConvGeom* gs = reinterpret_cast<ConvGeom*>(smem + off_geom);
     unsigned short* ppx = reinterpret_cast<unsigned short*>(smem + off_ppx);
     if (ctx.tid == 0) *gs = a.g;
     fill_pos_table(ctx, a.g.px, ppx);
     __syncthreads();
     const ConvGeom& g = *gs;
-    const int cluster_id = blockIdx.x / a.g.G;
     const int ny = a.g.ny, nx = a.g.nx;
     const size_t npix = (size_t)ny * nx;
     cplx<T>* spec = a.spec + (size_t)cluster_id * a.spec_stride;
     const int r0 = ctx.rank * a.g.rows_per_cta;
     for (;;) {
-        bool ready_ok;
-        const int img = next_item(ctx, a.queue, nullptr, a.count, &ready_ok);
+        const int img = next();
         if (img >= a.count) break;
         const T* src = a.in + (size_t)img * npix;
         if (a.mode == CONV_MAKE_TF) {
@@ -97,50 +96,22 @@ __global__ void __launch_bounds__(512, 1) bsgp_conv_kernel(const ConvArgs<T> a, 
     }
 }
 
-// Frame-mode twin of bsgp_conv_kernel: every item is processed by the whole (cooperative) grid.
+// one cluster per item, from the work queue
+template <typename T>
+__global__ void __launch_bounds__(512, 1) bsgp_conv_kernel(const ConvArgs<T> a, const unsigned off_geom, const unsigned off_ppx, const unsigned off_ws) {
+    DeviceCtx ctx = make_ctx(reinterpret_cast<SharedCtl*>(dyn_smem()), a.g.G);
+    conv_items(ctx, a, off_geom, off_ppx, off_ws, blockIdx.x / a.g.G, [&] {
+        bool ready_ok;
+        return next_item(ctx, a.queue, nullptr, a.count, &ready_ok);
+    });
+}
+
+// frame mode: every item, one after the other, by the whole (cooperative) grid
 template <typename T>
 __global__ void __launch_bounds__(512, 1) bsgp_conv_frame_kernel(const ConvArgs<T> a, const unsigned off_geom, const unsigned off_ppx, const unsigned off_ws,
                                                                  double* gpart) {
-    unsigned char* smem = dyn_smem();
-    GridCtx ctx = make_grid_ctx(reinterpret_cast<SharedCtl*>(smem), gpart);
-    ConvGeom* gs = reinterpret_cast<ConvGeom*>(smem + off_geom);
-    unsigned short* ppx = reinterpret_cast<unsigned short*>(smem + off_ppx);
-    if (ctx.tid == 0) *gs = a.g;
-    fill_pos_table(ctx, a.g.px, ppx);
-    __syncthreads();
-    const ConvGeom& g = *gs;
-    const int ny = a.g.ny, nx = a.g.nx;
-    const size_t npix = (size_t)ny * nx;
-    const int r0 = ctx.rank * a.g.rows_per_cta;
-    for (int img = 0; img < a.count; ++img) {
-        const T* src = a.in + (size_t)img * npix;
-        if (a.mode == CONV_MAKE_TF) {
-            const int lg_nx = a.g.lg_nx;
-            auto pf = [&](int i) {
-                const int row = i >> lg_nx, c = i & (nx - 1);
-                In1<T> r; r.a = ld2(src + (size_t)((r0 + row + (ny >> 1)) & (ny - 1)) * nx, (c + (nx >> 1)) & (nx - 1)); return r;
-            };
-            auto pe = [&](int, const In1<T>& in) -> V2<T> { return in.a; };
-            ctx.sync();
-            conv_rows_forward<2, true>(ctx, g, off_ws, a.twx, kNoSmem, 0, off_ppx, a.spec, pf, pe);
-            ctx.cluster_sync();
-            conv_cols<true>(ctx, gs, off_ws, a.twy, kNoSmem, 0, a.spec, a.tf + (size_t)img * a.tf_stride, CONV_MAKE_TF);
-        } else {
-            T* dst = a.out + (size_t)img * npix + (size_t)r0 * nx;
-            const T* s0 = src + (size_t)r0 * nx;
-            auto pf = [&](int i) { In1<T> r; r.a = ld2(s0, i); return r; };
-            auto pe = [&](int, const In1<T>& in) -> V2<T> { return in.a; };
-            auto cf = [&](int) { In1<T> r; r.a = mk2((T)0, (T)0); return r; };
-            auto ca = [&](int i, const In1<T>&, V2<T> v) { st2(dst, i, v); };
-            ctx.sync();
-            conv_rows_forward<2, true>(ctx, g, off_ws, a.twx, kNoSmem, 0, off_ppx, a.spec, pf, pe);
-            ctx.cluster_sync();
-            conv_cols<true>(ctx, gs, off_ws, a.twy, kNoSmem, 0, a.spec, a.tf + (a.n_psf > 1 ? (size_t)img * a.tf_stride : 0), a.mode);
-            ctx.cluster_sync();
-            conv_rows_inverse<2, true>(ctx, g, off_ws, a.twx, kNoSmem, 0, off_ppx, a.spec, cf, ca);
-        }
-        ctx.cluster_sync();   // spec is reused by the next item
-    }
+    GridCtx ctx = make_grid_ctx(reinterpret_cast<SharedCtl*>(dyn_smem()), gpart);
+    conv_items(ctx, a, off_geom, off_ppx, off_ws, 0, [img = 0]() mutable { return img++; });
 }
 
 // projectDF (flux_conserve_proj.py:7-144): one CTA per problem, x = clamp((c + lambda) / dia).
@@ -373,7 +344,8 @@ static int fail(int code, const char* fmt, ...) {
         if (e__ != cudaSuccess) return fail(BSGP_E_CUDA, "%s failed: %s", #expr, cudaGetErrorString(e__)); \
     } while (0)
 
-struct bsgp_plan {
+// a plan is its launch shape (bsgp_plan.h, plan_launch) and the device state that goes with it
+struct bsgp_plan : LaunchPlan {
     int ny = 0, nx = 0, dtype = 0, device = 0;   // ny, nx: the power-of-two FFT grid the kernels work on
     int img_ny = 0, img_nx = 0;                   // the caller's image shape (== grid unless the plan is wrapped)
     bool embedded = false;                        // wrapped plan: user arrays are moved to / from the grid by the library
@@ -383,19 +355,14 @@ struct bsgp_plan {
     int num_sms = 0, max_smem = 0, smem_per_sm = 0;
     int want_G = 0, want_threads = 0;
     bool configured = false;
-    bool small_try = true;       // automatic configuration of small slabs: try 3 CTAs x 128 threads first (plan_setup_t)
-    ConvGeom g{};
-    size_t ws_bytes = 0, smem_bytes = 0, conv_smem = 0, elem = 8;
-    SmemPlan sp{};
-    unsigned conv_off_geom = 0, conv_off_ppx = 0, conv_off_ws = 0;
-    int threads = 0, minb = 1, num_clusters = 0, conv_clusters = 0, resident_mask = 0;
+    size_t elem = 8;
+    int num_clusters = 0, conv_clusters = 0;
     void* twx = nullptr; void* twy = nullptr;
     void* tf = nullptr; int n_psf = 0; int tf_capacity = 0; size_t tf_stride = 0;
     void* tf_adj = nullptr; int n_psf_adj = 0; int tf_adj_capacity = 0;   // spectra of the second (adjoint) kernel
     void* work = nullptr; size_t work_stride = 0;
     void* spec = nullptr; size_t spec_stride = 0;
     int* queue = nullptr;
-    bool frame = false;          // one image over the whole grid (cooperative launch) instead of one per cluster
     double* gpart = nullptr;     // frame mode: all-reduce partials [2][G][kMaxK]
     size_t workspace_bytes = 0;
     // pipelined host path (bsgp_solve_batch_pinned): grow-only device staging, ready flags, two private streams
@@ -425,13 +392,6 @@ static void plan_free_buffers(bsgp_plan* p) {
     p->tf_capacity = 0; p->n_psf = 0; p->tf_adj = nullptr; p->tf_adj_capacity = 0; p->n_psf_adj = 0;
 }
 
-static inline size_t up128(size_t v) { return (v + 127) & ~(size_t)127; }
-static inline size_t tw_table_entries(int mode, int n) { return mode == 0 ? 0 : (mode == 1 ? (size_t)n : (size_t)64 + (size_t)(n >> 6)); }
-
-// Residency priority: the two projection buffers (read E times per iteration), then the arrays with
-// the most touches per iteration; the background image last (unused when the background is a scalar).
-static const int kResidencyOrder[NBUF] = {B_D, B_T1, B_G, B_X, B_XTF, B_DTF, B_GN, B_BKG};
-
 template <typename T> static const void* conv_frame_kernel_ptr() { return (const void*)bsgp_conv_frame_kernel<T>; }
 
 template <typename T> static int alloc_tables(bsgp_plan* p) {
@@ -445,176 +405,50 @@ template <typename T> static int alloc_tables(bsgp_plan* p) {
     return BSGP_OK;
 }
 
-template <typename T> static int plan_setup_frame(bsgp_plan* p) {
-    const size_t npix = (size_t)p->ny * p->nx;
-    p->elem = sizeof(T);
-    int G = 1;
-    while (2 * G <= p->num_sms && p->ny % (4 * G) == 0 && (p->nx / 2) % (2 * G) == 0) G *= 2;
-    const size_t ws_limit = 160 * 1024;
-    if (!make_geom(p->ny, p->nx, G, sizeof(cplx<T>), ws_limit, &p->g, &p->ws_bytes))
-        return fail(BSGP_E_SHAPE, "unsupported shape %dx%d for frame mode (grid of %d CTAs)", p->ny, p->nx, G);
-    p->threads = 512; p->minb = 1; p->resident_mask = 0; p->num_clusters = 1; p->conv_clusters = 1;
-    // Panel width of the exchange buffer (bsgp_conv.cuh, spec_idx).  A column tile narrower than the panel reads 16 bytes of
-    // every 32-byte sector per sweep; with panels of max(col_tile, 4) columns the sectors one sweep fetches are the ones
-    // the next column's sweep needs, and they are still in L2 (4-column panel x 8192 rows x 128 CTAs = 64 MB), so the
-    // column pass reads the buffer once from DRAM instead of twice (8192^2: 121.5 -> 103.4 ms per 10 iterations).
-    {
-        const int want = p->g.lg_col_tile > 2 ? p->g.lg_col_tile : 2;
-        if (want < p->g.lg_cp) p->g.lg_cp = want;
-    }
-    SmemPlan sp;
-    size_t off = up128(sizeof(SharedCtl));
-    sp.off_state = (unsigned)off; off = up128(off + sizeof(ImgState<T>));
-    sp.ctl_stride = (unsigned)((sizeof(CtlState<T>) + 15) & ~(size_t)15);
-    sp.off_ctl = (unsigned)off; off = up128(off + (size_t)(p->threads / 32) * sp.ctl_stride);
-    const size_t tw_bytes = ((size_t)p->nx + (p->ny != p->nx ? p->ny : 0)) * sizeof(cplx<T>);
-    sp.tw_smem = tw_bytes <= 16384 ? 1 : 2;             // long transforms: two-level tables (64 + n/64 entries)
-    sp.off_twx = sp.off_twy = (unsigned)off;
-    off = up128(off + tw_table_entries(sp.tw_smem, p->nx) * sizeof(cplx<T>));
-    if (p->ny != p->nx) { sp.off_twy = (unsigned)off; off = up128(off + tw_table_entries(sp.tw_smem, p->ny) * sizeof(cplx<T>)); }
-    sp.off_ppx = (unsigned)off; off = up128(off + (size_t)p->nx * sizeof(unsigned short));
-    sp.off_ws = (unsigned)off; off = up128(off + p->ws_bytes);
-    sp.off_bufs = (unsigned)off;
-    p->sp = sp;
-    p->smem_bytes = off;
-    p->conv_off_geom = (unsigned)up128(sizeof(SharedCtl));
-    p->conv_off_ppx = (unsigned)up128(p->conv_off_geom + sizeof(ConvGeom));
-    p->conv_off_ws = (unsigned)up128(p->conv_off_ppx + (size_t)p->nx * sizeof(unsigned short));
-    p->conv_smem = p->conv_off_ws + up128(p->ws_bytes);
-    if (p->smem_bytes > (size_t)p->max_smem || p->conv_smem > (size_t)p->max_smem)
-        return fail(BSGP_E_SHAPE, "shape %dx%d needs %zu B of shared memory per CTA (limit %d)", p->ny, p->nx, p->smem_bytes, p->max_smem);
-    int coop = 0;
-    CU(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, p->device));
-    if (!coop) return fail(BSGP_E_CUDA, "device does not support cooperative launches (frame mode)");
-    LaunchCfg lc{G, 512, 1, p->smem_bytes, nullptr, 1};
-    int per_sm = 0;
-    cudaError_t e = query_frame_ctas<T, false>(lc, &per_sm);
-    if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
-    if (per_sm < 1) return fail(BSGP_E_CUDA, "frame kernel does not fit: %zu B shared memory", p->smem_bytes);
-    CU(cudaFuncSetAttribute(conv_frame_kernel_ptr<T>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
-    int rc = alloc_tables<T>(p);
-    if (rc) return rc;
-    p->work_stride = NBUF * npix;
-    p->spec_stride = (size_t)p->ny * p->g.hx;
-    p->tf_stride = (size_t)(p->g.hx + 1) * p->ny;
-    CU(cudaMalloc(&p->work, p->work_stride * sizeof(T)));
-    CU(cudaMalloc(&p->spec, p->spec_stride * sizeof(cplx<T>)));
-    CU(cudaMalloc((void**)&p->queue, sizeof(int)));
-    CU(cudaMalloc((void**)&p->gpart, (size_t)2 * G * kMaxK * sizeof(double)));
-    p->workspace_bytes = p->work_stride * sizeof(T) + p->spec_stride * sizeof(cplx<T>);
-    p->configured = true;
-    return BSGP_OK;
-}
-
+// The launch shape (plan_launch), how many clusters of it fit the device, and the plan's device buffers.  A frame plan
+// is one "cluster" of G CTAs for both kernels.
 template <typename T> static int plan_setup_t(bsgp_plan* p) {
-    const size_t npix = (size_t)p->ny * p->nx;
+    const PlanRequest q{p->ny, p->nx, p->img_ny, p->img_nx, p->want_G, p->want_threads, p->num_sms, p->max_smem, p->smem_per_sm};
+    LaunchPlan L;
+    char err[256];
+    const int code = plan_launch<T>(q, &L, err, sizeof err);
+    if (code) return fail(code, "%s", err);
+    static_cast<LaunchPlan&>(*p) = L;
     p->elem = sizeof(T);
-    // Frame mode (bsgp_device.cuh, GridCtx): images of a megapixel or more get the whole GPU each
-    p->frame = (p->want_G == -1) || (p->want_G == 0 && npix >= ((size_t)1 << 20));
-    if (p->frame) return plan_setup_frame<T>(p);
-    // cluster size: slabs of <= 64 KB, at most 8 CTAs (portable cluster limit)
-    int G = p->want_G;
-    if (G <= 0) {
-        G = 1;
-        while (G < 8 && npix * sizeof(T) / G > 65536 && p->ny % (4 * G) == 0 && (p->nx / 2) % (2 * G) == 0) G *= 2;
+    const int G = p->g.G;
+    if (p->frame) {
+        int coop = 0;
+        CU(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, p->device));
+        if (!coop) return fail(BSGP_E_CUDA, "device does not support cooperative launches (frame mode)");
+        LaunchCfg lc{G, 512, 1, p->smem_bytes, nullptr, 1};
+        int per_sm = 0;
+        cudaError_t e = query_frame_ctas<T, false>(lc, &per_sm);
+        if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
+        if (per_sm < 1) return fail(BSGP_E_CUDA, "frame kernel does not fit: %zu B shared memory", p->smem_bytes);
+        CU(cudaFuncSetAttribute(conv_frame_kernel_ptr<T>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
+        p->num_clusters = p->conv_clusters = 1;
+    } else {
+        LaunchCfg lc{G * p->num_sms, p->threads, G, p->smem_bytes, nullptr, p->minb};
+        int nc = 0;
+        cudaError_t e = query_solve_clusters<T, false>(lc, p->num_sms, &nc);
+        if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
+        if (nc <= 0) return fail(BSGP_E_CUDA, "kernel does not fit: cluster %d, %d threads, %zu B shared memory", G, p->threads, p->smem_bytes);
+        p->num_clusters = nc;
+        LaunchCfg cc{G * p->num_sms, 512, G, p->conv_smem, nullptr};
+        e = query_clusters(conv_kernel_ptr<T>(), cc, p->num_sms, &nc);
+        if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
+        if (nc <= 0) return fail(BSGP_E_CUDA, "convolution kernel does not fit: cluster %d, %zu B shared memory", G, p->conv_smem);
+        p->conv_clusters = nc;
     }
-    // Threads and CTAs per SM.  The solve is a chain of short phases separated by reductions, so one CTA leaves
-    // the SM idle while it waits; several small CTAs of DIFFERENT images per SM fill those gaps (measured on
-    // B200, 320 solves of 256x256: 1 x 512 threads 112 ms, 2 x 256 threads 94 ms, 4 x 128 threads 87 ms).
-    //   big slabs   : 4 CTAs x 128 threads, 38 KB FFT workspace, per-image state in L2 / HBM
-    //   small slabs : (stamps) 2 CTAs x 256 threads, everything resident in shared memory
-    // The small-slab launch shapes compile DeviceCtxSmall, whose all-reduce (allreduce_sum8) sums over ONE CTA: a cluster of
-    // several CTAs takes the large-slab shapes whatever its slab size (with DeviceCtxSmall its CTAs would each see their
-    // own partial sums, take different control paths and never meet at the next cluster barrier).
-    const size_t nslab = npix / G;
-    const bool small_slab = G == 1 && nslab * sizeof(T) <= 16384;
-    int threads = p->want_threads;
-    if (threads <= 0) threads = small_slab ? (p->small_try ? 128 : 256) : 128;
-    if (threads != 256 && threads != 512 && threads != 128) return fail(BSGP_E_ARG, "threads must be 128, 256 or 512");
-    int minb = threads >= 512 ? 1 : (threads >= 256 ? (small_slab ? 2 : 1) : (small_slab ? 3 : 4));
-    size_t ws_limit = (minb >= 4 ? 38 : 76) * 1024;
-    // short sides that are not a power of two: dense DFT of the image's own length on the first slots of the grid (bsgp_wrap.h)
-    const int dny = p->ny != p->img_ny ? dense_len(p->img_ny) : 0, dnx = p->nx != p->img_nx ? dense_len(p->img_nx) : 0;
-    bool ok = make_geom(p->ny, p->nx, G, sizeof(cplx<T>), ws_limit, &p->g, &p->ws_bytes, dny, dnx);
-    if (!ok && p->want_threads <= 0) {
-        // one transform does not fit the small workspace (sides >= 4096): fall back to one big CTA per SM
-        threads = 512; minb = 1; ws_limit = 160 * 1024;
-        ok = make_geom(p->ny, p->nx, G, sizeof(cplx<T>), ws_limit, &p->g, &p->ws_bytes, dny, dnx);
-    }
-    if (!ok) return fail(BSGP_E_SHAPE, "unsupported shape %dx%d for cluster size %d (power-of-two sides >= 16 required)", p->ny, p->nx, G);
-    p->threads = threads;
-    p->minb = minb;
-    // shared-memory layout: [SharedCtl][ImgState][twiddles][position table][workspace][resident slabs]
-    SmemPlan sp;
-    size_t off = up128(sizeof(SharedCtl));
-    sp.off_state = (unsigned)off; off = up128(off + sizeof(ImgState<T>));
-    sp.ctl_stride = (unsigned)((sizeof(CtlState<T>) + 15) & ~(size_t)15);
-    sp.off_ctl = (unsigned)off; off = up128(off + (size_t)(threads / 32) * sp.ctl_stride);
-    const size_t tw_bytes = ((size_t)p->nx + (p->ny != p->nx ? p->ny : 0)) * sizeof(cplx<T>);
-    sp.tw_smem = tw_bytes <= 16384 ? 1 : 0;             // cluster mode: full tables in shared memory, or global
-    // a dense axis of an fp64 plan keeps the DMMA fragment table of its transform there instead (bsgp_fft.cuh, fill_dense_table)
-    auto tw_bytes_of = [&](int n, int dft_n) -> size_t {
-        if (dft_n && sizeof(T) == 8) return (size_t)8 * n * n;
-        return tw_table_entries(sp.tw_smem, n) * sizeof(cplx<T>);
-    };
-    sp.off_twx = (unsigned)off;
-    sp.off_twy = (unsigned)off;
-    off = up128(off + tw_bytes_of(p->nx, p->g.px.dft_n));
-    if (p->ny != p->nx || p->g.py.dft_n != p->g.px.dft_n) { sp.off_twy = (unsigned)off; off = up128(off + tw_bytes_of(p->ny, p->g.py.dft_n)); }
-    sp.off_ppx = (unsigned)off; off = up128(off + (size_t)p->nx * sizeof(unsigned short));
-    sp.off_ws = (unsigned)off; off = up128(off + p->ws_bytes);
-    sp.off_bufs = (unsigned)off;
-    p->sp = sp;
-    const size_t fixed = off;
-    // per-CTA budget: the opt-in maximum, or an equal share of the SM (1 KB per CTA is reserved by the system)
-    size_t budget = (size_t)p->max_smem;
-    if (p->minb > 1) {
-        const size_t share = ((size_t)p->smem_per_sm - (size_t)p->minb * 1024) / p->minb;
-        budget = share < budget ? share : budget;
-        budget &= ~(size_t)127;
-    }
-    const size_t slab_bytes = nslab * sizeof(T);
-    size_t used = fixed;
-    int mask = 0;
-    for (int k = 0; k < NBUF; ++k) {
-        if (used + slab_bytes <= budget) { mask |= 1 << kResidencyOrder[k]; used += slab_bytes; }
-    }
-    // Small slabs, automatic configuration: three 128-thread CTAs per SM if everything but the background image stays
-    // resident in a third of the SM's shared memory (32 x 32 fp64 stamps: 8192 stamps 19.7 ms against 22.8 ms for two
-    // 256-thread CTAs); otherwise (e.g. 31 x 31 cut-outs, whose tensor-core table takes 8 KB) two 256-thread CTAs.
-    if (p->small_try && small_slab && p->want_threads <= 0 && (mask | (1 << B_BKG)) != (1 << NBUF) - 1) {
-        p->small_try = false;
-        return plan_setup_t<T>(p);
-    }
-    p->resident_mask = mask;
-    p->smem_bytes = used;
-    if (p->smem_bytes > (size_t)p->max_smem)
-        return fail(BSGP_E_SHAPE, "shape %dx%d needs %zu B of shared memory per CTA (limit %d)", p->ny, p->nx, p->smem_bytes, p->max_smem);
-    LaunchCfg lc{G * p->num_sms, threads, G, p->smem_bytes, nullptr, p->minb};
-    int nc = 0;
-    cudaError_t e = query_solve_clusters<T, false>(lc, p->num_sms, &nc);
-    if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
-    if (nc <= 0) return fail(BSGP_E_CUDA, "kernel does not fit: cluster %d, %d threads, %zu B shared memory", G, threads, p->smem_bytes);
-    p->num_clusters = nc;
-    // stand-alone convolution kernel: [SharedCtl][ConvGeom][position table][workspace]
-    p->conv_off_geom = (unsigned)up128(sizeof(SharedCtl));
-    p->conv_off_ppx = (unsigned)up128(p->conv_off_geom + sizeof(ConvGeom));
-    p->conv_off_ws = (unsigned)up128(p->conv_off_ppx + (size_t)p->nx * sizeof(unsigned short));
-    p->conv_smem = p->conv_off_ws + up128(p->ws_bytes);
-    LaunchCfg cc{G * p->num_sms, 512, G, p->conv_smem, nullptr};
-    e = query_clusters(conv_kernel_ptr<T>(), cc, p->num_sms, &nc);
-    if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
-    if (nc <= 0) return fail(BSGP_E_CUDA, "convolution kernel does not fit: cluster %d, %zu B shared memory", G, p->conv_smem);
-    p->conv_clusters = nc;
-
     { int rc = alloc_tables<T>(p); if (rc) return rc; }
     const int nscratch = p->num_clusters > p->conv_clusters ? p->num_clusters : p->conv_clusters;
-    p->work_stride = NBUF * npix;
+    p->work_stride = NBUF * (size_t)p->ny * p->nx;
     p->spec_stride = (size_t)p->ny * p->g.hx;
     p->tf_stride = (size_t)(p->g.hx + 1) * p->ny;
     CU(cudaMalloc(&p->work, (size_t)p->num_clusters * p->work_stride * sizeof(T)));
     CU(cudaMalloc(&p->spec, (size_t)nscratch * p->spec_stride * sizeof(cplx<T>)));
     CU(cudaMalloc((void**)&p->queue, sizeof(int)));
+    if (p->frame) CU(cudaMalloc((void**)&p->gpart, (size_t)2 * G * kMaxK * sizeof(double)));
     p->workspace_bytes = (size_t)p->num_clusters * p->work_stride * sizeof(T) + (size_t)nscratch * p->spec_stride * sizeof(cplx<T>);
     p->configured = true;
     return BSGP_OK;
@@ -623,11 +457,7 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
 static int plan_setup(bsgp_plan* p) {
     if (p->configured) return BSGP_OK;
     CU(cudaSetDevice(p->device));
-    const int rc = p->dtype == BSGP_F64 ? plan_setup_t<double>(p) : plan_setup_t<float>(p);
-    if (rc) return rc;
-    p->g.wrap_ny = (p->ny != p->img_ny && !p->g.py.dft_n) ? p->img_ny : 0;      // fold widths; a dense axis is circular by itself
-    p->g.wrap_nx = (p->nx != p->img_nx && !p->g.px.dft_n) ? p->img_nx : 0;
-    return BSGP_OK;
+    return p->dtype == BSGP_F64 ? plan_setup_t<double>(p) : plan_setup_t<float>(p);
 }
 
 // Stream ordering of a plan.  A plan owns mutable device state (PSF spectra, per-cluster scratch, the work-queue counter),
@@ -838,6 +668,35 @@ static int check_params(const bsgp_params* q) {
     return BSGP_OK;
 }
 
+static int adjoint_on_wrapped_plan() {
+    return fail(BSGP_E_STATE, "bsgp_set_psf_adjoint: a plan whose sides are not powers of two builds both kernels in bsgp_set_psf");
+}
+
+// bsgp_set_psf / bsgp_set_psf_adjoint from host memory: the caller's PSFs [n_psf][img_ny][img_nx], staged for the call
+static int set_psf_host(bsgp_plan* p, const void* psf_host, int n_psf, bool adjoint) {
+    if (!p || !psf_host || n_psf < 1) return fail(BSGP_E_ARG, "bad argument");
+    if (adjoint && p->embedded) return adjoint_on_wrapped_plan();
+    CU(cudaSetDevice(p->device));
+    const size_t bytes = (size_t)n_psf * p->img_ny * p->img_nx * p->elem;
+    void* d = nullptr;
+    CU(cudaMalloc(&d, bytes));
+    cudaError_t e = cudaMemcpy(d, psf_host, bytes, cudaMemcpyHostToDevice);
+    int rc = e != cudaSuccess ? fail(BSGP_E_CUDA, "H2D copy failed: %s", cudaGetErrorString(e))
+                              : (adjoint ? bsgp_set_psf_adjoint : bsgp_set_psf)(p, d, n_psf, nullptr);
+    if (rc == BSGP_OK) { e = cudaDeviceSynchronize(); if (e != cudaSuccess) rc = fail(BSGP_E_CUDA, "PSF spectrum kernel failed: %s", cudaGetErrorString(e)); }
+    cudaFree(d);
+    return rc;
+}
+
+// the caller's device index, made current
+static int use_device(int device) {
+    int ndev = 0;
+    CU(cudaGetDeviceCount(&ndev));
+    if (device < 0 || device >= ndev) return fail(BSGP_E_CUDA, "device %d not available", device);
+    CU(cudaSetDevice(device));
+    return BSGP_OK;
+}
+
 extern "C" {
 
 int bsgp_device_count(void) {
@@ -888,7 +747,6 @@ int bsgp_plan_configure(bsgp_plan* p, int cluster_size, int threads) {
     plan_free_buffers(p);
     p->configured = false;
     p->want_G = cluster_size; p->want_threads = threads;
-    p->small_try = true;
     return plan_setup(p);
 }
 
@@ -925,22 +783,9 @@ int bsgp_set_psf(bsgp_plan* p, const void* psf_dev, int n_psf, void* stream) {
     return plan_leave(p, st);
 }
 
-int bsgp_set_psf_host(bsgp_plan* p, const void* psf_host, int n_psf) {
-    if (!p || !psf_host || n_psf < 1) return fail(BSGP_E_ARG, "bad argument");
-    CU(cudaSetDevice(p->device));
-    const size_t bytes = (size_t)n_psf * p->img_ny * p->img_nx * p->elem;
-    void* d = nullptr;
-    CU(cudaMalloc(&d, bytes));
-    cudaError_t e = cudaMemcpy(d, psf_host, bytes, cudaMemcpyHostToDevice);
-    int rc = e == cudaSuccess ? bsgp_set_psf(p, d, n_psf, nullptr) : fail(BSGP_E_CUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-    if (rc == BSGP_OK) { e = cudaDeviceSynchronize(); if (e != cudaSuccess) rc = fail(BSGP_E_CUDA, "PSF spectrum kernel failed: %s", cudaGetErrorString(e)); }
-    cudaFree(d);
-    return rc;
-}
-
 int bsgp_set_psf_adjoint(bsgp_plan* p, const void* psf_dev, int n_psf, void* stream) {
     if (!p || !psf_dev || n_psf < 1) return fail(BSGP_E_ARG, "bad argument");
-    if (p->embedded) return fail(BSGP_E_STATE, "bsgp_set_psf_adjoint: a plan whose sides are not powers of two builds both kernels in bsgp_set_psf");
+    if (p->embedded) return adjoint_on_wrapped_plan();
     if (misaligned(psf_dev)) return fail(BSGP_E_ARG, "image pointers must be 16-byte aligned (vector loads)");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -951,18 +796,8 @@ int bsgp_set_psf_adjoint(bsgp_plan* p, const void* psf_dev, int n_psf, void* str
     return plan_leave(p, st);
 }
 
-int bsgp_set_psf_adjoint_host(bsgp_plan* p, const void* psf_host, int n_psf) {
-    if (!p || !psf_host || n_psf < 1) return fail(BSGP_E_ARG, "bad argument");
-    CU(cudaSetDevice(p->device));
-    const size_t bytes = (size_t)n_psf * p->ny * p->nx * p->elem;
-    void* d = nullptr;
-    CU(cudaMalloc(&d, bytes));
-    cudaError_t e = cudaMemcpy(d, psf_host, bytes, cudaMemcpyHostToDevice);
-    int rc = e == cudaSuccess ? bsgp_set_psf_adjoint(p, d, n_psf, nullptr) : fail(BSGP_E_CUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-    if (rc == BSGP_OK) { e = cudaDeviceSynchronize(); if (e != cudaSuccess) rc = fail(BSGP_E_CUDA, "PSF spectrum kernel failed: %s", cudaGetErrorString(e)); }
-    cudaFree(d);
-    return rc;
-}
+int bsgp_set_psf_host(bsgp_plan* p, const void* psf_host, int n_psf) { return set_psf_host(p, psf_host, n_psf, false); }
+int bsgp_set_psf_adjoint_host(bsgp_plan* p, const void* psf_host, int n_psf) { return set_psf_host(p, psf_host, n_psf, true); }
 
 // Argument checks of every solve entry point.  The host entry points run them on the caller's pointers before they size
 // anything from batch or prm->maxit (the device copies they stage are present exactly where the caller's arrays are),
@@ -1256,13 +1091,10 @@ int bsgp_project_df(const double* b, const double* c, const double* dia, int n, 
 int bsgp_project_df_host(const double* b, const double* c, const double* dia, int n, int batch, double sat_cap, double lambda0,
                          double dlambda0, double tol_lam, int max_projs, int biter, int siter, double* x, int* evals, int* status, int device) {
     if (!b || !c || !dia || !x) return fail(BSGP_E_ARG, "NULL argument");
-    int ndev = 0;
-    CU(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return fail(BSGP_E_CUDA, "device %d not available", device);
-    CU(cudaSetDevice(device));
+    int rc;
+    TRY(use_device(device));
     const size_t vb = (size_t)n * batch * 8;
     DevBuf db, dc, dd, dx, de, ds;
-    int rc;
     TRY(db.up(b, (size_t)batch * 8)); TRY(dc.up(c, vb)); TRY(dd.up(dia, vb)); TRY(dx.alloc(true, vb));
     TRY(de.alloc(true, (size_t)batch * 4)); TRY(ds.alloc(true, (size_t)batch * 4));
     TRY(bsgp_project_df((const double*)db.d, (const double*)dc.d, (const double*)dd.d, n, batch, sat_cap, lambda0, dlambda0, tol_lam,
@@ -1275,12 +1107,9 @@ int bsgp_project_df_host(const double* b, const double* c, const double* dia, in
 
 int bsgp_beta_div_host(const double* y, const double* x, long long n, double beta, double* value, double* deriv, int device) {
     if (!y || !x || !value || n < 1) return fail(BSGP_E_ARG, "bad argument");
-    int ndev = 0;
-    CU(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return fail(BSGP_E_CUDA, "device %d not available", device);
-    CU(cudaSetDevice(device));
-    DevBuf dy, dx, dp, dd;
     int rc;
+    TRY(use_device(device));
+    DevBuf dy, dx, dp, dd;
     long long want = (n + 255) / 256;
     const int grid = (int)(want < 592 ? want : 592);
     TRY(dy.up(y, (size_t)n * 8)); TRY(dx.up(x, (size_t)n * 8)); TRY(dp.alloc(true, (size_t)grid * 3 * 8)); TRY(dd.alloc(deriv != nullptr, (size_t)n * 8));
@@ -1303,12 +1132,9 @@ int bsgp_beta_div_host(const double* y, const double* x, long long n, double bet
 }
 int bsgp_beta_grad_terms_host(const double* den, const double* gn, long long n, double beta, double* p1, double* u, int device) {
     if (!den || !gn || !p1 || !u || n < 1) return fail(BSGP_E_ARG, "bad argument");
-    int ndev = 0;
-    CU(cudaGetDeviceCount(&ndev));
-    if (device < 0 || device >= ndev) return fail(BSGP_E_CUDA, "device %d not available", device);
-    CU(cudaSetDevice(device));
-    DevBuf dd, dg, dp, du;
     int rc;
+    TRY(use_device(device));
+    DevBuf dd, dg, dp, du;
     TRY(dd.up(den, (size_t)n * 8)); TRY(dg.up(gn, (size_t)n * 8)); TRY(dp.alloc(true, (size_t)n * 8)); TRY(du.alloc(true, (size_t)n * 8));
     long long want = (n + 255) / 256;
     count_launch();
@@ -1350,19 +1176,11 @@ int bsgp_tile_boxes(int height, int width, int tile_h, int tile_w, double overla
     return BSGP_OK;
 }
 
-static int tile_grid(int device, size_t total, int* blocks) {
-    int sms = 0;
-    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-    size_t want = (total + 255) / 256, cap = (size_t)sms * 8;          // 8 CTAs of 256 threads per SM, grid-stride beyond
-    *blocks = (int)(want < cap ? (want ? want : 1) : cap);
-    return BSGP_OK;
-}
-
 int bsgp_extract_tiles(const void* frame_dev, int height, int width, int dtype, const int* origins_dev, int n, int tile_h, int tile_w, void* tiles_dev, int device, void* stream) {
     if (!frame_dev || !origins_dev || !tiles_dev || n < 1 || tile_h < 1 || tile_w < 1 || height < 1 || width < 1) return fail(BSGP_E_ARG, "bad argument");
     if (dtype != BSGP_F64 && dtype != BSGP_F32) return fail(BSGP_E_ARG, "bad dtype");
     CU(cudaSetDevice(device));
-    int blocks = 0, rc = tile_grid(device, (size_t)n * tile_h * tile_w, &blocks);
+    int blocks = 0, rc = data_grid(device, (size_t)n * tile_h * tile_w, &blocks);
     if (rc) return rc;
     count_launch();
     if (dtype == BSGP_F64) bsgp_extract_tiles_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>((const double*)frame_dev, height, width, origins_dev, n, tile_h, tile_w, (double*)tiles_dev);
@@ -1375,7 +1193,7 @@ int bsgp_assemble_tiles(const void* tiles_dev, const int* origins_dev, int n, in
     if (!frame_dev || !origins_dev || !tiles_dev || n < 1 || tile_h < 1 || tile_w < 1 || height < 1 || width < 1) return fail(BSGP_E_ARG, "bad argument");
     if (dtype != BSGP_F64 && dtype != BSGP_F32) return fail(BSGP_E_ARG, "bad dtype");
     CU(cudaSetDevice(device));
-    int blocks = 0, rc = tile_grid(device, (size_t)height * width, &blocks);
+    int blocks = 0, rc = data_grid(device, (size_t)height * width, &blocks);
     if (rc) return rc;
     count_launch();
     if (dtype == BSGP_F64) bsgp_assemble_tiles_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>((const double*)tiles_dev, origins_dev, n, tile_h, tile_w, feather, (double*)frame_dev, height, width);

@@ -25,31 +25,29 @@ template <class Ctx, typename T> __device__ __forceinline__ void fill_twiddles(C
     }
 }
 
-template <typename T, int NT, int MINB, bool MK>
-__global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride) {
-    unsigned char* smem = dyn_smem();
-    // 2 CTAs x 256 threads and 3 CTAs x 128 threads per SM are the configurations of images that are resident in shared memory
-    // (bsgp_kernels.cu, plan_setup_t)
-    typename std::conditional<(NT == 256 && MINB == 2) || (NT == 128 && MINB == 3), DeviceCtxSmall, DeviceCtx>::type ctx;
-    static_cast<DeviceCtx&>(ctx) = make_ctx(reinterpret_cast<SharedCtl*>(smem), a.g.G);
+// Prologue of both persistent kernels: this warp's controller state, the slab arrays (resident in shared memory or in
+// this cluster's global scratch), the twiddle and position tables, and the per-image constants in shared memory.  Frame
+// plans have no resident arrays, one scratch area and no dense axes (bsgp_plan.h): the constants below keep that code
+// out of the frame kernel.
+template <typename T, class Ctx>
+__device__ __forceinline__ ImgState<T>* solve_prologue(Ctx& ctx, unsigned char* smem, const SolveArgs<T>& a, const SmemPlan& sp, T* (&buf)[NBUF]) {
     ctx.wst = smem + sp.off_ctl + (threadIdx.x >> 5) * sp.ctl_stride;
     ImgState<T>* S = reinterpret_cast<ImgState<T>*>(smem + sp.off_state);
-    const int cluster_id = blockIdx.x / a.g.G;
+    const int cluster_id = Ctx::kFrame ? 0 : blockIdx.x / a.g.G;
+    const int resident = Ctx::kFrame ? 0 : a.resident_mask;
     const size_t npix = (size_t)a.g.ny * a.g.nx;
     const size_t nslab = (size_t)a.g.rows_per_cta * a.g.nx;
-    T* buf[NBUF];
     size_t soff = sp.off_bufs;
 #pragma unroll
     for (int b = 0; b < NBUF; ++b) {
-        if (a.resident_mask & (1 << b)) { buf[b] = reinterpret_cast<T*>(smem + soff); soff += nslab * sizeof(T); }
+        if (resident & (1 << b)) { buf[b] = reinterpret_cast<T*>(smem + soff); soff += nslab * sizeof(T); }
         else buf[b] = a.work + (size_t)cluster_id * a.work_stride + (size_t)b * npix + (size_t)ctx.rank * nslab;
     }
     cplx<T>* twx_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twx);
     cplx<T>* twy_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twy);
-    fill_twiddles(ctx, sp.tw_smem, a.g.nx, a.twx, twx_s, a.g.px.dft_n);
-    if (sp.off_twy != sp.off_twx) fill_twiddles(ctx, sp.tw_smem, a.g.ny, a.twy, twy_s, a.g.py.dft_n);
-    unsigned short* ppx = reinterpret_cast<unsigned short*>(smem + sp.off_ppx);
-    fill_pos_table(ctx, a.g.px, ppx);
+    fill_twiddles(ctx, sp.tw_smem, a.g.nx, a.twx, twx_s, Ctx::kFrame ? 0 : a.g.px.dft_n);
+    if (sp.off_twy != sp.off_twx) fill_twiddles(ctx, sp.tw_smem, a.g.ny, a.twy, twy_s, Ctx::kFrame ? 0 : a.g.py.dft_n);
+    fill_pos_table(ctx, a.g.px, reinterpret_cast<unsigned short*>(smem + sp.off_ppx));
     if (ctx.tid == 0) {
         S->geom = a.g;
         S->ppx_off = sp.off_ppx;
@@ -60,7 +58,7 @@ __global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T>
         // the whole spectrum into the workspace before it stores its first output; d_tf itself is dead across every
         // convolution: it is written by the consumer of A(d) (ph_ri_trial), read by the line search and, for the last
         // time, by the producer of the accepted step's A^T (ph_rf_grad).
-        const bool spec_in_dtf = a.g.G == 1 && ((a.resident_mask >> B_DTF) & 1) && 2 * a.g.row_tile_pairs == a.g.ny && a.g.col_tile == a.g.hx;
+        const bool spec_in_dtf = a.g.G == 1 && ((resident >> B_DTF) & 1) && 2 * a.g.row_tile_pairs == a.g.ny && a.g.col_tile == a.g.hx;
         S->spec = spec_in_dtf ? reinterpret_cast<cplx<T>*>(buf[B_DTF]) : a.spec + (size_t)cluster_id * a.spec_stride;
         S->twx = a.twx; S->twy = a.twy;
         S->twx_off = sp.tw_smem ? sp.off_twx : kNoSmem;
@@ -68,6 +66,18 @@ __global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T>
         S->tw_split = sp.tw_smem == 2;
     }
     __syncthreads();
+    return S;
+}
+
+template <typename T, int NT, int MINB, bool MK>
+__global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride) {
+    unsigned char* smem = dyn_smem();
+    // 2 CTAs x 256 threads and 3 CTAs x 128 threads per SM are the configurations of images that are resident in shared memory
+    // (bsgp_plan.h, plan_launch)
+    typename std::conditional<(NT == 256 && MINB == 2) || (NT == 128 && MINB == 3), DeviceCtxSmall, DeviceCtx>::type ctx;
+    static_cast<DeviceCtx&>(ctx) = make_ctx(reinterpret_cast<SharedCtl*>(smem), a.g.G);
+    T* buf[NBUF];
+    ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
     for (;;) {
         bool ready_ok;
         const int item = next_item(ctx, a.queue, a.ready, a.batch, &ready_ok);
@@ -88,29 +98,8 @@ template <typename T, bool MK>
 __global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart) {
     unsigned char* smem = dyn_smem();
     GridCtx ctx = make_grid_ctx(reinterpret_cast<SharedCtl*>(smem), gpart);
-    ctx.wst = smem + sp.off_ctl + (threadIdx.x >> 5) * sp.ctl_stride;
-    ImgState<T>* S = reinterpret_cast<ImgState<T>*>(smem + sp.off_state);
-    const size_t npix = (size_t)a.g.ny * a.g.nx;
-    const size_t nslab = (size_t)a.g.rows_per_cta * a.g.nx;
     T* buf[NBUF];
-#pragma unroll
-    for (int b = 0; b < NBUF; ++b) buf[b] = a.work + (size_t)b * npix + (size_t)ctx.rank * nslab;
-    cplx<T>* twx_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twx);
-    cplx<T>* twy_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twy);
-    fill_twiddles(ctx, sp.tw_smem, a.g.nx, a.twx, twx_s);
-    if (sp.off_twy != sp.off_twx) fill_twiddles(ctx, sp.tw_smem, a.g.ny, a.twy, twy_s);
-    fill_pos_table(ctx, a.g.px, reinterpret_cast<unsigned short*>(smem + sp.off_ppx));
-    if (ctx.tid == 0) {
-        S->geom = a.g;
-        S->ppx_off = sp.off_ppx;
-        S->ws_off = sp.off_ws;
-        S->spec = a.spec;
-        S->twx = a.twx; S->twy = a.twy;
-        S->twx_off = sp.tw_smem ? sp.off_twx : kNoSmem;
-        S->twy_off = sp.tw_smem ? sp.off_twy : kNoSmem;
-        S->tw_split = sp.tw_smem == 2;
-    }
-    __syncthreads();
+    ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
     for (int img = 0; img < a.batch; ++img) {
         cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)img * tf_stride : 0);
         cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)img * tf_stride : 0) : tf;

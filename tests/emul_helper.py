@@ -93,6 +93,21 @@ def solve(gn, psf, bkg, divergence="kl", flux=None, betaParam=1.005, obj=None, x
                 alpha=ta[1:n + 1], lam=tl[1:n + 1], beta_trace=tb[1:n + 1], trials=tt[1:n + 1], evals=te[1:n + 1])
 
 
+PLAN_FIELDS = ("frame", "cluster_size", "threads", "minb", "resident_mask", "smem_bytes", "conv_smem", "ws_bytes", "wrap_ny",
+               "wrap_nx", "grid_ny", "grid_nx")
+
+
+def plan_launch(shape, dtype, cluster_size=0, threads=0, *, num_sms, max_smem, smem_per_sm):
+    """The library's launch-shape planner (csrc/bsgp_plan.h, plan_launch) for an image of `shape` on the device described by
+    the keywords: (0, dict of PLAN_FIELDS) or (BSGP_E_* code, None)."""
+    L = lib()
+    out = (C.c_longlong * len(PLAN_FIELDS))()
+    L.emul_plan_launch.argtypes = [C.c_int] * 8 + [C.POINTER(C.c_longlong)]
+    rc = L.emul_plan_launch(shape[0], shape[1], capi.BSGP_F64 if dtype == "float64" else capi.BSGP_F32, cluster_size, threads,
+                            num_sms, max_smem, smem_per_sm, out)
+    return rc, (dict(zip(PLAN_FIELDS, out)) if rc == 0 else None)
+
+
 def project(c, dia, b, sat_cap=None, max_projs=1000, biter=0, siter=0):
     L = lib()
     c = np.ascontiguousarray(c, dtype=np.float64); dia = np.ascontiguousarray(dia, dtype=np.float64)

@@ -269,6 +269,22 @@ int emul_solve_wrapped(int iny, int inx, const bsgp_params* params, const double
     return 0;
 }
 
+// the library's launch-shape planner (bsgp_plan.h, plan_launch) for an image of iny x inx on the FFT grid bsgp_plan_create
+// picks; returns 0 or the BSGP_E_* code.  out: frame, G, threads, minb, resident_mask, smem_bytes, conv_smem, ws_bytes,
+// wrap_ny, wrap_nx, grid ny, grid nx
+int emul_plan_launch(int iny, int inx, int dtype, int want_G, int want_threads, int num_sms, int max_smem, int smem_per_sm,
+                     long long* out) {
+    const PlanRequest q{wrap_grid_side(iny), wrap_grid_side(inx), iny, inx, want_G, want_threads, num_sms, max_smem, smem_per_sm};
+    LaunchPlan L;
+    char err[256];
+    const int rc = dtype == BSGP_F64 ? plan_launch<double>(q, &L, err, sizeof err) : plan_launch<float>(q, &L, err, sizeof err);
+    if (rc) return rc;
+    const long long v[12] = {L.frame, L.g.G, L.threads, L.minb, L.resident_mask, (long long)L.smem_bytes, (long long)L.conv_smem,
+                             (long long)L.ws_bytes, L.g.wrap_ny, L.g.wrap_nx, q.ny, q.nx};
+    for (int k = 0; k < 12; ++k) out[k] = v[k];
+    return 0;
+}
+
 // projectDF root-find with the reference's x = (c + lambda) / dia evaluation
 int emul_project(const double* c, const double* dia, int n, double b, double sat_cap, int has_cap, int max_projs, int biter, int siter,
                  double* x, int* evals) {

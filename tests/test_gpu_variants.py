@@ -191,11 +191,37 @@ def test_variant_table_covers_every_kernel():
 def test_variant_lands_on_its_cell(bs, v):
     """A change of the automatic configuration must not move a row to another kernel unnoticed."""
     plan, padded, cell = _plan_cell(bs, v)
-    G = plan.info()["cluster_size"]
+    info = plan.info()
     if not padded:
         plan.close()
     assert cell == v.cell, cell
-    assert G == 1 or cell[2] not in ((128, 3), (256, 2)), "a cluster of several CTAs on a one-CTA launch shape"
+    assert info["cluster_size"] == 1 or cell[2] not in ((128, 3), (256, 2)), "a cluster of several CTAs on a one-CTA launch shape"
+    # the library's launch shape is the host-compiled planner's (tests/host_emul) for this device
+    import emul_helper as eh
+    import torch
+    prop = torch.cuda.get_device_properties(info["device"])
+    rc, s = eh.plan_launch((info["ny"], info["nx"]), v.dtype, 0 if padded else v.cfg.get("cluster_size", 0),
+                           0 if padded else v.cfg.get("threads", 0), num_sms=prop.multi_processor_count,
+                           max_smem=prop.shared_memory_per_block_optin, smem_per_sm=prop.shared_memory_per_multiprocessor)
+    assert rc == 0
+    for k in ("threads", "cluster_size", "smem_bytes", "resident_mask"):
+        assert info[k] == s[k], (k, info[k], s[k])
+
+
+def test_dense_axes_refuse_frame_mode(bs):
+    """A 31 x 31 plan transforms both axes with a dense 31-point DFT, which needs one CTA per image: frame mode is refused
+    (it used to run the radix FFT of the 32-point grid and fold the 61-long linear convolution on a 32-point circle)."""
+    with pytest.raises(bs._capi.BsgpError, match="frame mode"):
+        bs.Plan(31, 31, cluster_size=-1)
+
+
+def test_set_psf_adjoint_host_refuses_wrapped_plan(bs):
+    """bsgp_set_psf_adjoint_host on a wrapped plan takes the caller's image-sized buffer and returns BSGP_E_STATE before
+    it copies anything (it used to copy a grid-sized block from it first)."""
+    plan = bs.Plan(100, 75)
+    psf = np.full((100, 75), 1.0 / 7500)
+    assert bs._capi.lib().bsgp_set_psf_adjoint_host(plan._h, psf.ctypes.data, 1) == 5       # BSGP_E_STATE
+    plan.close()
 
 
 @pytest.mark.parametrize("run", ["beta", "kl"])

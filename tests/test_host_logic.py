@@ -373,3 +373,64 @@ def test_emulated_projection_counter_arguments(golden, mp, bi, si):
         xe, ev, st = eh.project(c, dia, float(b), max_projs=mp, biter=bi, siter=si)
         assert st == 0 and ev == cnt[-1]
         np.testing.assert_allclose(xe, xo, rtol=1e-12, atol=1e-15)
+
+
+# ------------------------------------------------------------------------------------------------
+# the launch-shape planner (csrc/bsgp_plan.h, plan_launch) with a B200's properties: 148 SMs, 227 KB of opt-in shared
+# memory per block, 228 KB per SM (cudaDevAttrMaxSharedMemoryPerMultiprocessor, read on a B200)
+# ------------------------------------------------------------------------------------------------
+B200 = dict(num_sms=148, max_smem=232448, smem_per_sm=233472)
+BSGP_E_SHAPE = 2                                          # include/bsgp.h
+
+
+def _planned_cell(v):
+    """The cell a row of tests/test_gpu_variants.py lands on by the planner alone.  Padded rows run on the front end's
+    P x P grid (engine.PaddedGeometry); the CTAs per SM of a cluster plan are the ones its kernel variant is compiled for."""
+    if v.kernel:
+        P = int(2 ** np.ceil(np.log2(max(v.shape[0] + v.kernel, v.shape[1] + v.kernel))))
+        assert P in (512, 1024)
+        rc, s = eh.plan_launch((P, P), v.dtype, **B200)
+    else:
+        rc, s = eh.plan_launch(v.shape, v.dtype, v.cfg.get("cluster_size", 0), v.cfg.get("threads", 0), **B200)
+    assert rc == 0, (v.label, rc)
+    mk = bool(v.kernel) or (s["grid_ny"], s["grid_nx"]) != v.shape
+    return (v.dtype, mk, "frame" if s["frame"] else (s["threads"], s["minb"]))
+
+
+def test_planner_lands_every_variant_on_its_cell():
+    """Every row of the variant table (padded rows included) lands on its (threads, CTAs per SM) or frame cell."""
+    from test_gpu_variants import VARIANTS
+    for v in VARIANTS:
+        assert _planned_cell(v) == v.cell, v.label
+
+
+def test_planner_keeps_clusters_off_one_cta_shapes():
+    """128 x 3 and 256 x 2 run DeviceCtxSmall, whose all-reduce sums over one CTA: no cluster of 2..16 CTAs gets them, on
+    any supported image shape and thread request."""
+    sides = [16, 31, 32, 33, 64, 75, 100, 128, 256, 450, 512, 1024, 2048, 4096, 8192]
+    checked = 0
+    for dtype in ("float64", "float32"):
+        for ny in sides:
+            for nx in sides:
+                for G in (2, 4, 8, 16):
+                    for threads in (0, 128, 256, 512):
+                        rc, s = eh.plan_launch((ny, nx), dtype, G, threads, **B200)
+                        if rc:
+                            continue
+                        checked += 1
+                        assert s["cluster_size"] == G and not s["frame"]
+                        assert (s["threads"], s["minb"]) not in ((128, 3), (256, 2)), (dtype, ny, nx, G, threads, s)
+    assert checked > 1000
+
+
+def test_planner_refuses_dense_axes_in_frame_mode():
+    """Sides of at most 32 that are not a power of two use a dense DFT of their own length, which needs one CTA per image.
+    Forced into frame mode (G = 16 on a 32 x 32 grid) such a plan used to fall back to the radix FFT and fold a 61-long
+    linear convolution on a 32-point circle; it is refused.  A wrapped axis in frame mode keeps its fold width."""
+    for dtype in ("float64", "float32"):
+        assert eh.plan_launch((31, 31), dtype, -1, **B200)[0] == BSGP_E_SHAPE
+        assert eh.plan_launch((15, 13), dtype, -1, **B200)[0] == BSGP_E_SHAPE
+        rc, s = eh.plan_launch((100, 75), dtype, -1, **B200)
+        assert rc == 0 and s["frame"] and (s["grid_ny"], s["grid_nx"], s["wrap_ny"], s["wrap_nx"]) == (256, 256, 100, 75)
+        rc, s = eh.plan_launch((31, 31), dtype, **B200)
+        assert rc == 0 and not s["frame"] and s["cluster_size"] == 1 and (s["wrap_ny"], s["wrap_nx"]) == (0, 0)
