@@ -425,7 +425,6 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
         cudaError_t e = query_frame_ctas<T, false>(lc, &per_sm);
         if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
         if (per_sm < 1) return fail(BSGP_E_CUDA, "frame kernel does not fit: %zu B shared memory", p->smem_bytes);
-        CU(cudaFuncSetAttribute(conv_frame_kernel_ptr<T>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
         p->num_clusters = p->conv_clusters = 1;
     } else {
         LaunchCfg lc{G * p->num_sms, p->threads, G, p->smem_bytes, nullptr, p->minb};
@@ -513,6 +512,9 @@ template <typename T> static int launch_conv(bsgp_plan* p, ConvArgs<T>& a, int c
         unsigned og = p->conv_off_geom, op = p->conv_off_ppx, ow = p->conv_off_ws;
         double* gp = p->gpart;
         void* args[] = {&a, &og, &op, &ow, &gp};
+        // the shared-memory limit is an attribute of the kernel, not of the plan: another frame plan of the same dtype may
+        // have set it lower since this plan was set up, so it is set again before every launch (as launch_clustered does)
+        CU(cudaFuncSetAttribute(conv_frame_kernel_ptr<T>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
         count_launch();
         cudaError_t e = cudaLaunchCooperativeKernel(conv_frame_kernel_ptr<T>(), dim3(p->g.G), dim3(512), args, p->conv_smem, st);
         if (e != cudaSuccess) return fail(BSGP_E_CUDA, "convolution kernel launch failed: %s", cudaGetErrorString(e));

@@ -110,9 +110,10 @@ def _f32_psf(p):
     return q
 
 
-def _scene(bs, shape, kernel, seed, fwhm=3.0):
+def _scene(bs, shape, kernel, seed, fwhm=3.0, with_truth=False):
     """(gn, psf, bkg image, flux): a star field blurred by the operator the row runs (circular on the image, or the
-    zero-padded one with a kernel x kernel PSF), a sloped sky, Poisson noise; all values exact in fp32."""
+    zero-padded one with a kernel x kernel PSF), a sloped sky, Poisson noise; all values exact in fp32.  with_truth:
+    the true star field (fp64) follows as a fifth element."""
     from oracle import sgp_oracle as orc
     ny, nx = shape
     rng = np.random.default_rng(seed)
@@ -126,7 +127,8 @@ def _scene(bs, shape, kernel, seed, fwhm=3.0):
     yy, xx = np.mgrid[0:ny, 0:nx]
     bkg = (300.0 + 20.0 * xx / nx - 10.0 * yy / ny).astype(np.float32).astype(np.float64)
     gn = rng.poisson(np.maximum(blur, 0) + bkg).astype(np.float64)
-    return gn, psf, bkg, float((gn - bkg).sum())
+    out = (gn, psf, bkg, float((gn - bkg).sum()))
+    return out + (truth,) if with_truth else out
 
 
 BETA0 = 1.0248357
@@ -369,6 +371,30 @@ def test_frame_mode_batch_per_image_psf(bs):
         assert np.abs(r.x[i] - o.x).max() <= 1e-8 * np.abs(o.x).max()
         assert abs(r.x[i].sum() - flux[i]) <= 1e-9 * flux[i]
     plan.close()
+
+
+def test_frame_plans_of_different_sizes_interleaved(bs):
+    """The shared-memory limit of the frame convolution kernel belongs to the kernel, which every frame plan of a dtype
+    shares.  A 1024^2 frame plan used again after a 100 x 75 frame plan was set up must still launch, with the same
+    result.  The limit used to be set only at plan set-up, so the 1024^2 plan then failed with "too many blocks in
+    cooperative launch" (first seen when the option runs left the 100 x 75 frame plan last before the megapixel test)."""
+    rng = np.random.default_rng(11)
+    big = bs.Plan(1024, 1024, cluster_size=-1)
+    small = None
+    try:
+        assert big.info()["num_clusters"] == 1
+        big.set_psf(_f32_psf(bs.synth.moffat_psf(1024, 1024, 3.0)))
+        x = rng.random((1, 1024, 1024))
+        y0 = big.apply_psf(x)
+        small = bs.Plan(100, 75, cluster_size=-1)
+        assert small.info()["num_clusters"] == 1
+        small.set_psf(_f32_psf(bs.synth.moffat_psf(100, 75, 3.0)))
+        small.apply_psf(rng.random((1, 100, 75)))
+        assert np.array_equal(big.apply_psf(x), y0)
+    finally:
+        big.close()
+        if small is not None:
+            small.close()
 
 
 @pytest.mark.parametrize("shape,cfg", [((32, 32), {}), ((256, 256), {}), ((128, 128), dict(cluster_size=8)),

@@ -434,3 +434,17 @@ def test_planner_refuses_dense_axes_in_frame_mode():
         assert rc == 0 and s["frame"] and (s["grid_ny"], s["grid_nx"], s["wrap_ny"], s["wrap_nx"]) == (256, 256, 100, 75)
         rc, s = eh.plan_launch((31, 31), dtype, **B200)
         assert rc == 0 and not s["frame"] and s["cluster_size"] == 1 and (s["wrap_ny"], s["wrap_nx"]) == (0, 0)
+
+
+import test_gpu_options as tgo  # noqa: E402  (the option runs of the GPU suite; importing it needs no device)
+
+
+@pytest.mark.parametrize("run", list(tgo.OPTION_RUNS))
+@pytest.mark.parametrize("shape,kernel", tgo._option_cells(), ids=lambda a: "x".join(map(str, a)) if isinstance(a, tuple) else f"k{a}")
+def test_option_run_premises(shape, kernel, run):
+    """The option runs of tests/test_gpu_options.py, on the oracle alone: every run ends by its own stop rule before
+    MAXIT (rules 2 and 3 inside TOL_WINDOW, tol at least TOL_MARGIN apart from the stop values on both sides of the
+    firing iteration), and the saturation cap of stop3-cap holds pixels at the cap.  Without this a scene change could
+    turn the GPU runs into MAXIT runs unnoticed."""
+    info = tgo.option_premises(shape, kernel, run)
+    print(f"\n{shape} kernel {kernel} {run}: {info}")
