@@ -105,6 +105,9 @@ def lib():
     L.bsgp_solve_batch.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
     L.bsgp_solve_batch_host.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs)]
     L.bsgp_solve_batch_pinned.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
+    L.bsgp_solve_batch_rows.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
+    L.bsgp_solve_batch_rows_host.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs)]
+    L.bsgp_solve_batch_rows_pinned.argtypes = [vp, C.POINTER(Params), ip, C.POINTER(Inputs), C.POINTER(Outputs), vp]
     L.bsgp_apply_psf.argtypes = [vp, vp, vp, ip, ip, vp]
     L.bsgp_apply_psf_host.argtypes = [vp, vp, vp, ip, ip]
     L.bsgp_project_df.argtypes = [vp, vp, vp, ip, ip, dp, dp, dp, dp, ip, ip, ip, vp, vp, vp, ip, vp]
@@ -130,6 +133,7 @@ def check(rc):
 
 
 EXPORTED = ["bsgp_plan_create", "bsgp_plan_destroy", "bsgp_plan_get_info", "bsgp_plan_configure", "bsgp_set_psf",
-            "bsgp_set_psf_host", "bsgp_set_psf_adjoint", "bsgp_set_psf_adjoint_host", "bsgp_solve_batch", "bsgp_solve_batch_host", "bsgp_solve_batch_pinned", "bsgp_apply_psf", "bsgp_apply_psf_host",
+            "bsgp_set_psf_host", "bsgp_set_psf_adjoint", "bsgp_set_psf_adjoint_host", "bsgp_solve_batch", "bsgp_solve_batch_host", "bsgp_solve_batch_pinned",
+            "bsgp_solve_batch_rows", "bsgp_solve_batch_rows_host", "bsgp_solve_batch_rows_pinned", "bsgp_apply_psf", "bsgp_apply_psf_host",
             "bsgp_project_df", "bsgp_project_df_host", "bsgp_tile_boxes", "bsgp_extract_tiles", "bsgp_assemble_tiles", "bsgp_psf_model_eval", "bsgp_beta_div_host", "bsgp_beta_grad_terms_host", "bsgp_device_count", "bsgp_launch_count",
             "bsgp_last_error_string", "bsgp_version"]

@@ -28,6 +28,7 @@
 #include "bsgp_device.cuh"
 #include "bsgp_launch.h"
 #include "bsgp_plan.h"
+#include "bsgp_rows.h"
 #include "bsgp_solver.cuh"
 #include "bsgp_wrap.h"
 
@@ -370,14 +371,18 @@ struct bsgp_plan : LaunchPlan {
     int* ready = nullptr; int* ones_host = nullptr; int ready_cap = 0;
     cudaStream_t s_copy = nullptr, s_run = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_flags = nullptr, ev_copy = nullptr, ev_run = nullptr;
+    // grow-only: the per-image keywords of the last mixed batch (bsgp_solve_batch_rows*).  A buffer of its own, not the
+    // staging arena `stage`: the device entry point has no staging area, and the pinned path's arena is still being filled
+    // on its copy stream when the rows go up on the launch stream.
+    bsgp_params* rows = nullptr; size_t rows_cap = 0;
 };
 
 template <typename T> static const void* conv_kernel_ptr() { return (const void*)bsgp_conv_kernel<T>; }
 
 static void plan_free_pipeline(bsgp_plan* p) {
     cudaFree(p->stage); cudaFree(p->ready); cudaFreeHost(p->ones_host);
-    cudaFree(p->emb_psf); cudaFree(p->emb_img);
-    p->emb_psf = p->emb_img = nullptr; p->emb_psf_cap = p->emb_img_cap = 0;
+    cudaFree(p->emb_psf); cudaFree(p->emb_img); cudaFree(p->rows);
+    p->emb_psf = p->emb_img = nullptr; p->emb_psf_cap = p->emb_img_cap = 0; p->rows = nullptr; p->rows_cap = 0;
     if (p->ev_last) { cudaEventDestroy(p->ev_last); p->ev_last = nullptr; }
     p->stage = nullptr; p->stage_cap = 0; p->ready = nullptr; p->ones_host = nullptr; p->ready_cap = 0;
     if (p->s_copy) cudaStreamDestroy(p->s_copy);
@@ -587,14 +592,18 @@ template <typename T> static int set_psf_wrapped(bsgp_plan* p, const void* psf_d
     return BSGP_OK;
 }
 
+// The keywords of one solve: `prm` holds the batch-level fields (the operator, and everything else when rows is NULL);
+// `rows` (or NULL) one bsgp_params per image; trace_stride the per-image stride of the trace outputs (bsgp_rows.h).
+struct Keywords { const bsgp_params* prm; const bsgp_params* rows; int trace_stride; };
+
 template <typename T>
-static int solve_grid(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready);
+static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready);
 
 // wrapped plans: move the caller's arrays onto the grid, solve there with the image window as the valid region (the
 // zero-padded operator's masked kernels) and the fold of the geometry, crop the restored images
 template <typename T>
-static int solve_t(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready) {
-    if (!p->embedded) return solve_grid<T>(p, prm, batch, in, out, st, ready);
+static int solve_t(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready) {
+    if (!p->embedded) return solve_grid<T>(p, kw, batch, in, out, st, ready);
     const size_t gb = (size_t)batch * p->ny * p->nx * sizeof(T);
     const int narr = 2 + (in->bkg_is_image ? 1 : 0) + (in->x0 ? 1 : 0) + (in->obj ? 1 : 0);
     int rc = grow(&p->emb_img, &p->emb_img_cap, (size_t)narr * gb);
@@ -614,17 +623,18 @@ static int solve_t(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_i
     if ((rc = up(in->x0, &gi.x0))) return rc;
     if ((rc = up(in->obj, &gi.obj))) return rc;
     go.x = base + (size_t)(k++) * gb;
-    bsgp_params q = *prm;
+    bsgp_params q = *kw.prm;
     q.region[0] = 0; q.region[1] = p->img_ny; q.region[2] = 0; q.region[3] = p->img_nx;
     q.div_a = q.div_at = 1.0;
     q.adjoint_second_psf = 1;
-    rc = solve_grid<T>(p, &q, batch, &gi, &go, st, ready);
+    rc = solve_grid<T>(p, Keywords{&q, kw.rows, kw.trace_stride}, batch, &gi, &go, st, ready);
     if (rc) return rc;
     return crop_images<T>(p, go.x, out->x, (size_t)batch, st);
 }
 
 template <typename T>
-static int solve_grid(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready) {
+static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready) {
+    const bsgp_params* prm = kw.prm;
     SolveArgs<T> a;
     memset(&a, 0, sizeof a);
     a.p = *prm; a.g = p->g; a.batch = batch;
@@ -640,11 +650,13 @@ static int solve_grid(bsgp_plan* p, const bsgp_params* prm, int batch, const bsg
     a.tr_beta = out->trace_beta; a.tr_trials = out->trace_trials; a.tr_evals = out->trace_evals;
     a.queue = p->queue;
     a.ready = p->frame ? nullptr : ready;
+    const RowArgs ra{kw.rows, kw.trace_stride};
+    const RowArgs* rows = kw.rows ? &ra : nullptr;                  // no rows: the kernels compiled without them
     if (p->frame) {
         LaunchCfg fc{p->g.G, 512, 1, p->smem_bytes, st, 1};
         const bool mk = prm->region[1] > prm->region[0];
         count_launch();
-        cudaError_t fe = mk ? launch_frame<T, true>(fc, a, p->sp, p->tf_stride, p->gpart) : launch_frame<T, false>(fc, a, p->sp, p->tf_stride, p->gpart);
+        cudaError_t fe = mk ? launch_frame<T, true>(fc, a, p->sp, p->tf_stride, p->gpart, rows) : launch_frame<T, false>(fc, a, p->sp, p->tf_stride, p->gpart, rows);
         if (fe != cudaSuccess) return fail(BSGP_E_CUDA, "frame kernel launch failed: %s", cudaGetErrorString(fe));
         return BSGP_OK;
     }
@@ -653,22 +665,12 @@ static int solve_grid(bsgp_plan* p, const bsgp_params* prm, int batch, const bsg
     LaunchCfg lc{nclu * p->g.G, p->threads, p->g.G, p->smem_bytes, st, p->minb};
     const bool mk = prm->region[1] > prm->region[0];
     count_launch();
-    cudaError_t e = mk ? launch_solve<T, true>(lc, a, p->sp, p->tf_stride) : launch_solve<T, false>(lc, a, p->sp, p->tf_stride);
+    cudaError_t e = mk ? launch_solve<T, true>(lc, a, p->sp, p->tf_stride, rows) : launch_solve<T, false>(lc, a, p->sp, p->tf_stride, rows);
     if (e != cudaSuccess) return fail(BSGP_E_CUDA, "solve kernel launch failed: %s", cudaGetErrorString(e));
     return BSGP_OK;
 }
 
 static inline bool misaligned(const void* p) { return ((uintptr_t)p & 15) != 0; }
-
-static int check_params(const bsgp_params* q) {
-    if (q->divergence != BSGP_DIV_KL && q->divergence != BSGP_DIV_BETA) return fail(BSGP_E_ARG, "bad divergence");
-    if (q->init_recon < 0 || q->init_recon > 3) return fail(BSGP_E_ARG, "init_recon must be 0..3");
-    if (q->proj_type < 0 || q->proj_type > 1) return fail(BSGP_E_ARG, "proj_type must be 0 or 1");
-    if (q->stop_criterion < 0 || q->stop_criterion > 4) return fail(BSGP_E_ARG, "stop_criterion must be 0..4");
-    if (q->maxit < 1) return fail(BSGP_E_ARG, "MAXIT must be >= 1");
-    if (q->m < 1 || q->m > kMaxMem || q->m_alpha < 1 || q->m_alpha > kMaxMem) return fail(BSGP_E_ARG, "M and M_alpha must be in 1..%d", kMaxMem);
-    return BSGP_OK;
-}
 
 static int adjoint_on_wrapped_plan() {
     return fail(BSGP_E_STATE, "bsgp_set_psf_adjoint: a plan whose sides are not powers of two builds both kernels in bsgp_set_psf");
@@ -801,20 +803,21 @@ int bsgp_set_psf_adjoint(bsgp_plan* p, const void* psf_dev, int n_psf, void* str
 int bsgp_set_psf_host(bsgp_plan* p, const void* psf_host, int n_psf) { return set_psf_host(p, psf_host, n_psf, false); }
 int bsgp_set_psf_adjoint_host(bsgp_plan* p, const void* psf_host, int n_psf) { return set_psf_host(p, psf_host, n_psf, true); }
 
-// Argument checks of every solve entry point.  The host entry points run them on the caller's pointers before they size
-// anything from batch or prm->maxit (the device copies they stage are present exactly where the caller's arrays are),
-// and they can read the queue order: the kernel indexes the images with it, so every entry must lie in 0..batch-1.
-static int check_solve(const bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, bool host) {
+// Argument checks of every solve entry point; they fill kw (rows: rows[0] holds the batch-level fields).  The host entry
+// points run them on the caller's pointers before they size anything from batch or the trace stride (the device copies
+// they stage are present exactly where the caller's arrays are), and they can read the queue order: the kernel indexes
+// the images with it, so every entry must lie in 0..batch-1.
+static int check_solve(const bsgp_plan* p, const bsgp_params* prm, const bsgp_params* rows, int batch, const bsgp_inputs* in,
+                       const bsgp_outputs* out, bool host, Keywords* kw) {
+    if (rows) prm = rows;
     if (!p || !prm || !in || !out) return fail(BSGP_E_ARG, "NULL argument");
     if (batch < 1) return fail(BSGP_E_ARG, "batch must be >= 1");
-    int rc = check_params(prm);
-    if (rc) return rc;
+    *kw = Keywords{prm, rows, 0};
+    char err[256];
+    int rc = check_batch_params(prm, rows, batch, in, out, &kw->trace_stride, err, sizeof err);
+    if (rc) return fail(rc, "%s", err);
     if (p->n_psf != 1 && p->n_psf != batch) return fail(BSGP_E_STATE, "bsgp_set_psf was called with %d PSFs; need 1 or batch (%d)", p->n_psf, batch);
     if (!in->gn || !in->bkg || !out->x || !out->iters || !out->status || !out->discr || !out->times) return fail(BSGP_E_ARG, "required pointer is NULL");
-    if (prm->has_flux && !in->flux) return fail(BSGP_E_ARG, "has_flux set but inputs.flux is NULL");
-    if (prm->divergence == BSGP_DIV_BETA && !in->beta0) return fail(BSGP_E_ARG, "beta-divergence needs inputs.beta0");
-    if (prm->init_recon == 1 && !in->x0) return fail(BSGP_E_ARG, "init_recon = 1 needs inputs.x0");
-    if (prm->errflag && (!in->obj || !out->err)) return fail(BSGP_E_ARG, "errflag needs inputs.obj and outputs.err");
     if (p->n_psf < 1) return fail(BSGP_E_STATE, "bsgp_set_psf has not been called");
     if (prm->adjoint_second_psf && (p->tf_adj == nullptr || p->n_psf_adj != p->n_psf))
         return fail(BSGP_E_STATE, "adjoint_second_psf set but bsgp_set_psf_adjoint was not called with the same number of PSFs");
@@ -830,22 +833,32 @@ static int check_solve(const bsgp_plan* p, const bsgp_params* prm, int batch, co
     return BSGP_OK;
 }
 
-// launch on device arrays that passed check_solve; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0
-static int solve_launch(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
+// launch on device arrays that passed check_solve; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0.
+// The host rows of a mixed batch go up to the plan's row buffer on the launch's stream, behind the plan's previous launch.
+static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
     if (!p->embedded && (misaligned(in->gn) || misaligned(out->x) || misaligned(in->x0) || misaligned(in->obj) || (in->bkg_is_image && misaligned(in->bkg))))
         return fail(BSGP_E_ARG, "image pointers must be 16-byte aligned (vector loads)");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     int rc = plan_enter(p, st);
     if (rc) return rc;
-    rc = p->dtype == BSGP_F64 ? solve_t<double>(p, prm, batch, in, out, st, ready) : solve_t<float>(p, prm, batch, in, out, st, ready);
+    Keywords dk = kw;
+    if (kw.rows) {
+        const size_t bytes = (size_t)batch * sizeof(bsgp_params);
+        if ((rc = grow((void**)&p->rows, &p->rows_cap, bytes))) return rc;
+        CU(cudaMemcpyAsync(p->rows, kw.rows, bytes, cudaMemcpyHostToDevice, st));
+        dk.rows = p->rows;
+    }
+    rc = p->dtype == BSGP_F64 ? solve_t<double>(p, dk, batch, in, out, st, ready) : solve_t<float>(p, dk, batch, in, out, st, ready);
     if (rc) return rc;
     return plan_leave(p, st);
 }
 
-int bsgp_solve_batch(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
-    const int rc = check_solve(p, prm, batch, in, out, false);
-    return rc ? rc : solve_launch(p, prm, batch, in, out, stream, nullptr);
+static int solve_device(bsgp_plan* p, const bsgp_params* prm, const bsgp_params* rows, int batch, const bsgp_inputs* in,
+                        const bsgp_outputs* out, void* stream) {
+    Keywords kw;
+    const int rc = check_solve(p, prm, rows, batch, in, out, false, &kw);
+    return rc ? rc : solve_launch(p, kw, batch, in, out, stream, nullptr);
 }
 
 // host staging helpers -----------------------------------------------------------------------
@@ -887,9 +900,9 @@ struct HostIO {
     int bkg_is_image;
     void* x_mapped;
 
-    HostIO(const bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* x_mapped_)
+    HostIO(const bsgp_plan* p, int trace_stride, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* x_mapped_)
         : img((size_t)p->img_ny * p->img_nx * p->elem), bkg_is_image(in->bkg_is_image), x_mapped(x_mapped_) {
-        const size_t B = (size_t)batch, tr = (size_t)prm->maxit + 1, imgs = B * img, it8 = B * tr * 8, it4 = B * tr * 4;
+        const size_t B = (size_t)batch, tr = (size_t)trace_stride, imgs = B * img, it8 = B * tr * 8, it4 = B * tr * 4;
         const void* const h[NSLOT] = {in->gn, in->bkg, in->x0, in->obj, in->flux, in->beta0, in->order,
                                       x_mapped ? nullptr : out->x, out->iters, out->status, out->discr, out->times, out->stop_value,
                                       out->err, out->beta_final, out->proj_evals, out->ls_trials, out->scalars,
@@ -906,7 +919,7 @@ struct HostIO {
     }
     bool image(int k) const { return k <= OBJ && (k != BKG || bkg_is_image); }
     // the solve on the staging area at `base`
-    int launch(bsgp_plan* p, const bsgp_params* prm, int batch, char* base, void* stream, const int* ready) const {
+    int launch(bsgp_plan* p, const Keywords& kw, int batch, char* base, void* stream, const int* ready) const {
         auto dev = [&](int k) -> void* { return host[k] ? base + off[k] : nullptr; };
         const bsgp_inputs in = {dev(GN), dev(BKG), bkg_is_image, (const double*)dev(FLUX), (const double*)dev(BETA0), dev(X0), dev(OBJ),
                                 (const int*)dev(ORDER)};
@@ -914,7 +927,7 @@ struct HostIO {
                                   (double*)dev(STOP_VALUE), (double*)dev(ERR), (double*)dev(BETA_FINAL), (int*)dev(PROJ_EVALS),
                                   (int*)dev(LS_TRIALS), (double*)dev(SCALARS), (double*)dev(TRACE_ALPHA), (double*)dev(TRACE_LAMBDA),
                                   (double*)dev(TRACE_BETA), (int*)dev(TRACE_TRIALS), (int*)dev(TRACE_EVALS)};
-        return solve_launch(p, prm, batch, &in, &out, stream, ready);
+        return solve_launch(p, kw, batch, &in, &out, stream, ready);
     }
     // the staged outputs to the caller's arrays, queued on `st`
     int copy_back(const char* base, cudaStream_t st) const {
@@ -925,17 +938,18 @@ struct HostIO {
 };
 
 // pageable host arrays: one staging allocation per call, freed before returning
-int bsgp_solve_batch_host(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
+static int solve_host(bsgp_plan* p, const bsgp_params* prm, const bsgp_params* rows, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
     int rc;
-    TRY(check_solve(p, prm, batch, in, out, true));
+    Keywords kw;
+    TRY(check_solve(p, prm, rows, batch, in, out, true, &kw));
     CU(cudaSetDevice(p->device));
-    const HostIO io(p, prm, batch, in, out, nullptr);
+    const HostIO io(p, kw.trace_stride, batch, in, out, nullptr);
     DevBuf area;
     TRY(area.alloc(true, io.size));
     char* base = (char*)area.d;
     for (int k = 0; k < HostIO::X; ++k)
         if (io.host[k]) CU(cudaMemcpy(base + io.off[k], io.host[k], io.bytes[k], cudaMemcpyHostToDevice));
-    TRY(io.launch(p, prm, batch, base, nullptr, nullptr));
+    TRY(io.launch(p, kw, batch, base, nullptr, nullptr));
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess) return fail(BSGP_E_CUDA, "solve kernel failed: %s", cudaGetErrorString(e));
     TRY(io.copy_back(base, nullptr));
@@ -962,15 +976,17 @@ static bool page_locked(const void* h) {
     return at.type == cudaMemoryTypeHost;
 }
 
-int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
+static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params* rows, int batch, const bsgp_inputs* in,
+                        const bsgp_outputs* out, void* stream) {
     int rc;
-    TRY(check_solve(p, prm, batch, in, out, true));
+    Keywords kw;
+    TRY(check_solve(p, prm, rows, batch, in, out, true, &kw));
     CU(cudaSetDevice(p->device));
     if (!page_locked(in->gn) || !page_locked(out->x) || !page_locked(in->x0) || !page_locked(in->obj) || (in->bkg_is_image && !page_locked(in->bkg)))
         return fail(BSGP_E_ARG, "bsgp_solve_batch_pinned needs page-locked image buffers (cudaHostAlloc / cudaHostRegister / torch pin_memory)");
     void* x_mapped = nullptr;
     CU(cudaHostGetDevicePointer(&x_mapped, out->x, 0));
-    const HostIO io(p, prm, batch, in, out, x_mapped);
+    const HostIO io(p, kw.trace_stride, batch, in, out, x_mapped);
     const size_t img = io.img, B = (size_t)batch;
     // images in the caller's own shape: a plan whose grid differs from it (sides that are not a power of two) moves them
     // to and from the grid on the device (solve_t), which needs all of them resident first, like frame mode
@@ -1035,7 +1051,7 @@ int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, con
     if (rc) { cudaGetLastError(); cudaStreamSynchronize(sc); cudaStreamSynchronize(sr); return rc; }
     // ---- run stream: the kernel.  Launched AFTER the copies are queued, so that a launch made synchronous by a tool
     // (ncu, compute-sanitizer, CUDA_LAUNCH_BLOCKING) cannot wait for flags that nobody has been asked to raise yet.
-    rc = io.launch(p, prm, batch, S, sr, resident_first ? nullptr : p->ready);
+    rc = io.launch(p, kw, batch, S, sr, resident_first ? nullptr : p->ready);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sr); return rc; }
     // ---- small outputs behind the kernel
     TRY(io.copy_back(S, sr));
@@ -1048,6 +1064,26 @@ int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, con
     if (e == cudaSuccess) e = cudaStreamSynchronize(sr);
     if (e != cudaSuccess) return fail(BSGP_E_CUDA, "pipelined solve failed: %s", cudaGetErrorString(e));
     return BSGP_OK;
+}
+
+int bsgp_solve_batch(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
+    return solve_device(p, prm, nullptr, batch, in, out, stream);
+}
+int bsgp_solve_batch_host(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
+    return solve_host(p, prm, nullptr, batch, in, out);
+}
+int bsgp_solve_batch_pinned(bsgp_plan* p, const bsgp_params* prm, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
+    return solve_pinned(p, prm, nullptr, batch, in, out, stream);
+}
+int bsgp_solve_batch_rows(bsgp_plan* p, const bsgp_params* rows, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream) {
+    return solve_device(p, nullptr, rows, batch, in, out, stream);
+}
+int bsgp_solve_batch_rows_host(bsgp_plan* p, const bsgp_params* rows, int batch, const bsgp_inputs* in, const bsgp_outputs* out) {
+    return solve_host(p, nullptr, rows, batch, in, out);
+}
+int bsgp_solve_batch_rows_pinned(bsgp_plan* p, const bsgp_params* rows, int batch, const bsgp_inputs* in, const bsgp_outputs* out,
+                                 void* stream) {
+    return solve_pinned(p, nullptr, rows, batch, in, out, stream);
 }
 
 int bsgp_apply_psf(bsgp_plan* p, const void* x_dev, void* y_dev, int batch, int adjoint, void* stream) {

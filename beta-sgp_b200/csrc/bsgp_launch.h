@@ -8,6 +8,7 @@
 namespace bsgp {
 
 template <typename T> struct SolveArgs;
+struct RowArgs;
 
 struct LaunchCfg {
     int grid, threads, G;
@@ -61,10 +62,12 @@ static inline cudaError_t query_clusters(const void* func, const LaunchCfg& lc, 
     return e;
 }
 
-// defined in bsgp_solve_f64.cu / bsgp_solve_f32.cu (MK = false) and bsgp_solve_f64_padded.cu / bsgp_solve_f32_padded.cu (MK = true)
-template <typename T, bool MK> cudaError_t launch_solve(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride);
+// rows: NULL, or a mixed batch (the ROWS kernels, bsgp_solve_kernel.cuh).  Defined in bsgp_solve_f64.cu / bsgp_solve_f32.cu (MK = false) and bsgp_solve_f64_padded.cu / bsgp_solve_f32_padded.cu (MK = true)
+template <typename T, bool MK> cudaError_t launch_solve(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride,
+                                                  const RowArgs* rows);
 template <typename T, bool MK> cudaError_t query_solve_clusters(const LaunchCfg& lc, int num_sms, int* out);
-template <typename T, bool MK> cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart);
+template <typename T, bool MK> cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart,
+                                                  const RowArgs* rows);
 template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm);
 
 }  // namespace bsgp

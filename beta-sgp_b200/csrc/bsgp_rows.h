@@ -1,0 +1,67 @@
+// Checks of a solve's keywords, shared by libbsgp (bsgp_kernels.cu) and the test-only host emulation: plain C++, no CUDA
+// call.  A batch either shares one bsgp_params or gives every image its own row (bsgp_solve_batch_rows); both go through
+// check_batch_params, which also fixes the per-image stride of the trace outputs.
+#pragma once
+#include <stdio.h>
+#include <string.h>
+
+#include "../../include/bsgp.h"
+#include "bsgp_smem.h"
+
+namespace bsgp {
+
+// One set of keywords and the inputs / outputs it needs.  `where` names the row in messages ("" for a shared set).
+inline int check_params_row(const bsgp_params* q, const bsgp_inputs* in, const bsgp_outputs* out, const char* where, char* err,
+                            size_t errlen) {
+    const char* msg = nullptr;
+    char mem[48];
+    snprintf(mem, sizeof mem, "M and M_alpha must be in 1..%d", kMaxMem);
+    if (q->divergence != BSGP_DIV_KL && q->divergence != BSGP_DIV_BETA) msg = "bad divergence";
+    else if (q->init_recon < 0 || q->init_recon > 3) msg = "init_recon must be 0..3";
+    else if (q->proj_type < 0 || q->proj_type > 1) msg = "proj_type must be 0 or 1";
+    else if (q->stop_criterion < 0 || q->stop_criterion > 4) msg = "stop_criterion must be 0..4";
+    else if (q->maxit < 1) msg = "MAXIT must be >= 1";
+    else if (q->m < 1 || q->m > kMaxMem || q->m_alpha < 1 || q->m_alpha > kMaxMem) msg = mem;
+    else if (q->has_flux && !in->flux) msg = "has_flux set but inputs.flux is NULL";
+    else if (q->divergence == BSGP_DIV_BETA && !in->beta0) msg = "beta-divergence needs inputs.beta0";
+    else if (q->init_recon == 1 && !in->x0) msg = "init_recon = 1 needs inputs.x0";
+    else if (q->errflag && (!in->obj || !out->err)) msg = "errflag needs inputs.obj and outputs.err";
+    if (!msg) return BSGP_OK;
+    snprintf(err, errlen, "%s%s", where, msg);
+    return BSGP_E_ARG;
+}
+
+// The fields that describe the operator and the plan rather than the solve: equal in every row of a batch.
+inline bool same_operator(const bsgp_params* a, const bsgp_params* b) {
+    return memcmp(a->region, b->region, sizeof a->region) == 0 && a->div_a == b->div_a && a->div_at == b->div_at &&
+           a->adjoint_second_psf == b->adjoint_second_psf;
+}
+
+// The keywords of a batch: `prm` shared by all images (rows == NULL), or rows[0 .. batch-1], one per image.  On success
+// *trace_stride is the per-image stride of discr, times, stop_value and trace_* (err: trace_stride + 1), the largest
+// maxit + 1 of the batch.
+inline int check_batch_params(const bsgp_params* prm, const bsgp_params* rows, int batch, const bsgp_inputs* in,
+                              const bsgp_outputs* out, int* trace_stride, char* err, size_t errlen) {
+    if (!rows) {
+        const int rc = check_params_row(prm, in, out, "", err, errlen);
+        if (rc) return rc;
+        *trace_stride = prm->maxit + 1;
+        return BSGP_OK;
+    }
+    int stride = 0;
+    for (int i = 0; i < batch; ++i) {
+        char where[48];
+        snprintf(where, sizeof where, "row %d: ", i);
+        const int rc = check_params_row(&rows[i], in, out, where, err, errlen);
+        if (rc) return rc;
+        if (!same_operator(&rows[i], &rows[0])) {
+            snprintf(err, errlen, "row %d: region, div_a, div_at and adjoint_second_psf describe the operator and must equal row 0's", i);
+            return BSGP_E_ARG;
+        }
+        if (rows[i].maxit + 1 > stride) stride = rows[i].maxit + 1;
+    }
+    *trace_stride = stride;
+    return BSGP_OK;
+}
+
+}  // namespace bsgp

@@ -7,6 +7,7 @@ namespace bsgp {
 constexpr int kMaxWarps = 16;      // 512 threads per CTA at most
 constexpr int kMaxG = 16;
 constexpr int kMaxK = 8;
+constexpr int kMaxMem = 16;        // M and M_alpha: the controller's history lengths (CtlState)
 
 struct SharedCtl {
     double warp_part[2][kMaxWarps][kMaxK];   // two halves (parity bit 0), so that a single-CTA all-reduce needs one barrier only

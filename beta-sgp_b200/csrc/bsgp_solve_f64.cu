@@ -2,8 +2,8 @@
 #include "bsgp_solve_kernel.cuh"
 
 namespace bsgp {
-template cudaError_t launch_solve<double, false>(const LaunchCfg&, const SolveArgs<double>&, const SmemPlan&, size_t);
+template cudaError_t launch_solve<double, false>(const LaunchCfg&, const SolveArgs<double>&, const SmemPlan&, size_t, const RowArgs*);
 template cudaError_t query_solve_clusters<double, false>(const LaunchCfg&, int, int*);
-template cudaError_t launch_frame<double, false>(const LaunchCfg&, const SolveArgs<double>&, const SmemPlan&, size_t, double*);
+template cudaError_t launch_frame<double, false>(const LaunchCfg&, const SolveArgs<double>&, const SmemPlan&, size_t, double*, const RowArgs*);
 template cudaError_t query_frame_ctas<double, false>(const LaunchCfg&, int*);
 }  // namespace bsgp

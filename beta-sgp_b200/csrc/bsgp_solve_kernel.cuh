@@ -69,12 +69,20 @@ __device__ __forceinline__ ImgState<T>* solve_prologue(Ctx& ctx, unsigned char* 
     return S;
 }
 
-template <typename T, int NT, int MINB, bool MK>
-__global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride) {
+// ROWS: a mixed batch (RowArgs, bsgp_solver.cuh).  The kernels without rows take no RowArgs and compile to the same code as
+// before the feature existed.
+// The ROWS kernels run their execution context as RowCtx<Ctx>, so every phase and helper they call is an instantiation of
+// its own: ptxas allocates the functions that the kernels without rows call exactly as it did before (callees shared by
+// both kernels would be allocated for both callers).
+template <class Ctx> struct RowCtx : Ctx {};
+template <bool ROWS, class Ctx> using CtxOf = typename std::conditional<ROWS, RowCtx<Ctx>, Ctx>::type;
+
+template <typename T, int NT, int MINB, bool MK, bool ROWS, typename... R>
+__global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, const R... ra) {
     unsigned char* smem = dyn_smem();
     // 2 CTAs x 256 threads and 3 CTAs x 128 threads per SM are the configurations of images that are resident in shared memory
     // (bsgp_plan.h, plan_launch)
-    typename std::conditional<(NT == 256 && MINB == 2) || (NT == 128 && MINB == 3), DeviceCtxSmall, DeviceCtx>::type ctx;
+    CtxOf<ROWS, typename std::conditional<(NT == 256 && MINB == 2) || (NT == 128 && MINB == 3), DeviceCtxSmall, DeviceCtx>::type> ctx;
     static_cast<DeviceCtx&>(ctx) = make_ctx(reinterpret_cast<SharedCtl*>(smem), a.g.G);
     T* buf[NBUF];
     ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
@@ -89,59 +97,74 @@ __global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T>
         }
         cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)img * tf_stride : 0);
         cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)img * tf_stride : 0) : tf;
-        solve_image<T, MK>(ctx, a, S, buf, tf, tfa, img);
+        solve_image<T, MK, ROWS>(ctx, a, S, buf, tf, tfa, img, ra...);
     }
 }
 
 // Frame mode (GridCtx): the images of the batch are restored one after the other, each by the whole grid.
-template <typename T, bool MK>
-__global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart) {
+template <typename T, bool MK, bool ROWS, typename... R>
+__global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart,
+                                                            const R... ra) {
     unsigned char* smem = dyn_smem();
-    GridCtx ctx = make_grid_ctx(reinterpret_cast<SharedCtl*>(smem), gpart);
+    CtxOf<ROWS, GridCtx> ctx;
+    static_cast<GridCtx&>(ctx) = make_grid_ctx(reinterpret_cast<SharedCtl*>(smem), gpart);
     T* buf[NBUF];
     ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
     for (int img = 0; img < a.batch; ++img) {
         cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)img * tf_stride : 0);
         cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)img * tf_stride : 0) : tf;
-        solve_image<T, MK>(ctx, a, S, buf, tf, tfa, img);
+        solve_image<T, MK, ROWS>(ctx, a, S, buf, tf, tfa, img, ra...);
         ctx.cluster_sync();          // the scratch arrays and the exchange buffer are reused by the next image
     }
 }
 
+// frame_kernel_ptr / solve_kernel_ptr: the kernel without rows, or with a RowArgs parameter
+template <typename T, bool MK, bool ROWS> static const void* frame_kernel_ptr() {
+    if constexpr (ROWS) return (const void*)bsgp_frame_kernel<T, MK, true, RowArgs>;
+    else return (const void*)bsgp_frame_kernel<T, MK, false>;
+}
+
 template <typename T, bool MK>
-cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart) {
+cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart, const RowArgs* rows) {
     SolveArgs<T> args = a;
     SmemPlan plan = sp;
     size_t tfs = tf_stride;
     double* gp = gpart;
-    void* params[] = {&args, &plan, &tfs, &gp};
-    const void* fn = (const void*)bsgp_frame_kernel<T, MK>;
+    RowArgs ra = rows ? *rows : RowArgs{};
+    void* params[] = {&args, &plan, &tfs, &gp, &ra};
+    const void* fn = rows ? frame_kernel_ptr<T, MK, true>() : frame_kernel_ptr<T, MK, false>();
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc.smem);
     if (e != cudaSuccess) return e;
     return cudaLaunchCooperativeKernel(fn, dim3(lc.grid), dim3(lc.threads), params, lc.smem, lc.stream);
 }
 
 template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm) {
-    const void* fn = (const void*)bsgp_frame_kernel<T, MK>;
+    const void* fn = frame_kernel_ptr<T, MK, false>();
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc.smem);
     if (e != cudaSuccess) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, fn, lc.threads, lc.smem);
 }
 
 // register budgets: 512 x 128, 256 x 255 (one CTA per SM), 256 x 128 (two CTAs per SM), 128 x 168 (three), 128 x 128 (four)
-template <typename T, bool MK> static const void* solve_kernel_ptr(int threads, int minb) {
-    if (threads <= 128) return minb >= 4 ? (const void*)bsgp_solve_kernel<T, 128, 4, MK> : (const void*)bsgp_solve_kernel<T, 128, 3, MK>;
-    if (threads <= 256) return minb >= 2 ? (const void*)bsgp_solve_kernel<T, 256, 2, MK> : (const void*)bsgp_solve_kernel<T, 256, 1, MK>;
-    return (const void*)bsgp_solve_kernel<T, 512, 1, MK>;
+template <typename T, int NT, int MINB, bool MK, bool ROWS> static const void* solve_kernel_fn() {
+    if constexpr (ROWS) return (const void*)bsgp_solve_kernel<T, NT, MINB, MK, true, RowArgs>;
+    else return (const void*)bsgp_solve_kernel<T, NT, MINB, MK, false>;
+}
+template <typename T, bool MK, bool ROWS = false> static const void* solve_kernel_ptr(int threads, int minb) {
+    if (threads <= 128) return minb >= 4 ? solve_kernel_fn<T, 128, 4, MK, ROWS>() : solve_kernel_fn<T, 128, 3, MK, ROWS>();
+    if (threads <= 256) return minb >= 2 ? solve_kernel_fn<T, 256, 2, MK, ROWS>() : solve_kernel_fn<T, 256, 1, MK, ROWS>();
+    return solve_kernel_fn<T, 512, 1, MK, ROWS>();
 }
 
 template <typename T, bool MK>
-cudaError_t launch_solve(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride) {
+cudaError_t launch_solve(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, const RowArgs* rows) {
     SolveArgs<T> args = a;
     SmemPlan plan = sp;
     size_t tfs = tf_stride;
-    void* params[] = {&args, &plan, &tfs};
-    return launch_clustered(solve_kernel_ptr<T, MK>(lc.threads, lc.minb), lc, params);
+    RowArgs ra = rows ? *rows : RowArgs{};
+    void* params[] = {&args, &plan, &tfs, &ra};
+    const void* fn = rows ? solve_kernel_ptr<T, MK, true>(lc.threads, lc.minb) : solve_kernel_ptr<T, MK, false>(lc.threads, lc.minb);
+    return launch_clustered(fn, lc, params);
 }
 
 template <typename T, bool MK> cudaError_t query_solve_clusters(const LaunchCfg& lc, int num_sms, int* out) {

@@ -25,9 +25,12 @@
 //   * den^beta = den^(beta-1) * den and den^(beta-2) = den^(beta-1) / den (one pow per pixel),
 //   * reductions are tree sums in fp64 (numpy: pairwise / BLAS dot).
 #pragma once
+#include <type_traits>
+
 #include "../../include/bsgp.h"
 #include "bsgp_conv.cuh"
 #include "bsgp_project.cuh"
+#include "bsgp_smem.h"
 
 #ifndef BSGP_U_TRIAL
 #define BSGP_U_TRIAL 2
@@ -42,7 +45,6 @@
 namespace bsgp {
 
 enum Buf { B_GN = 0, B_BKG, B_X, B_G, B_XTF, B_D, B_DTF, B_T1, NBUF };
-constexpr int kMaxMem = 16;
 
 template <typename T> struct SolveArgs {
     bsgp_params p;
@@ -62,6 +64,16 @@ template <typename T> struct SolveArgs {
     int* queue;
     const int* ready;               // [batch] or NULL: queue item i may start once ready[i] != 0 (pipelined upload, bsgp_solve_batch_pinned)
 };
+
+// A mixed batch (bsgp_solve_batch_rows): image i solves with its own keywords rows[i] (device, [batch]); the operator fields
+// (region, divisors, adjoint kernel) still come from SolveArgs::p.  trace_stride: the per-image stride of discr / times /
+// stop_value / trace_* (err: + 1), the largest maxit + 1 of the rows.  Only the ROWS kernels take it: a launch without rows
+// runs kernels compiled exactly as before the feature existed.
+struct RowArgs { const bsgp_params* rows; int trace_stride; };
+struct NoRow {};
+// the keywords the controller reads: the image's own copy of its row, or the batch's
+BSGP_DEV const bsgp_params& image_params(const bsgp_params& own, const bsgp_params&) { return own; }
+BSGP_DEV const bsgp_params& image_params(const NoRow&, const bsgp_params& shared) { return shared; }
 
 // Per-image constants of one CTA (shared memory).  Pointers address this CTA's slab of each array.
 template <typename T> struct ImgState {
@@ -737,7 +749,8 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE RfOut rootfind_call(Ctx 
 
 // Barzilai-Borwein steps and their alternation, learning-rate schedule, bookkeeping and stop rules of one iteration
 // (sgp.py:366-425 / 818-882).  bb: the seven all-reduced sums of ph_ri_bb.  Returns the value compared with tol.
-template <typename T> BSGP_NOINLINE double ctl_finish_iteration(const bsgp_params* Pp, CtlState<T>* W, R7 bbr) {
+// ROWS only separates the instantiations of the kernels with and without rows (bsgp_solve_kernel.cuh, RowCtx)
+template <typename T, bool ROWS = false> BSGP_NOINLINE double ctl_finish_iteration(const bsgp_params* Pp, CtlState<T>* W, R7 bbr) {
     const bsgp_params& P = *Pp;
     const double* bb = bbr.v;
     const int MA = P.m_alpha;
@@ -790,16 +803,27 @@ template <typename T, class Ctx> BSGP_NOINLINE void ctl_accept_step(Ctx ctx, Img
     if (keep_going) { T* t = S->x; S->x = S->d; S->d = t; }
 }
 
-template <typename T, bool MK, class Ctx>
-BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* const* buf, cplx<T>* tf, cplx<T>* tf_adj, int img) {
-    const bsgp_params& P = a.p;
+template <typename T, bool MK, bool ROWS = false, class Ctx>
+BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* const* buf, cplx<T>* tf, cplx<T>* tf_adj, int img,
+                          const RowArgs& ra = RowArgs{}) {
+    // A mixed batch: every thread keeps its own copy of the image's row, in local memory (its address reaches
+    // ctl_finish_iteration), the way a launch without rows reads SolveArgs::p.  The operator fields are equal in every row
+    // (bsgp_rows.h) and always come from a.p, where a wrapped plan sets them for its grid.
+    typename std::conditional<ROWS, bsgp_params, NoRow>::type own;
+    if constexpr (ROWS) {
+        own = ra.rows[img];
+        for (int k = 0; k < 4; ++k) own.region[k] = a.p.region[k];
+        own.div_a = a.p.div_a; own.div_at = a.p.div_at; own.adjoint_second_psf = a.p.adjoint_second_psf;
+    }
+    const bsgp_params& P = image_params(own, a.p);
     CtlState<T>* W = ctx.template ctl<CtlState<T>>();
     constexpr bool masked = MK;                                          // zero-padded operator: the image is a window of the grid
     const bool leader = (ctx.rank == 0 && ctx.tid == 0);
     const bool pflag = P.proj_type == 1;
     const bool is_beta = P.divergence == BSGP_DIV_BETA;
     const bool want_err = P.errflag && a.obj != nullptr && a.err != nullptr;
-    const size_t toff = (size_t)img * (P.maxit + 1);
+    const size_t stride = ROWS ? (size_t)ra.trace_stride : (size_t)(P.maxit + 1);
+    const size_t toff = (size_t)img * stride;
 
     ctx.sync();                      // the previous image's last phase may still be reading S
     {
@@ -891,7 +915,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         double e2[2] = {e.a, e.b};
         allreduce_fn<0, 2>(ctx, e2);
         W->truth_sq = e2[1];
-        if (leader) a.err[(size_t)img * (P.maxit + 2)] = sqrt(e2[0] / e2[1]);
+        if (leader) a.err[(size_t)img * (stride + 1)] = sqrt(e2[0] / e2[1]);
     }
 
     W->beta_p = is_beta ? a.beta0[img] : 1.0;
@@ -1032,7 +1056,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         allreduce_fn<0, 7>(ctx, bbr.v);
 
         // ---- Barzilai-Borwein steps, lr schedule, bookkeeping and stop rules (:366-425)
-        const double stop_val = ctl_finish_iteration<T>(&a.p, W, bbr);
+        const double stop_val = ctl_finish_iteration<T, ROWS>(&P, W, bbr);
         if (leader) {
             const int iter = W->iter;
             const size_t o = toff + (size_t)(iter - 1);
@@ -1044,7 +1068,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
             if (a.tr_beta) a.tr_beta[o] = W->beta_p;
             if (a.tr_trials) a.tr_trials[o] = W->trials;
             if (a.tr_evals) a.tr_evals[o] = W->evals;
-            if (want_err && iter <= P.maxit + 1) a.err[(size_t)img * (P.maxit + 2) + iter] = sqrt(bbr.v[6] / W->truth_sq);   // :394-396
+            if (want_err && iter <= P.maxit + 1) a.err[(size_t)img * (stride + 1) + iter] = sqrt(bbr.v[6] / W->truth_sq);   // :394-396
         }
         ctl_accept_step<T>(ctx, S, W->keep_going);
     }

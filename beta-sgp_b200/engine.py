@@ -25,6 +25,8 @@ _DT = {"float64": _capi.BSGP_F64, "float32": _capi.BSGP_F32}
 _SOLVER_KEYS = ("region", "div_a", "div_at", "adjoint_second_psf", "init_recon", "proj_type", "stop_criterion", "MAXIT", "gamma", "beta", "alpha", "alpha_min", "alpha_max",
                 "M_alpha", "tau", "M", "max_projs", "verbose", "ccd_sat_level", "scale_data", "errflag",
                 "tol_convergence", "adapt_beta", "lr", "lr_exp_param", "schedule_lr")
+_ROW_KEYS = ("divergence", "betaParam", "flux") + _SOLVER_KEYS         # what one entry of solve_batch(per_image=...) may set
+_OPERATOR_KEYS = ("region", "div_a", "div_at", "adjoint_second_psf")
 
 
 class Plan:
@@ -183,12 +185,18 @@ class BatchResult:
     trace: dict | None = None
 
 
-def _queue_order(divergence, beta0):
+def _queue_order(divergence, beta0, is_beta=None):
     """Order in which the persistent clusters pull images from the work queue.  Iteration counts of beta-SGP
     grow as beta approaches 1 (28..162 iterations over the reference's five beta initialisations,
     application_sgp_subdivisions.py:69-107), so the images with the smallest |beta - 1| go first: the long
-    solves do not end up alone at the tail of the queue.  Results do not depend on the order."""
-    if divergence != "beta" or beta0.size < 2 or np.all(beta0 == beta0[0]):
+    solves do not end up alone at the tail of the queue.  A mixed batch (is_beta: per image) hands out its beta-SGP
+    images in that order, then its KL images.  Results do not depend on the order."""
+    if is_beta is not None and not is_beta.all():
+        if not is_beta.any():
+            return None
+        key = np.where(is_beta, np.abs(beta0 - 1.0), np.inf)
+        return np.ascontiguousarray(np.argsort(key, kind="stable").astype(np.int32))
+    if (divergence != "beta" and is_beta is None) or beta0.size < 2 or np.all(beta0 == beta0[0]):
         return None
     return np.ascontiguousarray(np.argsort(np.abs(beta0 - 1.0), kind="stable").astype(np.int32))
 
@@ -233,6 +241,45 @@ def _params(divergence, kw, has_flux):
     if unknown:
         raise TypeError(f"unexpected keyword argument(s): {sorted(unknown)}")
     return _capi.make_params(DIV_KL if divergence == "kl" else DIV_BETA, has_flux=has_flux, **kw)
+
+
+def _check_per_image(per_image, B):
+    """per_image: B dicts of divergence / betaParam / flux / solver keywords (see solve_batch)."""
+    if not isinstance(per_image, (list, tuple)) or len(per_image) != B:
+        raise ValueError(f"per_image must be a list of {B} dicts, one per image")
+    for i, row in enumerate(per_image):
+        if not isinstance(row, dict):
+            raise ValueError(f"per_image[{i}] must be a dict of keyword arguments")
+        unknown = set(row) - set(_ROW_KEYS)
+        if unknown:
+            raise TypeError(f"per_image[{i}]: unexpected keyword argument(s): {sorted(unknown)}")
+        if row.get("divergence", "kl") not in ("kl", "beta"):
+            raise ValueError(f"per_image[{i}]: divergence must be 'kl' or 'beta'")
+
+
+def _row_betas(betaParam, per_image, B):
+    """The call's betaParam with the per-image overrides of per_image, as a host [B] array; betaParam itself if no row
+    sets one (a device tensor then stays on the device)."""
+    if not any("betaParam" in row for row in per_image):
+        return betaParam
+    base = betaParam.detach().cpu().numpy() if _is_tensor(betaParam) else betaParam
+    b = np.array(np.broadcast_to(np.asarray(base, dtype=np.float64).reshape(-1), (B,)))
+    for i, row in enumerate(per_image):
+        if "betaParam" in row:
+            b[i] = float(row["betaParam"])
+    return b
+
+
+def _row_flux(flux, per_image, B):
+    """(flux, per_image) with the per-image overrides of per_image: a row's "flux" (a number, or None for
+    sum(gn - bkg)) replaces the call's for that image.  If any row sets one, the flux comes back as a host [B] array and
+    every row carries its own "flux" entry; otherwise both come back unchanged."""
+    if not any("flux" in row for row in per_image):
+        return flux, per_image
+    base = None if flux is None else np.broadcast_to(np.asarray(flux.detach().cpu().numpy() if _is_tensor(flux) else flux,
+                                                                 dtype=np.float64).reshape(-1), (B,))
+    rows = [dict(row) if "flux" in row else dict(row, flux=None if base is None else float(base[i])) for i, row in enumerate(per_image)]
+    return np.array([0.0 if row["flux"] is None else float(row["flux"]) for row in rows]), rows
 
 
 # The solve's outputs besides the restored images, in the order of struct bsgp_outputs: (field, shape for B images and
@@ -293,9 +340,16 @@ class _Args:
     `vector(a, B, dtype)` (a scalar or [B] array as a contiguous [B] array of a numpy dtype) and `alloc(shape, dtype)`."""
 
     def __init__(self, gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, *, psf_arg, image,
-                 vector, alloc):
+                 vector, alloc, per_image=None):
         B = self.B = gn.shape[0]
         self.params = p = _params(divergence, kw, flux is not None)
+        # a mixed batch: one bsgp_params per image, its own keywords merged over the call's (betaParam: see _row_betas)
+        self.rows, self.is_beta, rows = None, None, [p]
+        if per_image is not None:
+            rows = [_params(r.get("divergence", divergence), {**kw, **{k: v for k, v in r.items() if k not in ("divergence", "betaParam", "flux")}},
+                            r["flux"] is not None if "flux" in r else flux is not None) for r in per_image]
+            self.rows = (_capi.Params * B)(*rows)
+            self.is_beta = np.array([r.divergence == DIV_BETA for r in rows])
         if not psf_is_set and plan.set_psf(psf_arg(psf)) not in (1, B):
             raise ValueError("psf must be one image or one per batch entry")
         self.gn, self.bkg_img, self.trace = gn, int(_ndim(bkg) == 3), trace
@@ -304,10 +358,11 @@ class _Args:
         self.beta0 = vector(betaParam, B, np.float64)
         self.x0 = None if x0 is None else image(x0, "x0")
         self.obj = None if obj is None else image(obj, "obj")
-        if p.init_recon == 1 and self.x0 is None:
+        if any(r.init_recon == 1 for r in rows) and self.x0 is None:
             raise ValueError("init_recon=1 needs x0 (the sgp()/sgp_betaDiv() wrappers draw it with seed 42)")
-        present = {None: True, "errflag": bool(p.errflag), "trace": bool(trace)}
-        self.out = {f: alloc(shape(B, p.maxit + 1), dt) if present[when] else None for f, shape, dt, when in _OUTPUTS}
+        present = {None: True, "errflag": any(r.errflag for r in rows), "trace": bool(trace)}
+        stride = max(r.maxit for r in rows) + 1                 # the library's trace stride (include/bsgp.h, bsgp_outputs)
+        self.out = {f: alloc(shape(B, stride), dt) if present[when] else None for f, shape, dt, when in _OUTPUTS}
 
     def structs(self, x, order):
         """_capi.Inputs / _capi.Outputs for restored images `x` and the work-queue order (None: natural order).  The
@@ -317,6 +372,15 @@ class _Args:
                           _ptr(self.obj), _ptr(order))
         return ci, _capi.Outputs(_ptr(x), *(_ptr(a) for a in self.out.values()))
 
+    def solve(self, plan, entry, ci, co, *stream):
+        """bsgp_solve_batch<entry> with the shared keywords, or its bsgp_solve_batch_rows<entry> twin for a mixed batch."""
+        L = lib()
+        if self.rows is None:
+            fn, prm = getattr(L, "bsgp_solve_batch" + entry), C.byref(self.params)
+        else:
+            fn, prm = getattr(L, "bsgp_solve_batch_rows" + entry), self.rows
+        check(fn(plan.handle, prm, self.B, C.byref(ci), C.byref(co), *stream))
+
     def result(self, x):
         out = dict(self.out)
         trace = {key: out.pop(f) for f, key in _TRACE_KEYS.items()}
@@ -324,7 +388,7 @@ class _Args:
 
 
 def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=None, obj=None, dtype="float64",
-                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, **kw):
+                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, per_image=None, **kw):
     """Restore a batch of independent images in one persistent kernel launch.
 
     gn [B,ny,nx]; psf [ny,nx] (shared) or [B,ny,nx]; bkg scalar, [B] or [B,ny,nx]; flux None or [B];
@@ -334,29 +398,43 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
     (upload, solve and download overlap; see bsgp_solve_batch_pinned in include/bsgp.h; ``x_out`` may name a
     pinned tensor that receives the restored images, so that a caller in a loop reuses its buffer); pageable CPU tensors
     are treated like numpy arrays.  ``padded=True`` selects the zero-padded operator of
-    use_original_SGP_Afunction=False (sgp.py:121-161): images of any size, kernel of any (smaller or equal) size."""
+    use_original_SGP_Afunction=False (sgp.py:121-161): images of any size, kernel of any (smaller or equal) size.
+
+    ``per_image``: a list of B dicts, one per image, of ``divergence``, ``betaParam``, ``flux`` and any solver keyword, each merged
+    over the call's own: images with different keywords (KL and beta-SGP, stop rule, MAXIT, projection, saturation, ...)
+    share one launch, and image i is exactly the solve of that image alone with its merged keywords.  The trace outputs
+    are then [B, max MAXIT + 1]; entries past an image's own iteration count stay zero.  Keywords that describe the
+    operator (region, div_a, div_at, adjoint_second_psf) must be the same in every row."""
     if divergence not in ("kl", "beta"):
         raise ValueError("divergence must be 'kl' or 'beta'")
+    if per_image is not None:
+        _check_per_image(per_image, int(gn.shape[0]))
+        betaParam = _row_betas(betaParam, per_image, int(gn.shape[0]))
+        flux, per_image = _row_flux(flux, per_image, int(gn.shape[0]))
     if padded:
         if _is_tensor(gn) and not gn.is_cuda:             # CPU tensors (pinned or not) take the numpy route of the padded operator
             def host(a):
                 return a.numpy() if _is_tensor(a) and not a.is_cuda else a
             gn, psf, bkg, flux, betaParam, x0, obj = (host(a) for a in (gn, psf, bkg, flux, betaParam, x0, obj))
             x_out = None
-        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, kw)
+        if per_image is not None and any(k in row for row in per_image for k in _OPERATOR_KEYS):
+            raise ValueError("per_image rows of the padded operator share its geometry: region, div_a, div_at and "
+                             "adjoint_second_psf are set by padded=True")
+        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, kw)
     if x_out is not None and not (_is_tensor(gn) and not gn.is_cuda and gn.is_pinned()):
         raise ValueError("x_out is only supported with pinned CPU tensor inputs")
     if _is_tensor(gn) and not gn.is_cuda and gn.is_pinned():
-        return _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, kw)
+        return _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image,
+                                   kw)
     if _is_tensor(gn) and gn.is_cuda:
-        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw)
+        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, kw)
     if _is_tensor(gn):                                    # pageable CPU tensor: the plain host path
         gn = gn.numpy()
         psf, bkg, flux, betaParam, x0, obj = (a.numpy() if _is_tensor(a) and not a.is_cuda else a for a in (psf, bkg, flux, betaParam, x0, obj))
-    return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, kw)
+    return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, kw)
 
 
-def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, kw):
+def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, kw):
     """Embed into the padded grid, solve there with the window mask, crop (see PaddedGeometry).  numpy inputs give
     numpy outputs; CUDA-tensor images stay on the device (the small kernels may be numpy or tensors)."""
     on_dev = _is_tensor(gn)
@@ -388,13 +466,13 @@ def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtyp
         res = solve_batch(geo.embed(gn, dt), None, geo.embed(bkg, dt) if _ndim(bkg) == 3 else bkg, divergence=divergence,
                           flux=flux, betaParam=betaParam, x0=None if x0 is None else geo.embed(x0, dt),
                           obj=None if obj is None else geo.embed(obj, dt), dtype=dtype, device=device, trace=trace, plan=plan,
-                          psf_is_set=True, **extra, **kw)
+                          psf_is_set=True, per_image=per_image, **extra, **kw)
     x = res.x[:, geo.rows, geo.cols]
     res.x = x.contiguous() if on_dev else np.ascontiguousarray(x)
     return res
 
 
-def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, kw):
+def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, kw):
     """numpy arrays -> numpy arrays; one call of bsgp_solve_batch_host."""
     npdt = _NP[dtype]
     gn = np.ascontiguousarray(gn, dtype=npdt)
@@ -407,14 +485,14 @@ def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype,
         return a
 
     args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw,
-                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros)
+                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros, per_image=per_image)
     x = np.empty(gn.shape, npdt)
-    ci, co = args.structs(x, _queue_order(divergence, args.beta0))
-    check(lib().bsgp_solve_batch_host(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co)))
+    ci, co = args.structs(x, _queue_order(divergence, args.beta0, args.is_beta))
+    args.solve(plan, "_host", ci, co)
     return args.result(x)
 
 
-def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw):
+def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, kw):
     """CUDA tensors -> CUDA tensors, asynchronous on the current stream: no host synchronisation, no host copies."""
     import torch
     if not gn.is_cuda:
@@ -445,20 +523,26 @@ def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trac
 
     with torch.cuda.device(dev):
         args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
-                     image=image, vector=vector, alloc=lambda shape, dt: torch.zeros(shape, dtype=_torch_dtype(dt), device=dev))
+                     image=image, vector=vector, alloc=lambda shape, dt: torch.zeros(shape, dtype=_torch_dtype(dt), device=dev),
+                     per_image=per_image)
         x = torch.empty_like(gn)
         order = None
-        if divergence == "beta" and args.B > 1:
+        if args.is_beta is not None and args.is_beta.any() and args.B > 1:
+            # mixed batch: beta-SGP images by |beta - 1|, then the KL images (see _queue_order)
+            kl = torch.as_tensor(~args.is_beta, device=dev)
+            key = torch.where(kl, torch.full_like(args.beta0, float("inf")), (args.beta0 - 1.0).abs())
+            order = torch.argsort(key, stable=True).to(torch.int32)
+        elif args.is_beta is None and divergence == "beta" and args.B > 1:
             # longest expected solve first (see _queue_order); computed on the device, no host sync
             order = torch.argsort((args.beta0 - 1.0).abs(), stable=True).to(torch.int32)
         ci, co = args.structs(x, order)
-        check(lib().bsgp_solve_batch(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co), _stream_ptr()))
+        args.solve(plan, "", ci, co, _stream_ptr())
         res = args.result(x)
         res._keepalive = (gn, args.bkg, args.flux, args.beta0, args.x0, args.obj, args.order)
     return res
 
 
-def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, kw):
+def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image, kw):
     """Page-locked CPU tensors -> page-locked CPU tensors; one call of bsgp_solve_batch_pinned (returns when the results
     are in host memory).  `device` selects the GPU.  Image-shaped arguments (bkg stack, x0, obj) must be pinned too."""
     import torch
@@ -481,15 +565,15 @@ def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, devi
 
     with torch.cuda.device(plan.device):
         args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
-                     image=pinned, vector=_host_vector, alloc=hbuf)
+                     image=pinned, vector=_host_vector, alloc=hbuf, per_image=per_image)
         if x_out is None:
             x = torch.empty(tuple(gn.shape), dtype=gn.dtype, pin_memory=True)
         else:
             x = x_out
             if not (_is_tensor(x) and not x.is_cuda and x.is_pinned() and x.dtype == gn.dtype and x.shape == gn.shape and x.is_contiguous()):
                 raise ValueError("x_out must be a contiguous pinned CPU tensor of the shape and dtype of gn")
-        ci, co = args.structs(x, _queue_order(divergence, args.beta0))
-        check(lib().bsgp_solve_batch_pinned(plan.handle, C.byref(args.params), args.B, C.byref(ci), C.byref(co), _stream_ptr()))
+        ci, co = args.structs(x, _queue_order(divergence, args.beta0, args.is_beta))
+        args.solve(plan, "_pinned", ci, co, _stream_ptr())
     res = args.result(x)
     for i in np.nonzero(res.status == _capi.ST_INPUT_TIMEOUT)[0]:      # skipped images: defined (zero) pixels, status says why
         x[int(i)].zero_()

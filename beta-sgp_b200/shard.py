@@ -22,11 +22,16 @@ import numpy as np
 
 
 def expected_cost_rank(n_items, betaParam=None, divergence="beta"):
-    """Permutation of 0..n-1, most expensive expected solve first (stable)."""
-    if divergence != "beta" or betaParam is None:
-        return np.arange(n_items)
-    b = np.broadcast_to(np.asarray(betaParam, dtype=np.float64).reshape(-1), (n_items,))
-    return np.argsort(np.abs(b - 1.0), kind="stable")
+    """Permutation of 0..n-1, most expensive expected solve first (stable).  divergence may be one per image (a mixed
+    batch): its beta-SGP images are ranked by |beta - 1|, its KL images follow, as engine._queue_order hands them out."""
+    if isinstance(divergence, str):
+        if divergence != "beta" or betaParam is None:
+            return np.arange(n_items)
+        is_beta = np.ones(n_items, bool)
+    else:
+        is_beta = np.asarray([d == "beta" for d in divergence], bool)
+    b = np.broadcast_to(np.asarray(1.0 if betaParam is None else betaParam, dtype=np.float64).reshape(-1), (n_items,))
+    return np.argsort(np.where(is_beta, np.abs(b - 1.0), np.inf), kind="stable")
 
 
 def shard_indices(n_items, rank, world_size, cost_rank=None):
@@ -127,7 +132,7 @@ _FIELDS = ("x", "iters", "status", "discr", "times", "beta_final", "proj_evals",
 
 
 def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=None, divergence="beta", group=None, device=None,
-                        width="auto", timing=None, cost_rank=None, **kw):
+                        width="auto", timing=None, cost_rank=None, per_image=None, **kw):
     """Every rank passes the FULL batch and gets the full result back: rank r restores the images
     shard_indices(B, r, W, expected_cost_rank(...)) on its own GPU (engine.solve_batch, one persistent kernel launch) and
     the per-image results are all-gathered.  No data-path collective: the images are independent problems.
@@ -135,6 +140,7 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
     numpy inputs -> dict of numpy arrays; CUDA tensors -> dict of CUDA tensors (inputs are sliced, solved and gathered on
     the device, asynchronously on the current stream; NCCL process group required when world_size > 1).
     psf: [ny,nx] shared or [B,ny,nx]; bkg: scalar, [B] or [B,ny,nx]; flux / betaParam: scalar or [B]; x0 / obj: [B,ny,nx].
+    per_image: B keyword dicts of a mixed batch (engine.solve_batch); each rank receives the rows of its images.
     width: "auto" picks the CTA configuration from the local batch size (engine.auto_config), or (cluster_size, threads).
     cost_rank: optional precomputed expected_cost_rank(...) (a host array); give it when betaParam is a device tensor, so
     that the dealing does not have to copy betaParam back to the host (a synchronisation) on every call.
@@ -151,15 +157,22 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
         device = (gn.device.index or 0) if on_dev else int(__import__("os").environ.get("LOCAL_RANK", rank))
     B = int(gn.shape[0])
     ny, nx = int(gn.shape[-2]), int(gn.shape[-1])
+    if per_image is not None:
+        engine._check_per_image(per_image, B)
+        betaParam = engine._row_betas(betaParam, per_image, B)
+        flux, per_image = engine._row_flux(flux, per_image, B)
     if cost_rank is None:
         b_host = betaParam.detach().cpu().numpy() if engine._is_tensor(betaParam) else betaParam
-        cost_rank = expected_cost_rank(B, b_host, divergence)
+        kinds = divergence if per_image is None else [row.get("divergence", divergence) for row in per_image]
+        cost_rank = expected_cost_rank(B, b_host, kinds)
     cost_rank = np.ascontiguousarray(cost_rank)
     idx = shard_indices(B, rank, world, cost_rank)
     n_local = len(idx)
     use_cuda = on_dev or (is_dist and dist.get_backend(group) == "nccl")
     dev = torch.device("cuda", device) if use_cuda else torch.device("cpu")
     maxit = int(kw.get("MAXIT", 500))
+    if per_image is not None:
+        maxit = max(int(row.get("MAXIT", maxit)) for row in per_image)     # the trace stride of the whole batch
 
     if on_dev:
         skey = ("sel", B, rank, world, str(gn.device), cost_rank.tobytes())
@@ -201,6 +214,8 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
         args = (take(gn, 2), take(psf, 2), bk)
         kwargs = dict(divergence=divergence, flux=take(flux, 0), betaParam=take(betaParam, 0), x0=take(x0, 2), obj=take(obj, 2),
                       device=device, plan=plan, dtype=dtype, **kw)
+        if per_image is not None:
+            kwargs["per_image"] = [per_image[int(i)] for i in idx]
         if ev:
             if plan is not None:
                 plan.set_psf(args[1])                      # PSF spectra outside the bracket: it times the solve kernel alone
@@ -212,6 +227,10 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
             timing["solve"] = ev
             timing["plan"] = (plan or engine.get_plan(ny, nx, dtype, device)).info()
         local = {k: (getattr(r, k) if on_dev else torch.as_tensor(np.ascontiguousarray(getattr(r, k))).to(dev)) for k in _FIELDS}
+        for k in ("discr", "times"):                    # a mixed batch: this shard's largest MAXIT may be below the batch's
+            t = local[k]
+            if t.shape[1] < maxit + 1:
+                local[k] = torch.cat([t, torch.zeros((t.shape[0], maxit + 1 - t.shape[1]), dtype=t.dtype, device=t.device)], dim=1)
     else:
         # an empty shard (B < world size): nothing to solve, zero rows for the gather (the collective must still be entered)
         xdt = gn.dtype if on_dev else (torch.float32 if str(gn.dtype).endswith("float32") else torch.float64)

@@ -106,6 +106,9 @@ typedef struct bsgp_outputs {
     void* x;               /* [batch][ny][nx] restored images (un-scaled, like the reference's return value) */
     int* iters;            /* [batch] iteration count as returned by the reference */
     int* status;           /* [batch] BSGP_ST_* */
+    /* Trace arrays: one row of `stride` entries per image, stride = maxit + 1 (err: maxit + 2).  A mixed batch
+     * (bsgp_solve_batch_rows) uses the largest maxit of its rows for every image; entries past an image's own iters
+     * (its own maxit + 1 for err) are left as the caller allocated them. */
     double* discr;         /* [batch][maxit+1]; entries [0, iters] valid */
     double* times;         /* [batch][maxit+1] seconds since the image's solve began (device %globaltimer) */
     double* stop_value;    /* [batch][maxit+1] quantity compared with tol (criteria 2-4); may be NULL */
@@ -167,6 +170,21 @@ int bsgp_solve_batch_host(bsgp_plan* plan, const bsgp_params* params, int batch,
  * (application_sgp_star_stamps.py:56-105, application_sgp_subdivisions.py:83-107). */
 int bsgp_solve_batch_pinned(bsgp_plan* plan, const bsgp_params* params, int batch, const bsgp_inputs* in_host,
                             const bsgp_outputs* out_host, void* stream);
+
+/* Mixed batches: the same three calls with one bsgp_params per image, rows[0 .. batch-1] in host memory (read before the
+ * call returns), so that images with different keywords (KL and beta-SGP, stop rule, maxit, projection, saturation, ...)
+ * share one persistent launch.  Image i is exactly a solve of that image alone with rows[i].  The operator fields
+ * (region, div_a, div_at, adjoint_second_psf) describe the plan's operator and must be equal in every row; a row with
+ * has_flux, errflag, init_recon = 1 or the beta-divergence needs inputs.flux, inputs.obj (and outputs.err), inputs.x0 or
+ * inputs.beta0, as with the shared keywords.  Any violation is BSGP_E_ARG, naming the row, before anything is launched.
+ * The trace outputs have the stride of the largest maxit of the rows (see bsgp_outputs).  The device entry point copies
+ * the rows to the plan's device memory on `stream`, behind the plan's previous launch. */
+int bsgp_solve_batch_rows(bsgp_plan* plan, const bsgp_params* rows, int batch, const bsgp_inputs* in_dev,
+                          const bsgp_outputs* out_dev, void* stream);
+int bsgp_solve_batch_rows_host(bsgp_plan* plan, const bsgp_params* rows, int batch, const bsgp_inputs* in_host,
+                               const bsgp_outputs* out_host);
+int bsgp_solve_batch_rows_pinned(bsgp_plan* plan, const bsgp_params* rows, int batch, const bsgp_inputs* in_host,
+                                 const bsgp_outputs* out_host, void* stream);
 
 /* y = real(ifftn(TF * fftn(x))) (adjoint = 0) or with conj(TF) (adjoint = 1) for `batch` images: the
  * reference's A / A^T closures (sgp.py:111-120). PSF index = image index if n_psf > 1. */
