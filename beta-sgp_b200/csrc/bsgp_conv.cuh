@@ -29,6 +29,8 @@
 // Producers / consumers follow the same protocol: `fetch(i)` only loads (i = even slab pixel index,
 // returns a small struct of V2 values), `eval` / `apply` compute, accumulate and store.
 #pragma once
+#include <type_traits>
+
 #include "bsgp_fft.cuh"
 
 namespace bsgp {
@@ -106,9 +108,242 @@ template <class Ctx> BSGP_DEV void fill_pos_table(Ctx& ctx, const FftPlan& pl, u
     for (int k = ctx.tid; k < pl.n; k += ctx.nt) tab[k] = (unsigned short)fpad(pos_of_freq(pl, k), pl.pad_shift);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Split transforms (frame mode, an axis of N = 2M points whose single transform does not fit the workspace: fp64 axes of
+// 16384 on a B200).  The geometry marks a split axis by an FFT plan of M = N / 2 points (px.n != nx, py.n != ny); the
+// execution context compiles the split path in through Ctx::kSplit (SplitCtx, only the kernels of such plans), so that the
+// kernels of every other plan carry none of it.
+//   rows    : one real row x per transform, packed z[j] = x[2j] + i x[2j+1] (M points); the untangle
+//             2X[k] = (Z[k] + conj Z[M-k]) - i W_N^k (Z[k] - conj Z[M-k]), k = 0 .. M, keeps the half-spectrum layout of
+//             the row-pair path (2X stored, column 0 = (2X[0], 2X[N/2])).  The inverse feeds
+//             Q[k] = (Y[k] + Y[k+M]) + i conj(W_N^k) (Y[k] - Y[k+M]), Y[k+M] = conj Y[M-k], whose unnormalised inverse is
+//             y[2j] + i y[2j+1] of the unnormalised N-point inverse.
+//   columns : one radix-2 step outside shared memory: u[j] = a[j] + a[j+M] (even frequencies), v[j] = (a[j] - a[j+M]) W_N^j
+//             (odd frequencies), each transformed with the M-point machinery and multiplied by its half of the PSF spectrum
+//             (tf column = [even frequencies][odd frequencies], each in M-point position order); out[j] = U[j] + W_N^-j V[j],
+//             out[j+M] = U[j] - W_N^-j V[j].  Only one half fits the workspace: v waits in the exchange buffer rows [M, N)
+//             while u is processed, and the inverse-transformed u waits in rows [0, M) while v is processed (2 N w bytes
+//             of extra exchange-buffer traffic per convolution, DESIGN.md section 4).
+// ---------------------------------------------------------------------------------------------
+template <class C, class = void> struct is_split : std::false_type {};
+template <class C> struct is_split<C, std::void_t<decltype(C::kSplit)>> : std::integral_constant<bool, C::kSplit> {};
+template <class Ctx> struct SplitCtx : Ctx { static constexpr bool kSplit = true; };
+
+// twiddle W_M^k of the M-point plan's table: two-level in shared memory, full in shared memory, or full in global memory
+template <typename T> BSGP_DEV cplx<T> split_tw_m(const cplx<T>* tw, unsigned tw_off, int tw_split, int k) {
+    if (tw_split) return twiddle_at<T, true>(smem_at<cplx<T>>(tw_off), k);
+    return tw_off != kNoSmem ? smem_at<cplx<T>>(tw_off)[k] : tw[k];
+}
+// W_N^1, N = 2M
+template <typename T> BSGP_DEV cplx<T> split_w1(int M) {
+    double s, c;
+#ifdef BSGP_HOST_EMUL
+    const long double a = 3.141592653589793238462643383279502884L / (long double)M;
+    s = (double)sinl(a); c = (double)cosl(a);
+#else
+    sincospi(1.0 / (double)M, &s, &c);
+#endif
+    return cmake<T>((T)c, (T)-s);
+}
+// W_N^k = W_M^(k >> 1) (times W_N^1 for odd k), k < N
+template <typename T> BSGP_DEV cplx<T> split_tw_n(const cplx<T>* tw, unsigned tw_off, int tw_split, cplx<T> w1, int k) {
+    const cplx<T> w = split_tw_m(tw, tw_off, tw_split, k >> 1);
+    return (k & 1) ? cmul(w, w1) : w;
+}
+
+template <bool INV, class Ctx, typename T>
+BSGP_DEV void split_fft(Ctx& ctx, unsigned ws_off, int nfft, int fstride, const FftPlan& pl, const cplx<T>* tw, unsigned tw_off, int tw_split) {
+    if (tw_split) fft_batch_split<INV, Ctx, T>(ctx, ws_off, nfft, fstride, pl, tw_off);
+    else fft_batch<INV, false>(ctx, ws_off, nfft, fstride, pl, tw, tw_off);
+}
+
+// rows_forward of a split row axis: row_tile_pairs rows (one transform each) per workspace tile
+template <class Ctx, typename T, class Fetch, class Eval>
+BSGP_DEV void split_rows_forward(Ctx& ctx, const ConvGeom& gg, unsigned ws_off, const cplx<T>* twx, unsigned twx_off, int tw_split, unsigned ppx_off, cplx<T>* spec, Fetch& fetch, Eval& eval) {
+    cplx<T>* ws = smem_at<cplx<T>>(ws_off);
+    const unsigned short* ppx = smem_at<unsigned short>(ppx_off);
+    const int M = gg.px.n, lgM = gg.px.log2n, ps = gg.px.pad_shift, lg_nx = gg.lg_nx, rs = gg.rowstride, R = gg.row_tile_pairs;
+    const int lg_ny = gg.lg_ny, lg_cp = gg.lg_cp, hx = gg.hx;
+    const int r0 = ctx.rank * gg.rows_per_cta;
+    const cplx<T> w1 = split_w1<T>(M);
+    for (int row0 = 0; row0 < gg.rows_per_cta; row0 += R) {
+        for (int e = ctx.tid; e < (R << lgM); e += ctx.nt) {
+            const int r = e >> lgM, j = e & (M - 1);
+            const int i = ((row0 + r) << lg_nx) + 2 * j;
+            const auto in = fetch(i);
+            const V2<T> v = eval(i, in);
+            ws[r * rs + fpad(j, ps)] = cmake<T>(v.x, v.y);
+        }
+        ctx.sync();
+        split_fft<false>(ctx, ws_off, R, rs, gg.px, twx, twx_off, tw_split);
+        for (int e = ctx.tid; e < (R << lgM); e += ctx.nt) {
+            const int r = e >> lgM, k = e & (M - 1);
+            const cplx<T>* a = ws + r * rs;
+            const cplx<T> zk = a[ppx[k]];
+            cplx<T> X;
+            if (k == 0) {
+                X = cmake<T>((T)2 * (zk.re + zk.im), (T)2 * (zk.re - zk.im));
+            } else {
+                const cplx<T> zm = a[ppx[M - k]];
+                const cplx<T> S = cmake<T>(zk.re + zm.re, zk.im - zm.im), D = cmake<T>(zk.re - zm.re, zk.im + zm.im);
+                const cplx<T> wd = cmul(split_tw_n(twx, twx_off, tw_split, w1, k), D);
+                X = cmake<T>(S.re + wd.im, S.im - wd.re);                      // S - i W D
+            }
+            spec[spec_idx<true>(r0 + row0 + r, k, lg_ny, lg_cp, hx)] = X;
+        }
+        ctx.sync();
+    }
+}
+
+// rows_inverse of a split row axis; WRAP: the column fold of a wrapped plan
+template <bool WRAP, class Ctx, typename T, class Fetch, class Apply>
+BSGP_DEV void split_rows_inverse(Ctx& ctx, const ConvGeom& gg, unsigned ws_off, const cplx<T>* twx, unsigned twx_off, int tw_split, unsigned ppx_off, const cplx<T>* spec, Fetch& fetch, Apply& apply) {
+    cplx<T>* ws = smem_at<cplx<T>>(ws_off);
+    const unsigned short* ppx = smem_at<unsigned short>(ppx_off);
+    const int M = gg.px.n, lgM = gg.px.log2n, ps = gg.px.pad_shift, lg_nx = gg.lg_nx, rs = gg.rowstride, R = gg.row_tile_pairs;
+    const int lg_ny = gg.lg_ny, lg_cp = gg.lg_cp, hx = gg.hx, wn = WRAP ? gg.wrap_nx : 0;
+    const int r0 = ctx.rank * gg.rows_per_cta;
+    const cplx<T> w1 = split_w1<T>(M);
+    for (int row0 = 0; row0 < gg.rows_per_cta; row0 += R) {
+        for (int e = ctx.tid; e < (R << lgM); e += ctx.nt) {
+            const int r = e >> lgM, k = e & (M - 1);
+            const int row = r0 + row0 + r;
+            const cplx<T> yk = spec[spec_idx<true>(row, k, lg_ny, lg_cp, hx)];
+            cplx<T> q;
+            if (k == 0) {
+                q = cmake<T>(yk.re + yk.im, yk.re - yk.im);                     // Y[0] = re, Y[M] = im, both real
+            } else {
+                const cplx<T> ym = spec[spec_idx<true>(row, M - k, lg_ny, lg_cp, hx)];
+                const cplx<T> S = cmake<T>(yk.re + ym.re, yk.im - ym.im), D = cmake<T>(yk.re - ym.re, yk.im + ym.im);
+                const cplx<T> wd = cmulc(D, split_tw_n(twx, twx_off, tw_split, w1, k));
+                q = cmake<T>(S.re - wd.im, S.im + wd.re);                      // S + i conj(W) D
+            }
+            ws[r * rs + ppx[k]] = q;
+        }
+        ctx.sync();
+        split_fft<true>(ctx, ws_off, R, rs, gg.px, twx, twx_off, tw_split);
+        for (int e = ctx.tid; e < (R << lgM); e += ctx.nt) {
+            const int r = e >> lgM, j = e & (M - 1);
+            const cplx<T>* a = ws + r * rs;
+            const cplx<T> z = a[fpad(j, ps)];
+            T v0 = z.re, v1 = z.im;
+            if (WRAP && 2 * j < wn) {
+                auto px = [&](int c) { const cplx<T> t = a[fpad(c >> 1, ps)]; return (c & 1) ? t.im : t.re; };
+                v0 += px(2 * j + wn);
+                if (2 * j + 1 < wn) v1 += px(2 * j + 1 + wn);
+            }
+            const int i = ((row0 + r) << lg_nx) + 2 * j;
+            const auto in = fetch(i);
+            apply(i, in, mk2<T>(v0, v1));
+        }
+        ctx.sync();
+    }
+}
+
+// the column pass of a split column axis (see above); GEN: wrapped plans fold the rows
+template <bool GEN, class Ctx, typename T>
+BSGP_NOINLINE void split_cols(Ctx ctx, const ConvGeom* gp, unsigned ws_off, const cplx<T>* twy, unsigned twy_off, int tw_split, cplx<T>* spec, cplx<T>* tf, int mode) {
+    cplx<T>* ws = smem_at<cplx<T>>(ws_off);
+    const int ny = gp->ny, nx = gp->nx, hx = gp->hx, lg_ny = gp->lg_ny, lg_cp = gp->lg_cp;
+    const int M = gp->py.n, lgM = gp->py.log2n, ps = gp->py.pad_shift, cs = gp->colstride;
+    const int ct = gp->col_tile, lct = gp->lg_col_tile, c0 = ctx.rank * gp->cols_per_cta;
+    const FftPlan& py = gp->py;
+    const cplx<T> w1 = split_w1<T>(M);
+    auto sidx = [&](int row, int col) { return spec_idx<true>(row, col, lg_ny, lg_cp, hx); };
+    const int total = ct << lgM;
+    for (int cc0 = c0; cc0 < c0 + gp->cols_per_cta; cc0 += ct) {
+        for (int e = ctx.tid; e < total; e += ctx.nt) {
+            const int j = e >> lct, cl = e & (ct - 1);
+            const cplx<T> lo = spec[sidx(j, cc0 + cl)], hi = spec[sidx(j + M, cc0 + cl)];
+            ws[cl * cs + fpad(j, ps)] = cadd(lo, hi);
+            spec[sidx(j + M, cc0 + cl)] = cmul(csub(lo, hi), split_tw_n(twy, twy_off, tw_split, w1, j));   // v waits here
+        }
+        ctx.sync();
+        for (int h = 0; h < 2; ++h) {
+            if (h == 1) {
+                for (int e = ctx.tid; e < total; e += ctx.nt) {
+                    const int j = e >> lct, cl = e & (ct - 1);
+                    ws[cl * cs + fpad(j, ps)] = spec[sidx(j + M, cc0 + cl)];
+                }
+                ctx.sync();
+            }
+            split_fft<false>(ctx, ws_off, ct, cs, py, twy, twy_off, tw_split);
+            const size_t hoff = (size_t)h * M;
+            // column 0 packs kx = 0 and kx = nx/2; frequency ky = 2 k + h pairs with N - ky = 2 k' + h, k' = (M - k - h) mod M
+            const int kend = h ? (M >> 1) - 1 : (M >> 1);
+            if (mode == CONV_MAKE_TF) {
+                const T sc = (T)0.25 / ((T)nx * (T)ny), sp = (T)0.0625 / ((T)nx * (T)ny);
+                for (int e = ctx.tid; e < total; e += ctx.nt) {
+                    const int cl = e >> lgM, p = e & (M - 1);
+                    if (cc0 + cl == 0) continue;
+                    tf[(size_t)(cc0 + cl) * ny + hoff + p] = cscale(ws[cl * cs + fpad(p, ps)], sc);
+                }
+                if (cc0 == 0) {
+                    for (int k = ctx.tid; k <= kend; k += ctx.nt) {
+                        const int pa = pos_of_freq(py, k), pb = pos_of_freq(py, (M - k - h) & (M - 1));
+                        const cplx<T> za = ws[fpad(pa, ps)], zb = ws[fpad(pb, ps)];
+                        const cplx<T> c0v = cmake<T>(za.re + zb.re, za.im - zb.im), chv = cmake<T>(za.im + zb.im, zb.re - za.re);
+                        tf[hoff + pa] = cscale(c0v, sp);
+                        tf[(size_t)hx * ny + hoff + pa] = cscale(chv, sp);
+                        tf[hoff + pb] = cscale(cconj(c0v), sp);
+                        tf[(size_t)hx * ny + hoff + pb] = cscale(cconj(chv), sp);
+                    }
+                }
+                ctx.sync();
+                continue;
+            }
+            for (int e = ctx.tid; e < total; e += ctx.nt) {
+                const int cl = e >> lgM, p = e & (M - 1);
+                if (cc0 + cl == 0) continue;
+                cplx<T>* z = ws + cl * cs + fpad(p, ps);
+                const cplx<T> t = tf[(size_t)(cc0 + cl) * ny + hoff + p];
+                *z = (mode == CONV_TF) ? cmul(*z, t) : cmulc(*z, t);
+            }
+            if (cc0 == 0) {
+                for (int k = ctx.tid; k <= kend; k += ctx.nt) {
+                    const int pa = pos_of_freq(py, k), pb = pos_of_freq(py, (M - k - h) & (M - 1));
+                    cplx<T> t0a = tf[hoff + pa], tha = tf[(size_t)hx * ny + hoff + pa], t0b = tf[hoff + pb], thb = tf[(size_t)hx * ny + hoff + pb];
+                    const cplx<T> za = ws[fpad(pa, ps)], zb = ws[fpad(pb, ps)];
+                    const cplx<T> c0a = cmake<T>(za.re + zb.re, za.im - zb.im), cha = cmake<T>(za.im + zb.im, zb.re - za.re);
+                    if (mode == CONV_CTF) { t0a = cconj(t0a); tha = cconj(tha); t0b = cconj(t0b); thb = cconj(thb); }
+                    const cplx<T> ya0 = cmul(t0a, c0a), yah = cmul(tha, cha);
+                    const cplx<T> yb0 = cmul(t0b, cconj(c0a)), ybh = cmul(thb, cconj(cha));
+                    ws[fpad(pa, ps)] = cmake<T>(ya0.re - yah.im, ya0.im + yah.re);
+                    if (pb != pa) ws[fpad(pb, ps)] = cmake<T>(yb0.re - ybh.im, yb0.im + ybh.re);
+                }
+            }
+            ctx.sync();
+            split_fft<true>(ctx, ws_off, ct, cs, py, twy, twy_off, tw_split);
+            for (int e = ctx.tid; e < total; e += ctx.nt) {
+                const int j = e >> lct, cl = e & (ct - 1);
+                const cplx<T> z = ws[cl * cs + fpad(j, ps)];
+                if (h == 0) {
+                    spec[sidx(j, cc0 + cl)] = z;                                  // U waits here
+                } else {
+                    const cplx<T> u = spec[sidx(j, cc0 + cl)], v = cmulc(z, split_tw_n(twy, twy_off, tw_split, w1, j));
+                    spec[sidx(j, cc0 + cl)] = cadd(u, v);
+                    spec[sidx(j + M, cc0 + cl)] = csub(u, v);
+                }
+            }
+            ctx.sync();
+        }
+        if (GEN && mode != CONV_MAKE_TF && gp->wrap_ny > 0) {                    // wrapped plan: z[i] += z[i + n]
+            const int wn = gp->wrap_ny;
+            for (int e = ctx.tid; e < ct * wn; e += ctx.nt) {
+                const int cl = e / wn, row = e - cl * wn;
+                spec[sidx(row, cc0 + cl)] = cadd(spec[sidx(row, cc0 + cl)], spec[sidx(row + wn, cc0 + cl)]);
+            }
+            ctx.sync();
+        }
+    }
+}
+
 // Producer: In fetch(i); V2 eval(i, In) for the slab pixel pair (i, i + 1), i = local_row * nx + col.
 template <int U_, bool GEN = false, class Ctx, typename T, class Fetch, class Eval>
 BSGP_DEV void conv_rows_forward(Ctx& ctx, const ConvGeom& gg, unsigned ws_off, const cplx<T>* twx, unsigned twx_off, int tw_split, unsigned ppx_off, cplx<T>* spec, Fetch& fetch, Eval& eval) {
+    if constexpr (is_split<Ctx>::value) {
+        if (gg.px.n != gg.nx) { split_rows_forward(ctx, gg, ws_off, twx, twx_off, tw_split, ppx_off, spec, fetch, eval); return; }
+    }
     constexpr int U = Ctx::kSmall ? 1 : U_;                  // small images: a thread has one or two steps per pass, batches would only be code
     cplx<T>* ws = smem_at<cplx<T>>(ws_off);
     const unsigned short* ppx = smem_at<unsigned short>(ppx_off);
@@ -187,13 +422,17 @@ BSGP_DEV void conv_rows_forward(Ctx& ctx, const ConvGeom& gg, unsigned ws_off, c
 // producer / consumer, so all convolutions of the solver share one copy of the code.
 template <bool GEN, class Ctx, typename T>
 BSGP_NOINLINE void conv_cols(Ctx ctx, const ConvGeom* gp, unsigned ws_off, const cplx<T>* twy, unsigned twy_off, int tw_split, cplx<T>* spec, cplx<T>* tf, int mode) {
+    if constexpr (is_split<Ctx>::value) {
+        if (gp->py.n != gp->ny) { split_cols<GEN>(ctx, gp, ws_off, twy, twy_off, tw_split, spec, tf, mode); return; }
+    }
     cplx<T>* ws = smem_at<cplx<T>>(ws_off);
     constexpr int U = Ctx::kSmall ? 1 : 8;
     struct { int ny, nx, hx, lg_ny, lg_col_tile, col_tile, colstride, cols_per_cta, lg_cp; } g;      // register copies
     g.ny = gp->ny; g.nx = gp->nx; g.hx = gp->hx; g.lg_ny = gp->lg_ny; g.lg_col_tile = gp->lg_col_tile; g.col_tile = gp->col_tile; g.lg_cp = gp->lg_cp;
     g.colstride = gp->colstride; g.cols_per_cta = gp->cols_per_cta;
     const FftPlan& py = gp->py;
-    const int ney = GEN ? fft_len(gp->py) : g.ny, nex = GEN ? fft_len(gp->px) : g.nx;     // transform lengths (== ny, nx unless an axis is a dense DFT)
+    // transform lengths (== ny, nx unless an axis is a dense DFT; a split axis has no dense DFT and px.n == nx / 2)
+    const int ney = GEN ? fft_len(gp->py) : g.ny, nex = (GEN && !is_split<Ctx>::value) ? fft_len(gp->px) : g.nx;
     const int c0 = ctx.rank * g.cols_per_cta;
     const int ps = gp->py.pad_shift;
     const int ntiles = g.cols_per_cta / g.col_tile;
@@ -309,6 +548,9 @@ BSGP_NOINLINE void conv_cols(Ctx ctx, const ConvGeom* gp, unsigned ws_off, const
 // for a dense row transform (the GEN features of row_geom).
 template <int U_, bool WRAP = false, class Ctx, typename T, class Fetch, class Apply>
 BSGP_DEV void conv_rows_inverse(Ctx& ctx, const ConvGeom& gg, unsigned ws_off, const cplx<T>* twx, unsigned twx_off, int tw_split, unsigned ppx_off, const cplx<T>* spec, Fetch& fetch, Apply& apply) {
+    if constexpr (is_split<Ctx>::value) {
+        if (gg.px.n != gg.nx) { split_rows_inverse<WRAP>(ctx, gg, ws_off, twx, twx_off, tw_split, ppx_off, spec, fetch, apply); return; }
+    }
     cplx<T>* ws = smem_at<cplx<T>>(ws_off);
     const unsigned short* ppx = smem_at<unsigned short>(ppx_off);
     constexpr int U = Ctx::kSmall ? 1 : U_;

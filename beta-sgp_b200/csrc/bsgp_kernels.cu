@@ -115,6 +115,15 @@ __global__ void __launch_bounds__(512, 1) bsgp_conv_frame_kernel(const ConvArgs<
     conv_items(ctx, a, off_geom, off_ppx, off_ws, 0, [img = 0]() mutable { return img++; });
 }
 
+// the same for plans with a split axis (bsgp_conv.cuh, split transforms)
+template <typename T>
+__global__ void __launch_bounds__(512, 1) bsgp_conv_frame_split_kernel(const ConvArgs<T> a, const unsigned off_geom, const unsigned off_ppx,
+                                                                       const unsigned off_ws, double* gpart) {
+    SplitCtx<GridCtx> ctx;
+    static_cast<GridCtx&>(ctx) = make_grid_ctx(reinterpret_cast<SharedCtl*>(dyn_smem()), gpart);
+    conv_items(ctx, a, off_geom, off_ppx, off_ws, 0, [img = 0]() mutable { return img++; });
+}
+
 // projectDF (flux_conserve_proj.py:7-144): one CTA per problem, x = clamp((c + lambda) / dia).
 __global__ void __launch_bounds__(512, 1) bsgp_project_kernel(const double* __restrict__ b, const double* __restrict__ c,
                                                               const double* __restrict__ dia, int n, int batch, double cap, int has_cap,
@@ -215,7 +224,7 @@ __global__ void bsgp_assemble_tiles_kernel(const T* __restrict__ tiles, const in
 }
 
 // ------------------------------------------------------------------------------------------------
-// Embedded plans: image sides that are not a power of two in [16, 8192] (the reference's numpy closure takes any
+// Embedded plans: image sides that are not a power of two, up to 8192 (the reference's numpy closure takes any
 // size, sgp.py:108-120; its star-stamp application runs it on 31 x 31 cut-outs, application_sgp_star_stamps.py:24,58).
 // Per axis (bsgp_wrap.h): a side n <= 32 keeps a grid of 16 or 32 slots and is transformed by a dense DFT of length n
 // over the first n slots (the circular operator itself, no fold); any other side is WRAPPED:
@@ -379,6 +388,17 @@ struct bsgp_plan : LaunchPlan {
 
 template <typename T> static const void* conv_kernel_ptr() { return (const void*)bsgp_conv_kernel<T>; }
 
+// device allocation of the plan's large buffers: running out of memory is BSGP_E_NOMEM with the size asked for (a 16384^2
+// plan holds several GiB, DESIGN.md section 5)
+static int dev_alloc(void** buf, size_t bytes, const char* what) {
+    const cudaError_t e = cudaMalloc(buf, bytes);
+    if (e == cudaSuccess) return BSGP_OK;
+    cudaGetLastError();
+    *buf = nullptr;
+    if (e == cudaErrorMemoryAllocation) return fail(BSGP_E_NOMEM, "out of device memory: %zu B for %s", bytes, what);
+    return fail(BSGP_E_CUDA, "cudaMalloc of %zu B for %s failed: %s", bytes, what, cudaGetErrorString(e));
+}
+
 static void plan_free_pipeline(bsgp_plan* p) {
     cudaFree(p->stage); cudaFree(p->ready); cudaFreeHost(p->ones_host);
     cudaFree(p->emb_psf); cudaFree(p->emb_img); cudaFree(p->rows);
@@ -397,14 +417,20 @@ static void plan_free_buffers(bsgp_plan* p) {
     p->tf_capacity = 0; p->n_psf = 0; p->tf_adj = nullptr; p->tf_adj_capacity = 0; p->n_psf_adj = 0;
 }
 
-template <typename T> static const void* conv_frame_kernel_ptr() { return (const void*)bsgp_conv_frame_kernel<T>; }
+// split kernels for fp64 only: an fp32 transform of every supported length fits the frame workspace
+template <typename T> static const void* conv_frame_kernel_ptr(bool split) {
+    if constexpr (sizeof(T) == 8) {
+        if (split) return (const void*)bsgp_conv_frame_split_kernel<T>;
+    }
+    return (const void*)bsgp_conv_frame_kernel<T>;
+}
 
 template <typename T> static int alloc_tables(bsgp_plan* p) {
     std::vector<cplx<T>> tw;
-    make_twiddles<T>(p->nx, tw, p->g.px.dft_n);
+    make_twiddles<T>(p->g.px.n, tw, p->g.px.dft_n);                   // nx, or nx / 2 on a split axis
     CU(cudaMalloc(&p->twx, tw.size() * sizeof(cplx<T>)));
     CU(cudaMemcpy(p->twx, tw.data(), tw.size() * sizeof(cplx<T>), cudaMemcpyHostToDevice));
-    make_twiddles<T>(p->ny, tw, p->g.py.dft_n);
+    make_twiddles<T>(p->g.py.n, tw, p->g.py.dft_n);
     CU(cudaMalloc(&p->twy, tw.size() * sizeof(cplx<T>)));
     CU(cudaMemcpy(p->twy, tw.data(), tw.size() * sizeof(cplx<T>), cudaMemcpyHostToDevice));
     return BSGP_OK;
@@ -427,7 +453,8 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
         if (!coop) return fail(BSGP_E_CUDA, "device does not support cooperative launches (frame mode)");
         LaunchCfg lc{G, 512, 1, p->smem_bytes, nullptr, 1};
         int per_sm = 0;
-        cudaError_t e = query_frame_ctas<T, false>(lc, &per_sm);
+        if (sizeof(T) != 8 && has_split(p->g)) return fail(BSGP_E_SHAPE, "split transforms are built for fp64 only");
+        cudaError_t e = query_frame_ctas<T, false>(lc, &per_sm, has_split(p->g));
         if (e != cudaSuccess) return fail(BSGP_E_CUDA, "occupancy query failed: %s", cudaGetErrorString(e));
         if (per_sm < 1) return fail(BSGP_E_CUDA, "frame kernel does not fit: %zu B shared memory", p->smem_bytes);
         p->num_clusters = p->conv_clusters = 1;
@@ -449,8 +476,8 @@ template <typename T> static int plan_setup_t(bsgp_plan* p) {
     p->work_stride = NBUF * (size_t)p->ny * p->nx;
     p->spec_stride = (size_t)p->ny * p->g.hx;
     p->tf_stride = (size_t)(p->g.hx + 1) * p->ny;
-    CU(cudaMalloc(&p->work, (size_t)p->num_clusters * p->work_stride * sizeof(T)));
-    CU(cudaMalloc(&p->spec, (size_t)nscratch * p->spec_stride * sizeof(cplx<T>)));
+    { int rc = dev_alloc(&p->work, (size_t)p->num_clusters * p->work_stride * sizeof(T), "the per-image scratch arrays"); if (rc) return rc; }
+    { int rc = dev_alloc(&p->spec, (size_t)nscratch * p->spec_stride * sizeof(cplx<T>), "the exchange buffer"); if (rc) return rc; }
     CU(cudaMalloc((void**)&p->queue, sizeof(int)));
     if (p->frame) CU(cudaMalloc((void**)&p->gpart, (size_t)2 * G * kMaxK * sizeof(double)));
     p->workspace_bytes = (size_t)p->num_clusters * p->work_stride * sizeof(T) + (size_t)nscratch * p->spec_stride * sizeof(cplx<T>);
@@ -478,10 +505,11 @@ static int plan_leave(bsgp_plan* p, cudaStream_t st) {
     return BSGP_OK;
 }
 
-static int grow(void** buf, size_t* cap, size_t bytes) {
+static int grow(void** buf, size_t* cap, size_t bytes, const char* what) {
     if (bytes <= *cap) return BSGP_OK;
     cudaFree(*buf); *buf = nullptr; *cap = 0;           // cudaFree waits for the work that may still use the old buffer
-    CU(cudaMalloc(buf, bytes));
+    const int rc = dev_alloc(buf, bytes, what);
+    if (rc) return rc;
     *cap = bytes;
     return BSGP_OK;
 }
@@ -519,9 +547,10 @@ template <typename T> static int launch_conv(bsgp_plan* p, ConvArgs<T>& a, int c
         void* args[] = {&a, &og, &op, &ow, &gp};
         // the shared-memory limit is an attribute of the kernel, not of the plan: another frame plan of the same dtype may
         // have set it lower since this plan was set up, so it is set again before every launch (as launch_clustered does)
-        CU(cudaFuncSetAttribute(conv_frame_kernel_ptr<T>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
+        const void* fn = conv_frame_kernel_ptr<T>(has_split(p->g));
+        CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->conv_smem));
         count_launch();
-        cudaError_t e = cudaLaunchCooperativeKernel(conv_frame_kernel_ptr<T>(), dim3(p->g.G), dim3(512), args, p->conv_smem, st);
+        cudaError_t e = cudaLaunchCooperativeKernel(fn, dim3(p->g.G), dim3(512), args, p->conv_smem, st);
         if (e != cudaSuccess) return fail(BSGP_E_CUDA, "convolution kernel launch failed: %s", cudaGetErrorString(e));
         return BSGP_OK;
     }
@@ -541,7 +570,8 @@ template <typename T> static int set_psf_t(bsgp_plan* p, const void* psf_dev, in
     int& cap = adjoint_kernel ? p->tf_adj_capacity : p->tf_capacity;
     if (n_psf > cap) {
         cudaFree(tfbuf); tfbuf = nullptr; cap = 0;
-        CU(cudaMalloc(&tfbuf, (size_t)n_psf * p->tf_stride * sizeof(cplx<T>)));
+        const int rc = dev_alloc(&tfbuf, (size_t)n_psf * p->tf_stride * sizeof(cplx<T>), "the PSF spectra");
+        if (rc) return rc;
         cap = n_psf;
     }
     (adjoint_kernel ? p->n_psf_adj : p->n_psf) = n_psf;
@@ -562,7 +592,7 @@ template <typename T> static int apply_psf_t(bsgp_plan* p, const void* x, void* 
     if (!p->embedded) return launch_conv<T>(p, a, batch, st);
     // wrapped plan: embed, convolve on the grid with the spectrum of h (A) or of h~ (A^T), fold (in the kernel), crop
     const size_t gb = (size_t)batch * p->ny * p->nx * sizeof(T);
-    int rc = grow(&p->emb_img, &p->emb_img_cap, 2 * gb);
+    int rc = grow(&p->emb_img, &p->emb_img_cap, 2 * gb, "the images on the FFT grid");
     if (rc) return rc;
     T* xe = (T*)p->emb_img; T* ye = (T*)((char*)p->emb_img + gb);
     rc = embed_images<T>(p, x, xe, batch, st);
@@ -577,7 +607,7 @@ template <typename T> static int apply_psf_t(bsgp_plan* p, const void* x, void* 
 // bsgp_set_psf on a wrapped plan: both kernels (h for A, h~ for A^T) are built on the grid from the caller's PSFs
 template <typename T> static int set_psf_wrapped(bsgp_plan* p, const void* psf_dev, int n_psf, cudaStream_t st) {
     const size_t gb = (size_t)n_psf * p->ny * p->nx * sizeof(T);
-    int rc = grow(&p->emb_psf, &p->emb_psf_cap, gb);
+    int rc = grow(&p->emb_psf, &p->emb_psf_cap, gb, "the PSFs on the FFT grid");
     if (rc) return rc;
     int blocks = 0;
     rc = data_grid(p->device, (size_t)n_psf * p->ny * p->nx, &blocks);
@@ -606,7 +636,7 @@ static int solve_t(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_input
     if (!p->embedded) return solve_grid<T>(p, kw, batch, in, out, st, ready);
     const size_t gb = (size_t)batch * p->ny * p->nx * sizeof(T);
     const int narr = 2 + (in->bkg_is_image ? 1 : 0) + (in->x0 ? 1 : 0) + (in->obj ? 1 : 0);
-    int rc = grow(&p->emb_img, &p->emb_img_cap, (size_t)narr * gb);
+    int rc = grow(&p->emb_img, &p->emb_img_cap, (size_t)narr * gb, "the images on the FFT grid");
     if (rc) return rc;
     char* base = (char*)p->emb_img;
     int k = 0;
@@ -656,7 +686,9 @@ static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_in
         LaunchCfg fc{p->g.G, 512, 1, p->smem_bytes, st, 1};
         const bool mk = prm->region[1] > prm->region[0];
         count_launch();
-        cudaError_t fe = mk ? launch_frame<T, true>(fc, a, p->sp, p->tf_stride, p->gpart, rows) : launch_frame<T, false>(fc, a, p->sp, p->tf_stride, p->gpart, rows);
+        const bool split = has_split(p->g);
+        cudaError_t fe = mk ? launch_frame<T, true>(fc, a, p->sp, p->tf_stride, p->gpart, rows, split)
+                            : launch_frame<T, false>(fc, a, p->sp, p->tf_stride, p->gpart, rows, split);
         if (fe != cudaSuccess) return fail(BSGP_E_CUDA, "frame kernel launch failed: %s", cudaGetErrorString(fe));
         return BSGP_OK;
     }
@@ -683,7 +715,7 @@ static int set_psf_host(bsgp_plan* p, const void* psf_host, int n_psf, bool adjo
     CU(cudaSetDevice(p->device));
     const size_t bytes = (size_t)n_psf * p->img_ny * p->img_nx * p->elem;
     void* d = nullptr;
-    CU(cudaMalloc(&d, bytes));
+    if (int rc = dev_alloc(&d, bytes, "the staged PSFs")) return rc;
     cudaError_t e = cudaMemcpy(d, psf_host, bytes, cudaMemcpyHostToDevice);
     int rc = e != cudaSuccess ? fail(BSGP_E_CUDA, "H2D copy failed: %s", cudaGetErrorString(e))
                               : (adjoint ? bsgp_set_psf_adjoint : bsgp_set_psf)(p, d, n_psf, nullptr);
@@ -720,11 +752,9 @@ int bsgp_plan_create(int ny, int nx, int dtype, int device, bsgp_plan** plan) {
     *plan = nullptr;
     if (dtype != BSGP_F64 && dtype != BSGP_F32) return fail(BSGP_E_ARG, "dtype must be BSGP_F64 or BSGP_F32");
     if (ny < 1 || nx < 1) return fail(BSGP_E_SHAPE, "unsupported image shape %dx%d", ny, nx);
-    // FFT grid: a power-of-two side in [16, 8192] is used as it is; any other side n runs on a grid of side
-    // P = 2^k >= 2 n - 1 (linear convolution + fold, see "Wrapped plans" above)
+    // FFT grid: a power-of-two side in [16, 16384] is used as it is; any other side n runs on a grid of side
+    // P = 2^k >= 2 n - 1 (linear convolution + fold, see "Wrapped plans" above).  plan_launch refuses grids beyond kMaxSide.
     const int gy = wrap_grid_side(ny), gx = wrap_grid_side(nx);
-    if (gy > 8192 || gx > 8192)
-        return fail(BSGP_E_SHAPE, "unsupported image shape %dx%d: sides that are not a power of two are limited to 4096 (FFT grid of 8192)", ny, nx);
     int ndev = 0;
     CU(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(BSGP_E_CUDA, "device %d not available (%d CUDA devices)", device, ndev);
@@ -845,7 +875,7 @@ static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_
     Keywords dk = kw;
     if (kw.rows) {
         const size_t bytes = (size_t)batch * sizeof(bsgp_params);
-        if ((rc = grow((void**)&p->rows, &p->rows_cap, bytes))) return rc;
+        if ((rc = grow((void**)&p->rows, &p->rows_cap, bytes, "the per-image keywords"))) return rc;
         CU(cudaMemcpyAsync(p->rows, kw.rows, bytes, cudaMemcpyHostToDevice, st));
         dk.rows = p->rows;
     }
@@ -867,13 +897,13 @@ struct DevBuf {
     ~DevBuf() { cudaFree(d); }
     int up(const void* h, size_t bytes) {
         if (!h) return BSGP_OK;
-        CU(cudaMalloc(&d, bytes));
+        if (int rc = dev_alloc(&d, bytes, "host staging")) return rc;
         CU(cudaMemcpy(d, h, bytes, cudaMemcpyHostToDevice));
         return BSGP_OK;
     }
     int alloc(bool want, size_t bytes) {
         if (!want) return BSGP_OK;
-        CU(cudaMalloc(&d, bytes));
+        if (int rc = dev_alloc(&d, bytes, "host staging")) return rc;
         CU(cudaMemset(d, 0, bytes));
         return BSGP_OK;
     }
@@ -991,7 +1021,7 @@ static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params*
     // images in the caller's own shape: a plan whose grid differs from it (sides that are not a power of two) moves them
     // to and from the grid on the device (solve_t), which needs all of them resident first, like frame mode
     const bool resident_first = p->frame || p->embedded;
-    TRY(grow(&p->stage, &p->stage_cap, io.size));
+    TRY(grow(&p->stage, &p->stage_cap, io.size, "the staging area"));
     if (batch > p->ready_cap) {
         CU(cudaDeviceSynchronize());
         cudaFree(p->ready); cudaFreeHost(p->ones_host); p->ready = nullptr; p->ones_host = nullptr; p->ready_cap = 0;

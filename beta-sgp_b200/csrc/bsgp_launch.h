@@ -66,8 +66,9 @@ static inline cudaError_t query_clusters(const void* func, const LaunchCfg& lc, 
 template <typename T, bool MK> cudaError_t launch_solve(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride,
                                                   const RowArgs* rows);
 template <typename T, bool MK> cudaError_t query_solve_clusters(const LaunchCfg& lc, int num_sms, int* out);
+// split: the plan has an axis of split transforms (bsgp_conv.cuh), run by the frame kernels of SplitCtx
 template <typename T, bool MK> cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart,
-                                                  const RowArgs* rows);
-template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm);
+                                                  const RowArgs* rows, bool split);
+template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm, bool split);
 
 }  // namespace bsgp

@@ -89,10 +89,13 @@ template <typename T> inline void make_twiddles(int n, std::vector<cplx<T>>& tw,
 // Geometry for a cluster of G CTAs and a shared-memory FFT workspace of at most ws_limit bytes.
 // Returns false if the shape cannot be handled.
 // dft_ny / dft_nx: 0, or the length of the dense DFT that replaces the radix transform along that axis (bsgp_fft.cuh).
+// split: bit 0 / bit 1: the rows / columns run split transforms of nx / 2 / ny / 2 points (bsgp_conv.cuh; frame mode only),
+// marked in the geometry by px.n == nx / 2 / py.n == ny / 2.  A split row tile holds row_tile_pairs single rows.
 inline bool make_geom(int ny, int nx, int G, size_t elem_bytes /* sizeof(cplx<T>) */, size_t ws_limit, ConvGeom* g,
-                      size_t* ws_bytes, int dft_ny = 0, int dft_nx = 0) {
+                      size_t* ws_bytes, int dft_ny = 0, int dft_nx = 0, int split = 0) {
     if (!is_pow2(ny) || !is_pow2(nx) || ny < 16 || nx < 16) return false;
-    if (!make_fft_plan(nx, &g->px, dft_nx) || !make_fft_plan(ny, &g->py, dft_ny)) return false;
+    if (split && (dft_ny || dft_nx)) return false;
+    if (!make_fft_plan((split & 1) ? nx / 2 : nx, &g->px, dft_nx) || !make_fft_plan((split & 2) ? ny / 2 : ny, &g->py, dft_ny)) return false;
     if ((dft_ny || dft_nx) && G != 1) return false;          // dense transforms: small images, one CTA each
     g->ny = ny; g->nx = nx; g->hx = nx / 2;
     g->lg_nx = ilog2(nx); g->lg_ny = ilog2(ny); g->lg_hx = g->lg_nx - 1;
@@ -116,6 +119,14 @@ inline bool make_geom(int ny, int nx, int G, size_t elem_bytes /* sizeof(cplx<T>
     *ws_bytes = a > b ? a : b;
     return true;
 }
+
+// The axes whose single transform does not fit a workspace of ws_limit bytes (bit 0: rows, bit 1: columns), make_geom's split
+inline int split_axes(int ny, int nx, size_t elem_bytes, size_t ws_limit) {
+    FftPlan px, py;
+    if (!make_fft_plan(nx, &px) || !make_fft_plan(ny, &py)) return 0;
+    return ((size_t)px.plen * elem_bytes > ws_limit ? 1 : 0) | ((size_t)(py.plen | 1) * elem_bytes > ws_limit ? 2 : 0);
+}
+inline bool has_split(const ConvGeom& g) { return g.px.n != g.nx || g.py.n != g.ny; }
 
 // A plan's request: the FFT grid, the caller's image shape, the cluster size (0: automatic, -1: frame mode) and threads
 // per CTA (0: automatic) asked for, and the device's SM count, opt-in shared memory per block and shared memory per SM.
@@ -150,9 +161,31 @@ constexpr int kResidencyOrder[NBUF] = {B_D, B_T1, B_G, B_X, B_XTF, B_DTF, B_GN, 
 template <typename T> inline int plan_launch(const PlanRequest& q, LaunchPlan* out, char* err, size_t errlen) {
     LaunchPlan L;
     const size_t npix = (size_t)q.ny * q.nx;
-    // Frame mode (bsgp_device.cuh, GridCtx): images of a megapixel or more get the whole GPU each, one CTA per SM on the
-    // largest power of two of SMs that divides the image
-    L.frame = q.want_G == -1 || (q.want_G == 0 && npix >= ((size_t)1 << 20));
+    // short sides that are not a power of two: dense DFT of the image's own length on the first slots of the grid
+    // (bsgp_wrap.h); make_geom refuses them for more than one CTA per image, frame mode included
+    const int dny = q.ny != q.img_ny ? dense_len(q.img_ny) : 0, dnx = q.nx != q.img_nx ? dense_len(q.img_nx) : 0;
+    if (q.ny > kMaxSide || q.nx > kMaxSide) {
+        snprintf(err, errlen, "unsupported image shape %dx%d: power-of-two sides up to %d, other sides up to %d", q.img_ny, q.img_nx,
+                 kMaxSide, kMaxSide / 2);
+        return BSGP_E_SHAPE;
+    }
+    // A 16384-point axis: one transform takes (16384 + 2048) complex elements of workspace, 144 KB in fp32.  Only frame mode
+    // has a workspace that large with room for the 32 KB position table, and only frame mode runs split transforms (fp64:
+    // 288 KB, more than a CTA's shared memory); a dense axis runs one CTA per image.
+    const bool long_axis = q.ny > kMaxClusterSide || q.nx > kMaxClusterSide;
+    if (long_axis) {
+        const char* why = dny || dnx ? "a dense axis (a side of at most 32 that is not a power of two) runs one CTA per image"
+                        : q.want_G > 0 ? "it runs in frame mode only (cluster size -1 or 0)"
+                        : nullptr;
+        if (why) {
+            snprintf(err, errlen, "unsupported shape %dx%d (FFT grid %dx%d) with a %d-point axis: %s", q.img_ny, q.img_nx, q.ny, q.nx,
+                     kMaxSide, why);
+            return BSGP_E_SHAPE;
+        }
+    }
+    // Frame mode (bsgp_device.cuh, GridCtx): images of a megapixel or more, and every grid with a 16384-point axis, get the
+    // whole GPU each, one CTA per SM on the largest power of two of SMs that divides the image
+    L.frame = q.want_G == -1 || (q.want_G == 0 && (npix >= ((size_t)1 << 20) || long_axis));
     int G = q.want_G > 0 ? q.want_G : 1;
     if (L.frame) {
         while (2 * G <= q.num_sms && q.ny % (4 * G) == 0 && (q.nx / 2) % (2 * G) == 0) G *= 2;
@@ -175,9 +208,6 @@ template <typename T> inline int plan_launch(const PlanRequest& q, LaunchPlan* o
     // several CTAs takes the large-slab shapes whatever its slab size (with DeviceCtxSmall its CTAs would each see their
     // own partial sums, take different control paths and never meet at the next cluster barrier).
     const bool small_slab = !L.frame && G == 1 && npix / G * sizeof(T) <= 16384;
-    // short sides that are not a power of two: dense DFT of the image's own length on the first slots of the grid
-    // (bsgp_wrap.h); make_geom refuses them for more than one CTA per image, frame mode included
-    const int dny = q.ny != q.img_ny ? dense_len(q.img_ny) : 0, dnx = q.nx != q.img_nx ? dense_len(q.img_nx) : 0;
     // Small slabs, automatic configuration: three 128-thread CTAs per SM if everything but the background image stays
     // resident in a third of the SM's shared memory (32 x 32 fp64 stamps: 8192 stamps 19.7 ms against 22.8 ms for two
     // 256-thread CTAs); otherwise (e.g. 31 x 31 cut-outs, whose tensor-core table takes 8 KB) two 256-thread CTAs.
@@ -187,6 +217,11 @@ template <typename T> inline int plan_launch(const PlanRequest& q, LaunchPlan* o
         L.minb = L.threads >= 512 ? 1 : (L.threads >= 256 ? (small_slab ? 2 : 1) : (small_slab ? 3 : 4));
         const size_t ws_limit = L.frame ? 160 * 1024 : (L.minb >= 4 ? 38 : 76) * 1024;
         bool ok = make_geom(q.ny, q.nx, G, sizeof(cplx<T>), ws_limit, &L.g, &L.ws_bytes, dny, dnx);
+        if (!ok && L.frame && !dny && !dnx) {
+            // one transform of an axis does not fit the frame workspace (fp64 16384): split transforms along that axis only
+            const int split = split_axes(q.ny, q.nx, sizeof(cplx<T>), ws_limit);
+            ok = split && make_geom(q.ny, q.nx, G, sizeof(cplx<T>), ws_limit, &L.g, &L.ws_bytes, 0, 0, split);
+        }
         if (!ok && !L.frame && auto_threads) {
             // one transform does not fit the small workspace (sides >= 4096): fall back to one big CTA per SM
             L.threads = 512; L.minb = 1;

@@ -4,6 +4,6 @@
 namespace bsgp {
 template cudaError_t launch_solve<float, true>(const LaunchCfg&, const SolveArgs<float>&, const SmemPlan&, size_t, const RowArgs*);
 template cudaError_t query_solve_clusters<float, true>(const LaunchCfg&, int, int*);
-template cudaError_t launch_frame<float, true>(const LaunchCfg&, const SolveArgs<float>&, const SmemPlan&, size_t, double*, const RowArgs*);
-template cudaError_t query_frame_ctas<float, true>(const LaunchCfg&, int*);
+template cudaError_t launch_frame<float, true>(const LaunchCfg&, const SolveArgs<float>&, const SmemPlan&, size_t, double*, const RowArgs*, bool);
+template cudaError_t query_frame_ctas<float, true>(const LaunchCfg&, int*, bool);
 }  // namespace bsgp

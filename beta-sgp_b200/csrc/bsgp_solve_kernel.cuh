@@ -45,8 +45,10 @@ __device__ __forceinline__ ImgState<T>* solve_prologue(Ctx& ctx, unsigned char* 
     }
     cplx<T>* twx_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twx);
     cplx<T>* twy_s = reinterpret_cast<cplx<T>*>(smem + sp.off_twy);
-    fill_twiddles(ctx, sp.tw_smem, a.g.nx, a.twx, twx_s, Ctx::kFrame ? 0 : a.g.px.dft_n);
-    if (sp.off_twy != sp.off_twx) fill_twiddles(ctx, sp.tw_smem, a.g.ny, a.twy, twy_s, Ctx::kFrame ? 0 : a.g.py.dft_n);
+    // the tables of the FFT plans: of nx / 2 or ny / 2 points on a split axis (bsgp_conv.cuh, split transforms)
+    constexpr bool kSplit = is_split<Ctx>::value;
+    fill_twiddles(ctx, sp.tw_smem, kSplit ? a.g.px.n : a.g.nx, a.twx, twx_s, Ctx::kFrame ? 0 : a.g.px.dft_n);
+    if (sp.off_twy != sp.off_twx) fill_twiddles(ctx, sp.tw_smem, kSplit ? a.g.py.n : a.g.ny, a.twy, twy_s, Ctx::kFrame ? 0 : a.g.py.dft_n);
     fill_pos_table(ctx, a.g.px, reinterpret_cast<unsigned short*>(smem + sp.off_ppx));
     if (ctx.tid == 0) {
         S->geom = a.g;
@@ -102,11 +104,10 @@ __global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T>
 }
 
 // Frame mode (GridCtx): the images of the batch are restored one after the other, each by the whole grid.
-template <typename T, bool MK, bool ROWS, typename... R>
-__global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart,
-                                                            const R... ra) {
+template <typename T, bool MK, bool ROWS, class Ctx, typename... R>
+__device__ __forceinline__ void frame_body(const SolveArgs<T>& a, const SmemPlan& sp, const size_t tf_stride, double* gpart, const R&... ra) {
     unsigned char* smem = dyn_smem();
-    CtxOf<ROWS, GridCtx> ctx;
+    Ctx ctx;
     static_cast<GridCtx&>(ctx) = make_grid_ctx(reinterpret_cast<SharedCtl*>(smem), gpart);
     T* buf[NBUF];
     ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
@@ -118,28 +119,55 @@ __global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a
     }
 }
 
+template <typename T, bool MK, bool ROWS, typename... R>
+__global__ void __launch_bounds__(512, 1) bsgp_frame_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart,
+                                                            const R... ra) {
+    frame_body<T, MK, ROWS, CtxOf<ROWS, GridCtx>>(a, sp, tf_stride, gpart, ra...);
+}
+
+// the same for plans with a split axis (SplitCtx, bsgp_conv.cuh): a kernel of its own, so that the frame kernel above keeps its code
+template <typename T, bool MK, bool ROWS, typename... R>
+__global__ void __launch_bounds__(512, 1) bsgp_frame_split_kernel(const SolveArgs<T> a, const SmemPlan sp, const size_t tf_stride, double* gpart,
+                                                                  const R... ra) {
+    frame_body<T, MK, ROWS, CtxOf<ROWS, SplitCtx<GridCtx>>>(a, sp, tf_stride, gpart, ra...);
+}
+
 // frame_kernel_ptr / solve_kernel_ptr: the kernel without rows, or with a RowArgs parameter
-template <typename T, bool MK, bool ROWS> static const void* frame_kernel_ptr() {
-    if constexpr (ROWS) return (const void*)bsgp_frame_kernel<T, MK, true, RowArgs>;
-    else return (const void*)bsgp_frame_kernel<T, MK, false>;
+template <typename T, bool MK, bool ROWS, bool SPLIT = false> static const void* frame_kernel_ptr() {
+    if constexpr (SPLIT) {
+        if constexpr (ROWS) return (const void*)bsgp_frame_split_kernel<T, MK, true, RowArgs>;
+        else return (const void*)bsgp_frame_split_kernel<T, MK, false>;
+    } else {
+        if constexpr (ROWS) return (const void*)bsgp_frame_kernel<T, MK, true, RowArgs>;
+        else return (const void*)bsgp_frame_kernel<T, MK, false>;
+    }
+}
+
+// split: the plan has a split axis (fp64 only: an fp32 transform of every supported length fits the workspace)
+template <typename T, bool MK> static const void* frame_fn(bool rows, bool split) {
+    if constexpr (sizeof(T) == 8) {
+        if (split) return rows ? frame_kernel_ptr<T, MK, true, true>() : frame_kernel_ptr<T, MK, false, true>();
+    }
+    return rows ? frame_kernel_ptr<T, MK, true>() : frame_kernel_ptr<T, MK, false>();
 }
 
 template <typename T, bool MK>
-cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart, const RowArgs* rows) {
+cudaError_t launch_frame(const LaunchCfg& lc, const SolveArgs<T>& a, const SmemPlan& sp, size_t tf_stride, double* gpart, const RowArgs* rows,
+                         bool split) {
     SolveArgs<T> args = a;
     SmemPlan plan = sp;
     size_t tfs = tf_stride;
     double* gp = gpart;
     RowArgs ra = rows ? *rows : RowArgs{};
     void* params[] = {&args, &plan, &tfs, &gp, &ra};
-    const void* fn = rows ? frame_kernel_ptr<T, MK, true>() : frame_kernel_ptr<T, MK, false>();
+    const void* fn = frame_fn<T, MK>(rows != nullptr, split);
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc.smem);
     if (e != cudaSuccess) return e;
     return cudaLaunchCooperativeKernel(fn, dim3(lc.grid), dim3(lc.threads), params, lc.smem, lc.stream);
 }
 
-template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm) {
-    const void* fn = frame_kernel_ptr<T, MK, false>();
+template <typename T, bool MK> cudaError_t query_frame_ctas(const LaunchCfg& lc, int* per_sm, bool split) {
+    const void* fn = frame_fn<T, MK>(false, split);
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc.smem);
     if (e != cudaSuccess) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, fn, lc.threads, lc.smem);

@@ -20,7 +20,11 @@
 
 namespace bsgp {
 
-constexpr int kMaxSide = 8192;
+// Largest grid side: power-of-two sides up to kMaxSide run on their own grid; any other side up to kMaxSide / 2 wraps onto
+// a grid of at most kMaxSide (2 n - 1 <= kMaxSide - 1).  Grid sides above kMaxClusterSide run in frame mode only
+// (bsgp_plan.h, plan_launch).
+constexpr int kMaxSide = 16384;
+constexpr int kMaxClusterSide = 8192;
 constexpr int kMaxDense = 32;
 
 // Short sides that are not a power of two (n <= 32: the reference's 31 x 31 cut-outs) do not wrap: they keep a grid of

@@ -451,8 +451,8 @@ def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtyp
     psf_h = psf.detach().cpu().numpy() if _is_tensor(psf) else np.asarray(psf)
     psf_h = np.asarray(psf_h, dtype=np.float64)
     geo = PaddedGeometry(ny, nx, psf_h.shape[-2], psf_h.shape[-1])
-    if geo.P > 8192:
-        raise ValueError(f"padded grid {geo.P} exceeds the largest supported side (8192)")
+    if geo.P > 16384:
+        raise ValueError(f"padded grid {geo.P} exceeds the largest supported side (16384)")
     plan = get_plan(geo.P, geo.P, dtype, device)
     big, div_a = geo.kernel(psf_h, npdt)
     bigt, div_at = geo.kernel(np.conj(np.swapaxes(psf_h, -1, -2)), npdt)          # psf.conj().T, sgp.py:157

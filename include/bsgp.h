@@ -17,10 +17,11 @@
  * CUDA device every compute entry point fails with BSGP_E_CUDA.
  *
  * Shapes.  Any ny x nx (the reference's numpy closure accepts any size, sgp.py:108-120; its star-stamp application
- * uses 31 x 31 cut-outs, application_sgp_star_stamps.py:24,58).  Sides that are powers of two in [16, 8192] run on
+ * uses 31 x 31 cut-outs, application_sgp_star_stamps.py:24,58).  Sides that are powers of two in [16, 16384] run on
  * their own FFT grid and need 16-byte aligned image pointers.  Any other side n <= 32 keeps a grid of 16 or 32 slots and
- * is transformed by a dense DFT of length n; any other side n <= 4096 runs on a grid of side 2^k >= 2n - 1 ("wrapped":
- * linear convolution + fold).  Both are exactly the circular operator with the reference's np.fft.fftshift placement,
+ * is transformed by a dense DFT of length n; any other side n <= 8192 runs on a grid of side 2^k >= 2n - 1 ("wrapped":
+ * linear convolution + fold).  A grid with a 16384-point side runs in frame mode and cannot pair with a dense axis
+ * (BSGP_E_SHAPE otherwise); in BSGP_F64 its 16384-point axes run split transforms of two 8192-point halves.  Both are exactly the circular operator with the reference's np.fft.fftshift placement,
  * including its one-pixel offset for odd n; the library moves the caller's arrays to and from the grid itself and only
  * needs element alignment.
  *
@@ -138,7 +139,8 @@ typedef struct bsgp_plan_info {
 } bsgp_plan_info;
 
 /* One plan per (shape, dtype, device): twiddle tables, per-cluster scratch, PSF spectra.  Any shape with sides in
- * [1, 8192] (powers of two) or [1, 4096] (other sizes, see "Shapes" above). */
+ * [1, 16384] (powers of two) or [1, 8192] (other sizes), with the limits on 16384-point grids of "Shapes" above.
+ * BSGP_E_NOMEM (with the size in bsgp_last_error_string) when the device cannot hold the plan's buffers. */
 int bsgp_plan_create(int ny, int nx, int dtype, int device, bsgp_plan** plan);
 int bsgp_plan_destroy(bsgp_plan* plan);
 int bsgp_plan_get_info(const bsgp_plan* plan, bsgp_plan_info* info);
