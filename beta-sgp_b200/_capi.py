@@ -40,7 +40,8 @@ class Params(C.Structure):
 
 class Inputs(C.Structure):
     _fields_ = [("gn", C.c_void_p), ("bkg", C.c_void_p), ("bkg_is_image", C.c_int), ("flux", C.c_void_p),
-                ("beta0", C.c_void_p), ("x0", C.c_void_p), ("obj", C.c_void_p), ("order", C.c_void_p)]
+                ("beta0", C.c_void_p), ("x0", C.c_void_p), ("obj", C.c_void_p), ("order", C.c_void_p),
+                ("source", C.c_void_p), ("n_sources", C.c_int)]
 
 
 class Outputs(C.Structure):

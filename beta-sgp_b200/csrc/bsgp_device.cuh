@@ -265,11 +265,15 @@ __device__ __forceinline__ int poll_ready(const int* flag) {
 }
 
 // next work item for the whole cluster (leader claims it, waits for its upload if there is one, and pushes the item and
-// the verdict into every CTA's shared memory).  *ready_ok = false: the item's inputs never arrived.
-__device__ __forceinline__ int next_item(DeviceCtx& ctx, int* queue, const int* ready, int batch, bool* ready_ok) {
+// the verdict into every CTA's shared memory).  *ready_ok = false: the item's inputs never arrived.  The flags belong to
+// the queue items, or with a source map (source != NULL, the mixed-batch kernels only) to the observations: item v then
+// waits for the flag of the observation its solve order[v] reads.
+__device__ __forceinline__ int next_item(DeviceCtx& ctx, int* queue, const int* ready, int batch, bool* ready_ok,
+                                         const int* order = nullptr, const int* source = nullptr) {
     if (ctx.rank == 0 && ctx.tid == 0) {
         const int v = atomicAdd(queue, 1);
-        const int ok = (ready && v < batch) ? poll_ready(ready + v) : 1;
+        const int f = (source && v < batch) ? source[order ? order[v] : v] : v;
+        const int ok = (ready && v < batch) ? poll_ready(ready + f) : 1;
         if (ctx.G > 1) {
             cg::cluster_group cl = cg::this_cluster();
             for (int r = 0; r < ctx.G; ++r) { *cl.map_shared_rank(&ctx.sh->next_img, r) = v; *cl.map_shared_rank(&ctx.sh->ready_verdict, r) = ok; }

@@ -384,6 +384,8 @@ struct bsgp_plan : LaunchPlan {
     // staging arena `stage`: the device entry point has no staging area, and the pinned path's arena is still being filled
     // on its copy stream when the rows go up on the launch stream.
     bsgp_params* rows = nullptr; size_t rows_cap = 0;
+    // grow-only: the source map of the last launch with one (bsgp_inputs.source), on the launch stream like the rows
+    int* source = nullptr; size_t source_cap = 0;
 };
 
 template <typename T> static const void* conv_kernel_ptr() { return (const void*)bsgp_conv_kernel<T>; }
@@ -401,8 +403,9 @@ static int dev_alloc(void** buf, size_t bytes, const char* what) {
 
 static void plan_free_pipeline(bsgp_plan* p) {
     cudaFree(p->stage); cudaFree(p->ready); cudaFreeHost(p->ones_host);
-    cudaFree(p->emb_psf); cudaFree(p->emb_img); cudaFree(p->rows);
+    cudaFree(p->emb_psf); cudaFree(p->emb_img); cudaFree(p->rows); cudaFree(p->source);
     p->emb_psf = p->emb_img = nullptr; p->emb_psf_cap = p->emb_img_cap = 0; p->rows = nullptr; p->rows_cap = 0;
+    p->source = nullptr; p->source_cap = 0;
     if (p->ev_last) { cudaEventDestroy(p->ev_last); p->ev_last = nullptr; }
     p->stage = nullptr; p->stage_cap = 0; p->ready = nullptr; p->ones_host = nullptr; p->ready_cap = 0;
     if (p->s_copy) cudaStreamDestroy(p->s_copy);
@@ -630,21 +633,23 @@ template <typename T>
 static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready);
 
 // wrapped plans: move the caller's arrays onto the grid, solve there with the image window as the valid region (the
-// zero-padded operator's masked kernels) and the fold of the geometry, crop the restored images
+// zero-padded operator's masked kernels) and the fold of the geometry, crop the restored images.  Inputs are embedded once
+// per observation (bsgp_inputs.source), the restored images are one per solve.
 template <typename T>
 static int solve_t(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, cudaStream_t st, const int* ready) {
     if (!p->embedded) return solve_grid<T>(p, kw, batch, in, out, st, ready);
-    const size_t gb = (size_t)batch * p->ny * p->nx * sizeof(T);
-    const int narr = 2 + (in->bkg_is_image ? 1 : 0) + (in->x0 ? 1 : 0) + (in->obj ? 1 : 0);
-    int rc = grow(&p->emb_img, &p->emb_img_cap, (size_t)narr * gb, "the images on the FFT grid");
+    const size_t nobs = (size_t)observation_count(in, batch);
+    const size_t gb = (size_t)batch * p->ny * p->nx * sizeof(T), ob = nobs * p->ny * p->nx * sizeof(T);
+    const int narr = 1 + (in->bkg_is_image ? 1 : 0) + (in->x0 ? 1 : 0) + (in->obj ? 1 : 0);
+    int rc = grow(&p->emb_img, &p->emb_img_cap, (size_t)narr * ob + gb, "the images on the FFT grid");
     if (rc) return rc;
     char* base = (char*)p->emb_img;
     int k = 0;
     auto up = [&](const void* src, const void** dst) -> int {
         if (!src) { *dst = nullptr; return BSGP_OK; }
-        void* d = base + (size_t)(k++) * gb;
+        void* d = base + (size_t)(k++) * ob;
         *dst = d;
-        return embed_images<T>(p, src, d, (size_t)batch, st);
+        return embed_images<T>(p, src, d, nobs, st);
     };
     bsgp_inputs gi = *in;
     bsgp_outputs go = *out;
@@ -652,7 +657,7 @@ static int solve_t(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_input
     if (in->bkg_is_image && (rc = up(in->bkg, &gi.bkg))) return rc;
     if ((rc = up(in->x0, &gi.x0))) return rc;
     if ((rc = up(in->obj, &gi.obj))) return rc;
-    go.x = base + (size_t)(k++) * gb;
+    go.x = base + (size_t)k * ob;
     bsgp_params q = *kw.prm;
     q.region[0] = 0; q.region[1] = p->img_ny; q.region[2] = 0; q.region[3] = p->img_nx;
     q.div_a = q.div_at = 1.0;
@@ -680,7 +685,7 @@ static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_in
     a.tr_beta = out->trace_beta; a.tr_trials = out->trace_trials; a.tr_evals = out->trace_evals;
     a.queue = p->queue;
     a.ready = p->frame ? nullptr : ready;
-    const RowArgs ra{kw.rows, kw.trace_stride};
+    const RowArgs ra{kw.rows, kw.trace_stride, in->source};
     const RowArgs* rows = kw.rows ? &ra : nullptr;                  // no rows: the kernels compiled without them
     if (p->frame) {
         LaunchCfg fc{p->g.G, 512, 1, p->smem_bytes, st, 1};
@@ -846,7 +851,8 @@ static int check_solve(const bsgp_plan* p, const bsgp_params* prm, const bsgp_pa
     char err[256];
     int rc = check_batch_params(prm, rows, batch, in, out, &kw->trace_stride, err, sizeof err);
     if (rc) return fail(rc, "%s", err);
-    if (p->n_psf != 1 && p->n_psf != batch) return fail(BSGP_E_STATE, "bsgp_set_psf was called with %d PSFs; need 1 or batch (%d)", p->n_psf, batch);
+    if ((rc = check_sources(in, batch, err, sizeof err))) return fail(rc, "%s", err);
+    if ((rc = check_psf_count(p->n_psf, in, batch, err, sizeof err))) return fail(rc, "%s", err);
     if (!in->gn || !in->bkg || !out->x || !out->iters || !out->status || !out->discr || !out->times) return fail(BSGP_E_ARG, "required pointer is NULL");
     if (p->n_psf < 1) return fail(BSGP_E_STATE, "bsgp_set_psf has not been called");
     if (prm->adjoint_second_psf && (p->tf_adj == nullptr || p->n_psf_adj != p->n_psf))
@@ -864,7 +870,9 @@ static int check_solve(const bsgp_plan* p, const bsgp_params* prm, const bsgp_pa
 }
 
 // launch on device arrays that passed check_solve; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0.
-// The host rows of a mixed batch go up to the plan's row buffer on the launch's stream, behind the plan's previous launch.
+// The host rows of a mixed batch go up to the plan's row buffer on the launch's stream, behind the plan's previous launch,
+// and so does a source map.  A launch with a map runs the mixed-batch kernels: shared keywords become equal rows here.
+// `ready` is then indexed by observation.
 static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
     if (!p->embedded && (misaligned(in->gn) || misaligned(out->x) || misaligned(in->x0) || misaligned(in->obj) || (in->bkg_is_image && misaligned(in->bkg))))
         return fail(BSGP_E_ARG, "image pointers must be 16-byte aligned (vector loads)");
@@ -873,12 +881,24 @@ static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_
     int rc = plan_enter(p, st);
     if (rc) return rc;
     Keywords dk = kw;
-    if (kw.rows) {
+    std::vector<bsgp_params> uniform;
+    if (in->source && !kw.rows) { uniform.assign((size_t)batch, *kw.prm); dk.rows = uniform.data(); }
+    if (dk.rows) {
         const size_t bytes = (size_t)batch * sizeof(bsgp_params);
         if ((rc = grow((void**)&p->rows, &p->rows_cap, bytes, "the per-image keywords"))) return rc;
-        CU(cudaMemcpyAsync(p->rows, kw.rows, bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(p->rows, dk.rows, bytes, cudaMemcpyHostToDevice, st));
         dk.rows = p->rows;
     }
+    bsgp_inputs din = *in;
+    if (in->source) {
+        // copied through pageable memory, which cudaMemcpyAsync stages before it returns: the caller's map is read here
+        const std::vector<int> map(in->source, in->source + batch);
+        const size_t bytes = (size_t)batch * sizeof(int);
+        if ((rc = grow((void**)&p->source, &p->source_cap, bytes, "the source map"))) return rc;
+        CU(cudaMemcpyAsync(p->source, map.data(), bytes, cudaMemcpyHostToDevice, st));
+        din.source = p->source;
+    }
+    in = &din;
     rc = p->dtype == BSGP_F64 ? solve_t<double>(p, dk, batch, in, out, st, ready) : solve_t<float>(p, dk, batch, in, out, st, ready);
     if (rc) return rc;
     return plan_leave(p, st);
@@ -918,7 +938,7 @@ struct DevBuf {
 // The host I/O of one solve, laid out in one device staging area: the caller's pointer of every array (nullptr: absent),
 // its size for this batch and its offset in the area, inputs first, then the outputs, which are zero-filled before the
 // launch and copied back after it.  The restored images are staged too, unless the kernel stores them straight into
-// host memory through `x_mapped`.
+// host memory through `x_mapped`.  The image-shaped inputs hold one image per observation (bsgp_inputs.source).
 struct HostIO {
     enum Slot { GN, BKG, X0, OBJ, FLUX, BETA0, ORDER,                 // inputs, the image-shaped ones first
                 X, ITERS, STATUS, DISCR, TIMES, STOP_VALUE, ERR, BETA_FINAL, PROJ_EVALS, LS_TRIALS, SCALARS,
@@ -929,15 +949,18 @@ struct HostIO {
     size_t img;                           // bytes of one image
     int bkg_is_image;
     void* x_mapped;
+    const int* source; int n_sources;     // the caller's map (host memory), passed on as it is
 
     HostIO(const bsgp_plan* p, int trace_stride, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* x_mapped_)
-        : img((size_t)p->img_ny * p->img_nx * p->elem), bkg_is_image(in->bkg_is_image), x_mapped(x_mapped_) {
+        : img((size_t)p->img_ny * p->img_nx * p->elem), bkg_is_image(in->bkg_is_image), x_mapped(x_mapped_), source(in->source),
+          n_sources(in->n_sources) {
         const size_t B = (size_t)batch, tr = (size_t)trace_stride, imgs = B * img, it8 = B * tr * 8, it4 = B * tr * 4;
+        const size_t O = (size_t)observation_count(in, batch), obs = O * img;
         const void* const h[NSLOT] = {in->gn, in->bkg, in->x0, in->obj, in->flux, in->beta0, in->order,
                                       x_mapped ? nullptr : out->x, out->iters, out->status, out->discr, out->times, out->stop_value,
                                       out->err, out->beta_final, out->proj_evals, out->ls_trials, out->scalars,
                                       out->trace_alpha, out->trace_lambda, out->trace_beta, out->trace_trials, out->trace_evals};
-        const size_t n[NSLOT] = {imgs, bkg_is_image ? imgs : B * p->elem, imgs, imgs, B * 8, B * 8, B * 4,
+        const size_t n[NSLOT] = {obs, bkg_is_image ? obs : O * p->elem, obs, obs, B * 8, B * 8, B * 4,
                                  imgs, B * 4, B * 4, it8, it8, it8,
                                  B * (tr + 1) * 8, B * 8, B * 4, B * 4, B * BSGP_NSCALARS * 8,
                                  it8, it8, it8, it4, it4};
@@ -952,7 +975,7 @@ struct HostIO {
     int launch(bsgp_plan* p, const Keywords& kw, int batch, char* base, void* stream, const int* ready) const {
         auto dev = [&](int k) -> void* { return host[k] ? base + off[k] : nullptr; };
         const bsgp_inputs in = {dev(GN), dev(BKG), bkg_is_image, (const double*)dev(FLUX), (const double*)dev(BETA0), dev(X0), dev(OBJ),
-                                (const int*)dev(ORDER)};
+                                (const int*)dev(ORDER), source, n_sources};
         const bsgp_outputs out = {x_mapped ? x_mapped : dev(X), (int*)dev(ITERS), (int*)dev(STATUS), (double*)dev(DISCR), (double*)dev(TIMES),
                                   (double*)dev(STOP_VALUE), (double*)dev(ERR), (double*)dev(BETA_FINAL), (int*)dev(PROJ_EVALS),
                                   (int*)dev(LS_TRIALS), (double*)dev(SCALARS), (double*)dev(TRACE_ALPHA), (double*)dev(TRACE_LAMBDA),
@@ -998,6 +1021,8 @@ static int solve_host(bsgp_plan* p, const bsgp_params* prm, const bsgp_params* r
 //                   come back with ordinary copies after the kernel.
 // Small images (< 64 KB) with a permuted queue would need one tiny copy per image; they are uploaded as whole arrays
 // instead (one flag write for everything), still with the zero-copy output.  Frame mode: upload, then launch.
+// With a source map (bsgp_inputs.source) every observation goes up once, in the order of its first use in the queue, and
+// the flags belong to the observations: the kernel waits for the flag of the observation a solve reads.
 // ---------------------------------------------------------------------------------------------
 static bool page_locked(const void* h) {
     if (!h) return true;
@@ -1017,18 +1042,20 @@ static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params*
     void* x_mapped = nullptr;
     CU(cudaHostGetDevicePointer(&x_mapped, out->x, 0));
     const HostIO io(p, kw.trace_stride, batch, in, out, x_mapped);
-    const size_t img = io.img, B = (size_t)batch;
+    const size_t img = io.img;
+    const int nobs = observation_count(in, batch);
+    const size_t F = (size_t)(in->source ? nobs : batch);          // ready flags: per queue item, or per observation
     // images in the caller's own shape: a plan whose grid differs from it (sides that are not a power of two) moves them
     // to and from the grid on the device (solve_t), which needs all of them resident first, like frame mode
     const bool resident_first = p->frame || p->embedded;
     TRY(grow(&p->stage, &p->stage_cap, io.size, "the staging area"));
-    if (batch > p->ready_cap) {
+    if ((int)F > p->ready_cap) {
         CU(cudaDeviceSynchronize());
         cudaFree(p->ready); cudaFreeHost(p->ones_host); p->ready = nullptr; p->ones_host = nullptr; p->ready_cap = 0;
-        CU(cudaMalloc((void**)&p->ready, B * sizeof(int)));
-        CU(cudaHostAlloc((void**)&p->ones_host, B * sizeof(int), cudaHostAllocDefault));
-        for (int i = 0; i < batch; ++i) p->ones_host[i] = 1;
-        p->ready_cap = batch;
+        CU(cudaMalloc((void**)&p->ready, F * sizeof(int)));
+        CU(cudaHostAlloc((void**)&p->ones_host, F * sizeof(int), cudaHostAllocDefault));
+        for (size_t i = 0; i < F; ++i) p->ones_host[i] = 1;
+        p->ready_cap = (int)F;
     }
     if (!p->s_copy) {
         CU(cudaStreamCreateWithFlags(&p->s_copy, cudaStreamNonBlocking));
@@ -1045,7 +1072,7 @@ static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params*
     for (int k = 0; k < HostIO::X; ++k)
         if (io.host[k] && !io.image(k)) CU(cudaMemcpyAsync(S + io.off[k], io.host[k], io.bytes[k], cudaMemcpyHostToDevice, sr));
     CU(cudaMemsetAsync(S + io.out_begin, 0, io.size - io.out_begin, sr));
-    CU(cudaMemsetAsync(p->ready, 0, B * sizeof(int), sr));
+    CU(cudaMemsetAsync(p->ready, 0, F * sizeof(int), sr));
     CU(cudaEventRecord(p->ev_flags, sr));
     CU(cudaStreamWaitEvent(sc, p->ev_flags, 0));                   // no flag may be raised before the flags are cleared
     // ---- copy stream: items [first, first + n) of every image-shaped input, then the flags that hand them to the kernel
@@ -1055,24 +1082,40 @@ static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params*
                 CU(cudaMemcpyAsync(S + io.off[k] + first * img, (const char*)io.host[k] + first * img, n * img, cudaMemcpyHostToDevice, sc));
         return BSGP_OK;
     };
-    const bool per_item = !p->frame && (img >= 65536 || in->order == nullptr);
+    // the observations in the order the queue first needs them: without a map queue item i reads image order[i] and owns
+    // flag i; with one, the observations in the order of their first use, each owning its own flag
+    std::vector<int> seq;
+    bool in_order = in->order == nullptr;
+    if (in->source) {
+        std::vector<char> seen((size_t)nobs, 0);
+        for (int i = 0; i < batch; ++i) {
+            const int o = in->source[in->order ? in->order[i] : i];
+            if (!seen[o]) { seen[o] = 1; seq.push_back(o); }
+        }
+        in_order = true;
+        for (size_t i = 0; i < seq.size(); ++i) in_order = in_order && seq[i] == (int)i;
+    }
+    const int nseq = in->source ? (int)seq.size() : batch;
+    auto obs_at = [&](int i) { return in->source ? seq[i] : (in->order ? in->order[i] : i); };
+    const bool per_item = !p->frame && (img >= 65536 || in_order);
     auto feed = [&]() -> int {
         if (resident_first) {                                      // no per-item hand-over: everything resident first
-            TRY(upload(0, B));
+            TRY(upload(0, (size_t)nobs));
             CU(cudaEventRecord(p->ev_copy, sc));
             CU(cudaStreamWaitEvent(sr, p->ev_copy, 0));
         } else if (!per_item) {
-            TRY(upload(0, B));
-            CU(cudaMemcpyAsync(p->ready, p->ones_host, B * sizeof(int), cudaMemcpyHostToDevice, sc));
+            TRY(upload(0, (size_t)nobs));
+            CU(cudaMemcpyAsync(p->ready, p->ones_host, F * sizeof(int), cudaMemcpyHostToDevice, sc));
         } else {
             // images in queue order, flags behind them; consecutive queue items that are also consecutive in memory
             // travel as one copy of <= ~1 MB per array
             const size_t max_run = img >= ((size_t)1 << 20) ? 1 : (((size_t)1 << 20) / img);
-            for (int i0 = 0, n = 0; i0 < batch; i0 += n) {
-                const int first = in->order ? in->order[i0] : i0;
-                for (n = 1; i0 + n < batch && (size_t)n < max_run && (in->order ? in->order[i0 + n] : i0 + n) == first + n;) ++n;
+            for (int i0 = 0, n = 0; i0 < nseq; i0 += n) {
+                const int first = obs_at(i0);
+                for (n = 1; i0 + n < nseq && (size_t)n < max_run && obs_at(i0 + n) == first + n;) ++n;
                 TRY(upload((size_t)first, (size_t)n));
-                CU(cudaMemcpyAsync(p->ready + i0, p->ones_host, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, sc));
+                const int flag = in->source ? first : i0;
+                CU(cudaMemcpyAsync(p->ready + flag, p->ones_host, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, sc));
             }
         }
         return BSGP_OK;

@@ -64,4 +64,31 @@ inline int check_batch_params(const bsgp_params* prm, const bsgp_params* rows, i
     return BSGP_OK;
 }
 
+// The observations of a batch (bsgp_inputs.source, host memory): without a map, image i is observation i; with one, every
+// entry must name one of n_sources >= 1 observations, since the kernels index gn, bkg, x0, obj and the PSF spectra with it.
+inline int check_sources(const bsgp_inputs* in, int batch, char* err, size_t errlen) {
+    if (!in->source) return BSGP_OK;
+    if (in->n_sources < 1) {
+        snprintf(err, errlen, "n_sources must be >= 1 with a source map (got %d)", in->n_sources);
+        return BSGP_E_ARG;
+    }
+    for (int i = 0; i < batch; ++i)
+        if (in->source[i] < 0 || in->source[i] >= in->n_sources) {
+            snprintf(err, errlen, "solve %d: source %d is outside 0..%d", i, in->source[i], in->n_sources - 1);
+            return BSGP_E_ARG;
+        }
+    return BSGP_OK;
+}
+
+// The number of observations a batch reads: n_sources with a map, else one per image.
+inline int observation_count(const bsgp_inputs* in, int batch) { return in->source ? in->n_sources : batch; }
+
+// PSF spectra set on the plan: one for all, or one per observation.
+inline int check_psf_count(int n_psf, const bsgp_inputs* in, int batch, char* err, size_t errlen) {
+    if (n_psf == 1 || n_psf == observation_count(in, batch)) return BSGP_OK;
+    if (in->source) snprintf(err, errlen, "bsgp_set_psf was called with %d PSFs; need 1 or n_sources (%d)", n_psf, in->n_sources);
+    else snprintf(err, errlen, "bsgp_set_psf was called with %d PSFs; need 1 or batch (%d)", n_psf, batch);
+    return BSGP_E_STATE;
+}
+
 }  // namespace bsgp

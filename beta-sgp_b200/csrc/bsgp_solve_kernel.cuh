@@ -90,15 +90,18 @@ __global__ void __launch_bounds__(NT, MINB) bsgp_solve_kernel(const SolveArgs<T>
     ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
     for (;;) {
         bool ready_ok;
-        const int item = next_item(ctx, a.queue, a.ready, a.batch, &ready_ok);
+        int item;
+        if constexpr (ROWS) item = next_item(ctx, a.queue, a.ready, a.batch, &ready_ok, a.order, ra.source...);   // flags by observation
+        else item = next_item(ctx, a.queue, a.ready, a.batch, &ready_ok);
         if (item >= a.batch) break;
         const int img = a.order ? a.order[item] : item;
         if (!ready_ok) {                                   // upload never arrived: report and skip (cluster-uniform)
             if (ctx.rank == 0 && ctx.tid == 0) { a.status[img] = BSGP_ST_INPUT_TIMEOUT; a.iters[img] = 0; }
             continue;
         }
-        cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)img * tf_stride : 0);
-        cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)img * tf_stride : 0) : tf;
+        const int obs = source_of(img, ra...);             // the spectrum of the observation the solve reads
+        cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)obs * tf_stride : 0);
+        cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)obs * tf_stride : 0) : tf;
         solve_image<T, MK, ROWS>(ctx, a, S, buf, tf, tfa, img, ra...);
     }
 }
@@ -112,8 +115,9 @@ __device__ __forceinline__ void frame_body(const SolveArgs<T>& a, const SmemPlan
     T* buf[NBUF];
     ImgState<T>* S = solve_prologue(ctx, smem, a, sp, buf);
     for (int img = 0; img < a.batch; ++img) {
-        cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)img * tf_stride : 0);
-        cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)img * tf_stride : 0) : tf;
+        const int obs = source_of(img, ra...);
+        cplx<T>* tf = a.tf + (a.n_psf > 1 ? (size_t)obs * tf_stride : 0);
+        cplx<T>* tfa = a.tf_adj ? a.tf_adj + (a.n_psf > 1 ? (size_t)obs * tf_stride : 0) : tf;
         solve_image<T, MK, ROWS>(ctx, a, S, buf, tf, tfa, img, ra...);
         ctx.cluster_sync();          // the scratch arrays and the exchange buffer are reused by the next image
     }

@@ -69,8 +69,13 @@ template <typename T> struct SolveArgs {
 // (region, divisors, adjoint kernel) still come from SolveArgs::p.  trace_stride: the per-image stride of discr / times /
 // stop_value / trace_* (err: + 1), the largest maxit + 1 of the rows.  Only the ROWS kernels take it: a launch without rows
 // runs kernels compiled exactly as before the feature existed.
-struct RowArgs { const bsgp_params* rows; int trace_stride; };
+// source: [batch] (device) or NULL: the observation each solve reads (bsgp_inputs.source).  A launch with a map always runs
+// the ROWS kernels (the host expands shared keywords into equal rows), so the kernels without rows never see one.
+struct RowArgs { const bsgp_params* rows; int trace_stride; const int* source; };
 struct NoRow {};
+// the observation solve `img` reads: gn, bkg, x0, obj and the PSF spectra are indexed by it
+BSGP_DEV int source_of(int img) { return img; }
+BSGP_DEV int source_of(int img, const RowArgs& ra) { return ra.source ? ra.source[img] : img; }
 // the keywords the controller reads: the image's own copy of its row, or the batch's
 BSGP_DEV const bsgp_params& image_params(const bsgp_params& own, const bsgp_params&) { return own; }
 BSGP_DEV const bsgp_params& image_params(const NoRow&, const bsgp_params& shared) { return shared; }
@@ -829,9 +834,13 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
     {
         const int nslab = a.g.rows_per_cta * a.g.nx;
         const size_t npix = (size_t)a.g.ny * a.g.nx;
-        const size_t goff = (size_t)img * npix + (size_t)ctx.rank * nslab;
+        // inputs at the offset of the observation the solve reads, the restored image at the solve's own
+        int obs = img;
+        if constexpr (ROWS) obs = source_of(img, ra);
+        const size_t goff = (size_t)obs * npix + (size_t)ctx.rank * nslab;
+        const size_t xoff = (size_t)img * npix + (size_t)ctx.rank * nslab;
         const bool bkg_img = a.bkg_is_image != 0;
-        const T bkg_raw_s = bkg_img ? (T)0 : a.bkg[img];
+        const T bkg_raw_s = bkg_img ? (T)0 : a.bkg[obs];
         if (ctx.tid == 0) {
             S->gn = buf[B_GN]; S->bkg = buf[B_BKG]; S->x = buf[B_X]; S->g = buf[B_G];
             S->xtf = buf[B_XTF]; S->d = buf[B_D]; S->dtf = buf[B_DTF]; S->t1 = buf[B_T1];
@@ -839,7 +848,7 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
             S->bkg_raw = bkg_img ? a.bkg + goff : a.gn + goff;             // never dereferenced when !bkg_img
             S->x0_raw = (P.init_recon == 1) ? a.x0 + goff : a.gn + goff;
             S->truth = want_err ? a.obj + goff : a.gn + goff;
-            S->x_out = a.x_out + goff;
+            S->x_out = a.x_out + xoff;
             S->tf = tf;
             // A^T: conj(TF) of the same PSF (sgp.py:110), or the spectrum of a second kernel, psf.conj().T (sgp.py:157)
             S->tf_at = P.adjoint_second_psf ? tf_adj : tf;

@@ -257,6 +257,38 @@ def _check_per_image(per_image, B):
             raise ValueError(f"per_image[{i}]: divergence must be 'kl' or 'beta'")
 
 
+def _size(a):
+    return int(a.numel()) if _is_tensor(a) else int(np.size(a))
+
+
+def _source_map(source, gn, psf, bkg, flux, betaParam, x0, obj):
+    """solve_batch(source=...): the map as a contiguous host int32 array, after the shape rules of shared observations.
+    gn, bkg, x0, obj and the PSF hold one entry per observation (gn.shape[0] of them); flux and betaParam one per solve."""
+    s = source.detach().cpu().numpy() if _is_tensor(source) else np.asarray(source)
+    if s.ndim != 1 or s.size < 1 or not np.issubdtype(s.dtype, np.integer):
+        raise ValueError("source must be a non-empty 1-D integer array: one observation index per solve")
+    if _ndim(gn) != 3:
+        raise ValueError("gn must be [n_sources, ny, nx] with a source map")
+    n, B = int(gn.shape[0]), int(s.size)
+    bad = np.nonzero((s < 0) | (s >= n))[0]
+    if bad.size:
+        i = int(bad[0])
+        raise ValueError(f"source[{i}] = {int(s[i])} is outside 0..{n - 1}: gn holds {n} observations")
+    if psf is not None and _ndim(psf) == 3 and int(psf.shape[0]) not in (1, n):
+        raise ValueError(f"psf has {int(psf.shape[0])} images; with a source map it is one image or one per observation ({n})")
+    nb = _ndim(bkg)
+    if (nb == 3 and int(bkg.shape[0]) != n) or nb == 2 or (nb == 1 and _size(bkg) not in (1, n)):
+        raise ValueError(f"bkg must be a scalar, [{n}] or [{n}, ny, nx] (one per observation) with a source map; got shape "
+                         f"{tuple(bkg.shape)}")
+    for name, a in (("x0", x0), ("obj", obj)):
+        if a is not None and (_ndim(a) != 3 or int(a.shape[0]) != n):
+            raise ValueError(f"{name} must be [{n}, ny, nx] (one per observation) with a source map; got shape {tuple(a.shape)}")
+    for name, a in (("flux", flux), ("betaParam", betaParam)):
+        if a is not None and _size(a) not in (1, B):
+            raise ValueError(f"{name} is per solve: a scalar or [{B}] with a source map of {B} solves; got {_size(a)} values")
+    return np.ascontiguousarray(s, dtype=np.int32)
+
+
 def _row_betas(betaParam, per_image, B):
     """The call's betaParam with the per-image overrides of per_image, as a host [B] array; betaParam itself if no row
     sets one (a device tensor then stays on the device)."""
@@ -340,8 +372,11 @@ class _Args:
     `vector(a, B, dtype)` (a scalar or [B] array as a contiguous [B] array of a numpy dtype) and `alloc(shape, dtype)`."""
 
     def __init__(self, gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, *, psf_arg, image,
-                 vector, alloc, per_image=None):
-        B = self.B = gn.shape[0]
+                 vector, alloc, per_image=None, source=None):
+        # B solves of n_obs observations: one each, or solve i of observation source[i] (_source_map)
+        n_obs = int(gn.shape[0])
+        B = self.B = n_obs if source is None else int(source.size)
+        self.source, self.n_sources = source, (0 if source is None else n_obs)
         self.params = p = _params(divergence, kw, flux is not None)
         # a mixed batch: one bsgp_params per image, its own keywords merged over the call's (betaParam: see _row_betas)
         self.rows, self.is_beta, rows = None, None, [p]
@@ -350,10 +385,10 @@ class _Args:
                             r["flux"] is not None if "flux" in r else flux is not None) for r in per_image]
             self.rows = (_capi.Params * B)(*rows)
             self.is_beta = np.array([r.divergence == DIV_BETA for r in rows])
-        if not psf_is_set and plan.set_psf(psf_arg(psf)) not in (1, B):
-            raise ValueError("psf must be one image or one per batch entry")
+        if not psf_is_set and plan.set_psf(psf_arg(psf)) not in (1, n_obs):
+            raise ValueError("psf must be one image or one per batch entry" if source is None else "psf must be one image or one per observation")
         self.gn, self.bkg_img, self.trace = gn, int(_ndim(bkg) == 3), trace
-        self.bkg = image(bkg, "bkg") if self.bkg_img else vector(bkg, B, _NP[plan.dtype])
+        self.bkg = image(bkg, "bkg") if self.bkg_img else vector(bkg, n_obs, _NP[plan.dtype])
         self.flux = None if flux is None else vector(flux, B, np.float64)
         self.beta0 = vector(betaParam, B, np.float64)
         self.x0 = None if x0 is None else image(x0, "x0")
@@ -369,7 +404,7 @@ class _Args:
         structs hold raw addresses, so the order is kept here, with the other arrays, for as long as the arguments live."""
         self.order = order
         ci = _capi.Inputs(_ptr(self.gn), _ptr(self.bkg), self.bkg_img, _ptr(self.flux), _ptr(self.beta0), _ptr(self.x0),
-                          _ptr(self.obj), _ptr(order))
+                          _ptr(self.obj), _ptr(order), _ptr(self.source), self.n_sources)
         return ci, _capi.Outputs(_ptr(x), *(_ptr(a) for a in self.out.values()))
 
     def solve(self, plan, entry, ci, co, *stream):
@@ -388,7 +423,7 @@ class _Args:
 
 
 def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=None, obj=None, dtype="float64",
-                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, per_image=None, **kw):
+                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, per_image=None, source=None, **kw):
     """Restore a batch of independent images in one persistent kernel launch.
 
     gn [B,ny,nx]; psf [ny,nx] (shared) or [B,ny,nx]; bkg scalar, [B] or [B,ny,nx]; flux None or [B];
@@ -404,13 +439,22 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
     over the call's own: images with different keywords (KL and beta-SGP, stop rule, MAXIT, projection, saturation, ...)
     share one launch, and image i is exactly the solve of that image alone with its merged keywords.  The trace outputs
     are then [B, max MAXIT + 1]; entries past an image's own iteration count stay zero.  Keywords that describe the
-    operator (region, div_a, div_at, adjoint_second_psf) must be the same in every row."""
+    operator (region, div_a, div_at, adjoint_second_psf) must be the same in every row.
+
+    ``source``: shared observations.  A [B] integer array (host memory): solve i restores observation source[i], so
+    several solves of one image (a beta sweep, KL and beta-SGP runs of one sub-frame) carry its pixels and its PSF once.
+    gn is then [n_sources, ny, nx]; bkg a scalar, [n_sources] or [n_sources, ny, nx]; psf one image or [n_sources, ...];
+    x0 and obj [n_sources, ...].  flux, betaParam and per_image stay per solve, and the result has B entries, each
+    bit-identical to the same solve with its observation replicated (gn[source], ...)."""
     if divergence not in ("kl", "beta"):
         raise ValueError("divergence must be 'kl' or 'beta'")
+    if source is not None:
+        source = _source_map(source, gn, psf, bkg, flux, betaParam, x0, obj)
+    B = int(gn.shape[0]) if source is None else int(source.size)
     if per_image is not None:
-        _check_per_image(per_image, int(gn.shape[0]))
-        betaParam = _row_betas(betaParam, per_image, int(gn.shape[0]))
-        flux, per_image = _row_flux(flux, per_image, int(gn.shape[0]))
+        _check_per_image(per_image, B)
+        betaParam = _row_betas(betaParam, per_image, B)
+        flux, per_image = _row_flux(flux, per_image, B)
     if padded:
         if _is_tensor(gn) and not gn.is_cuda:             # CPU tensors (pinned or not) take the numpy route of the padded operator
             def host(a):
@@ -420,23 +464,25 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
         if per_image is not None and any(k in row for row in per_image for k in _OPERATOR_KEYS):
             raise ValueError("per_image rows of the padded operator share its geometry: region, div_a, div_at and "
                              "adjoint_second_psf are set by padded=True")
-        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, kw)
+        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source, kw)
     if x_out is not None and not (_is_tensor(gn) and not gn.is_cuda and gn.is_pinned()):
         raise ValueError("x_out is only supported with pinned CPU tensor inputs")
     if _is_tensor(gn) and not gn.is_cuda and gn.is_pinned():
         return _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image,
-                                   kw)
+                                   source, kw)
     if _is_tensor(gn) and gn.is_cuda:
-        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, kw)
+        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source, kw)
     if _is_tensor(gn):                                    # pageable CPU tensor: the plain host path
         gn = gn.numpy()
         psf, bkg, flux, betaParam, x0, obj = (a.numpy() if _is_tensor(a) and not a.is_cuda else a for a in (psf, bkg, flux, betaParam, x0, obj))
-    return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, kw)
+    return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, source,
+                             kw)
 
 
-def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, kw):
+def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source, kw):
     """Embed into the padded grid, solve there with the window mask, crop (see PaddedGeometry).  numpy inputs give
-    numpy outputs; CUDA-tensor images stay on the device (the small kernels may be numpy or tensors)."""
+    numpy outputs; CUDA-tensor images stay on the device (the small kernels may be numpy or tensors).  With a source map
+    the observations and their kernels are embedded once each."""
     on_dev = _is_tensor(gn)
     if on_dev:
         import torch
@@ -462,17 +508,17 @@ def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtyp
         if on_dev:
             big, bigt = torch.as_tensor(big, device=gn.device), torch.as_tensor(bigt, device=gn.device)
         if plan.set_psf(big) not in (1, B) or plan.set_psf_adjoint(bigt) not in (1, B):
-            raise ValueError("psf must be one kernel or one per batch entry")
+            raise ValueError("psf must be one kernel or one per batch entry" if source is None else "psf must be one kernel or one per observation")
         res = solve_batch(geo.embed(gn, dt), None, geo.embed(bkg, dt) if _ndim(bkg) == 3 else bkg, divergence=divergence,
                           flux=flux, betaParam=betaParam, x0=None if x0 is None else geo.embed(x0, dt),
                           obj=None if obj is None else geo.embed(obj, dt), dtype=dtype, device=device, trace=trace, plan=plan,
-                          psf_is_set=True, per_image=per_image, **extra, **kw)
+                          psf_is_set=True, per_image=per_image, source=source, **extra, **kw)
     x = res.x[:, geo.rows, geo.cols]
     res.x = x.contiguous() if on_dev else np.ascontiguousarray(x)
     return res
 
 
-def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, kw):
+def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, source, kw):
     """numpy arrays -> numpy arrays; one call of bsgp_solve_batch_host."""
     npdt = _NP[dtype]
     gn = np.ascontiguousarray(gn, dtype=npdt)
@@ -485,14 +531,14 @@ def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype,
         return a
 
     args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw,
-                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros, per_image=per_image)
-    x = np.empty(gn.shape, npdt)
+                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros, per_image=per_image, source=source)
+    x = np.empty((args.B,) + gn.shape[1:], npdt)
     ci, co = args.structs(x, _queue_order(divergence, args.beta0, args.is_beta))
     args.solve(plan, "_host", ci, co)
     return args.result(x)
 
 
-def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, kw):
+def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source, kw):
     """CUDA tensors -> CUDA tensors, asynchronous on the current stream: no host synchronisation, no host copies."""
     import torch
     if not gn.is_cuda:
@@ -524,8 +570,8 @@ def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trac
     with torch.cuda.device(dev):
         args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
                      image=image, vector=vector, alloc=lambda shape, dt: torch.zeros(shape, dtype=_torch_dtype(dt), device=dev),
-                     per_image=per_image)
-        x = torch.empty_like(gn)
+                     per_image=per_image, source=source)
+        x = torch.empty((args.B,) + tuple(gn.shape[1:]), dtype=gn.dtype, device=dev)
         order = None
         if args.is_beta is not None and args.is_beta.any() and args.B > 1:
             # mixed batch: beta-SGP images by |beta - 1|, then the KL images (see _queue_order)
@@ -542,7 +588,7 @@ def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trac
     return res
 
 
-def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image, kw):
+def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image, source, kw):
     """Page-locked CPU tensors -> page-locked CPU tensors; one call of bsgp_solve_batch_pinned (returns when the results
     are in host memory).  `device` selects the GPU.  Image-shaped arguments (bkg stack, x0, obj) must be pinned too."""
     import torch
@@ -565,13 +611,14 @@ def _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, devi
 
     with torch.cuda.device(plan.device):
         args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
-                     image=pinned, vector=_host_vector, alloc=hbuf, per_image=per_image)
+                     image=pinned, vector=_host_vector, alloc=hbuf, per_image=per_image, source=source)
+        xshape = (args.B,) + tuple(gn.shape[1:])
         if x_out is None:
-            x = torch.empty(tuple(gn.shape), dtype=gn.dtype, pin_memory=True)
+            x = torch.empty(xshape, dtype=gn.dtype, pin_memory=True)
         else:
             x = x_out
-            if not (_is_tensor(x) and not x.is_cuda and x.is_pinned() and x.dtype == gn.dtype and x.shape == gn.shape and x.is_contiguous()):
-                raise ValueError("x_out must be a contiguous pinned CPU tensor of the shape and dtype of gn")
+            if not (_is_tensor(x) and not x.is_cuda and x.is_pinned() and x.dtype == gn.dtype and tuple(x.shape) == xshape and x.is_contiguous()):
+                raise ValueError("x_out must be a contiguous pinned CPU tensor of the dtype of gn, one image per solve")
         ci, co = args.structs(x, _queue_order(divergence, args.beta0, args.is_beta))
         args.solve(plan, "_pinned", ci, co, _stream_ptr())
     res = args.result(x)

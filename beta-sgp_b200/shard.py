@@ -132,7 +132,7 @@ _FIELDS = ("x", "iters", "status", "discr", "times", "beta_final", "proj_evals",
 
 
 def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=None, divergence="beta", group=None, device=None,
-                        width="auto", timing=None, cost_rank=None, per_image=None, **kw):
+                        width="auto", timing=None, cost_rank=None, per_image=None, source=None, **kw):
     """Every rank passes the FULL batch and gets the full result back: rank r restores the images
     shard_indices(B, r, W, expected_cost_rank(...)) on its own GPU (engine.solve_batch, one persistent kernel launch) and
     the per-image results are all-gathered.  No data-path collective: the images are independent problems.
@@ -141,6 +141,8 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
     the device, asynchronously on the current stream; NCCL process group required when world_size > 1).
     psf: [ny,nx] shared or [B,ny,nx]; bkg: scalar, [B] or [B,ny,nx]; flux / betaParam: scalar or [B]; x0 / obj: [B,ny,nx].
     per_image: B keyword dicts of a mixed batch (engine.solve_batch); each rank receives the rows of its images.
+    source: [B] shared observations (engine.solve_batch): gn, psf, bkg, x0 and obj then hold one entry per observation, and
+    each rank receives only the observations its solves read, with the map renumbered to them; B is the number of solves.
     width: "auto" picks the CTA configuration from the local batch size (engine.auto_config), or (cluster_size, threads).
     cost_rank: optional precomputed expected_cost_rank(...) (a host array); give it when betaParam is a device tensor, so
     that the dealing does not have to copy betaParam back to the host (a synchronisation) on every call.
@@ -155,7 +157,10 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
     on_dev = engine._is_tensor(gn) and gn.is_cuda
     if device is None:
         device = (gn.device.index or 0) if on_dev else int(__import__("os").environ.get("LOCAL_RANK", rank))
-    B = int(gn.shape[0])
+    n_obs = int(gn.shape[0])
+    if source is not None:
+        source = engine._source_map(source, gn, psf, bkg, flux, betaParam, x0, obj)
+    B = n_obs if source is None else int(source.size)
     ny, nx = int(gn.shape[-2]), int(gn.shape[-1])
     if per_image is not None:
         engine._check_per_image(per_image, B)
@@ -168,6 +173,11 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
     cost_rank = np.ascontiguousarray(cost_rank)
     idx = shard_indices(B, rank, world, cost_rank)
     n_local = len(idx)
+    # the observations this rank's solves read (all of them are per solve without a map), and the map renumbered to them
+    obs_idx, local_source = idx, None
+    if source is not None:
+        obs_idx, local_source = np.unique(source[idx], return_inverse=True)
+        local_source = np.ascontiguousarray(local_source.reshape(-1), dtype=np.int32)
     use_cuda = on_dev or (is_dist and dist.get_backend(group) == "nccl")
     dev = torch.device("cuda", device) if use_cuda else torch.device("cpu")
     maxit = int(kw.get("MAXIT", 500))
@@ -175,26 +185,30 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
         maxit = max(int(row.get("MAXIT", maxit)) for row in per_image)     # the trace stride of the whole batch
 
     if on_dev:
-        skey = ("sel", B, rank, world, str(gn.device), cost_rank.tobytes())
+        skey = ("sel", B, rank, world, str(gn.device), cost_rank.tobytes(), None if source is None else source.tobytes())
         sel = _index_cache.get(skey)
         if sel is None:
-            sel = _index_cache[skey] = torch.as_tensor(idx, device=gn.device, dtype=torch.long)
+            sel = _index_cache[skey] = (torch.as_tensor(idx, device=gn.device, dtype=torch.long),
+                                        torch.as_tensor(obs_idx, device=gn.device, dtype=torch.long))
 
-        def take(a, per_image_ndim):
+        def take(a, per_image_ndim, obs=False):
+            """this rank's entries of a per-solve array, or with obs=True of a per-observation one"""
             if a is None:
                 return None
+            rows, n, t = (obs_idx, n_obs, sel[1]) if obs else (idx, B, sel[0])
             if engine._is_tensor(a):
-                return a.index_select(0, sel) if a.dim() == per_image_ndim + 1 and a.shape[0] == B else a
+                return a.index_select(0, t) if a.dim() == per_image_ndim + 1 and a.shape[0] == n else a
             a = np.asarray(a)
-            return a[idx] if a.ndim == per_image_ndim + 1 and a.shape[0] == B else a
+            return a[rows] if a.ndim == per_image_ndim + 1 and a.shape[0] == n else a
     else:
         gn = np.asarray(gn)
 
-        def take(a, per_image_ndim):
+        def take(a, per_image_ndim, obs=False):
             if a is None:
                 return None
+            rows, n = (obs_idx, n_obs) if obs else (idx, B)
             a = np.asarray(a)
-            return a[idx] if a.ndim == per_image_ndim + 1 and a.shape[0] == B else a
+            return a[rows] if a.ndim == per_image_ndim + 1 and a.shape[0] == n else a
 
     if n_local:
         dtype = "float32" if str(gn.dtype).endswith("float32") else "float64"
@@ -204,18 +218,20 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
             plan = engine.get_plan(ny, nx, dtype, device, cs, th)
         bk = bkg
         if engine._is_tensor(bkg):
-            bk = take(bkg, 2) if bkg.dim() == 3 else (take(bkg, 0) if bkg.dim() == 1 else bkg)
+            bk = take(bkg, 2, True) if bkg.dim() == 3 else (take(bkg, 0, True) if bkg.dim() == 1 else bkg)
         else:
             ba = np.asarray(bkg)
-            bk = ba[idx] if ba.ndim >= 1 and ba.shape[0] == B and ba.size > 1 else ba
+            bk = ba[obs_idx] if ba.ndim >= 1 and ba.shape[0] == n_obs and ba.size > 1 else ba
         ev = None
         if timing is not None and on_dev:
             ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-        args = (take(gn, 2), take(psf, 2), bk)
-        kwargs = dict(divergence=divergence, flux=take(flux, 0), betaParam=take(betaParam, 0), x0=take(x0, 2), obj=take(obj, 2),
+        args = (take(gn, 2, True), take(psf, 2, True), bk)
+        kwargs = dict(divergence=divergence, flux=take(flux, 0), betaParam=take(betaParam, 0), x0=take(x0, 2, True), obj=take(obj, 2, True),
                       device=device, plan=plan, dtype=dtype, **kw)
         if per_image is not None:
             kwargs["per_image"] = [per_image[int(i)] for i in idx]
+        if local_source is not None:
+            kwargs["source"] = local_source
         if ev:
             if plan is not None:
                 plan.set_psf(args[1])                      # PSF spectra outside the bracket: it times the solve kernel alone

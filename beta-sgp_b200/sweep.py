@@ -59,19 +59,17 @@ def sgp_betaDiv_sweep(gn, psf, bkg, flux=None, betas=None, measure=None, device=
     g = dev_t(gn)
     S, ny, nx = g.shape
     rep = lambda t: t.repeat_interleave(nb, dim=0)                      # noqa: E731  stamp-major: (s, k) -> s * nb + k
-    gb = rep(g)
+    source = np.repeat(np.arange(S, dtype=np.int32), nb)                # solve s * nb + k restores stamp s: one copy of each
     pt = dev_t(psf)
-    pb = rep(pt) if pt.dim() == 3 else pt
     bt = dev_t(bkg) if np.ndim(bkg) > 0 or type(bkg).__module__.startswith("torch") else torch.full((S,), float(bkg), dtype=torch.float64, device=dev)
     bt = bt.reshape(S) if bt.numel() == S else bt
-    bb = rep(bt)
     fb = None if flux is None else rep(dev_t(flux).reshape(S))
     b0 = torch.as_tensor(np.tile(betas, S), device=dev)
     kw.setdefault("proj_type", 1)
-    res = solve_batch(gb, pb, bb, divergence="beta", flux=fb, betaParam=b0, **kw)
+    res = solve_batch(g, pt, bt, divergence="beta", flux=fb, betaParam=b0, source=source, **kw)
     measure = measure or aperture_flux
-    orig = measure(gb, bb)
-    restored = measure(res.x, bb)
+    orig = rep(measure(g, bt))                                          # the original flux, measured once per stamp
+    restored = measure(res.x, rep(bt))
     metric = (1.0 - restored / orig).reshape(S, nb).cpu().numpy()          # flux_fractional_difference, :90
     best = select_best(metric)
     idx = torch.as_tensor(np.arange(S) * nb + best, device=dev)

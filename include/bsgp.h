@@ -99,6 +99,16 @@ typedef struct bsgp_inputs {
     const int* order;      /* [batch] permutation: the work queue hands out image order[0], order[1], ... (longest expected
                               solve first keeps the tail of the queue short); NULL = 0, 1, 2, ...  Results are always
                               stored at the image's own index. */
+    /* Shared observations: solve i reads observation source[i], so several solves of one image (a beta sweep, KL and
+     * beta-SGP runs of one sub-frame) need one copy of its pixels and one PSF spectrum.  source: [batch] in HOST memory
+     * on every entry point (read before the call returns), each entry in [0, n_sources), n_sources >= 1; NULL = the
+     * identity (n_sources ignored), which is the behaviour without this field.  With a map, everything that describes the
+     * observation is indexed by source: gn, bkg (stack or per-image scalar), x0, obj, and the PSF spectra, whose count
+     * must then be 1 or n_sources (bsgp_set_psf; the adjoint kernel the same).  Everything that describes the solve
+     * stays indexed by solve: flux, beta0, order, the rows of a mixed batch, and every output.  A bad index is
+     * BSGP_E_ARG naming the solve, before anything is launched. */
+    const int* source;
+    int n_sources;
 } bsgp_inputs;
 
 #define BSGP_NSCALARS 8    /* scaling, flux (scaled), X_low_bound, X_upp_bound, tol, fv_final, alpha_final, tau_final */
@@ -150,7 +160,8 @@ int bsgp_plan_get_info(const bsgp_plan* plan, bsgp_plan_info* info);
 int bsgp_plan_configure(bsgp_plan* plan, int cluster_size, int threads);
 
 /* TF = fftn(fftshift(psf)) for n_psf PSFs of the image shape (sgp.py:109 / 571); n_psf is 1 (shared by
- * the whole batch) or the batch size (one PSF per image). */
+ * the whole batch) or the batch size (one PSF per image).  A solve with a source map (bsgp_inputs.source) needs 1 or
+ * n_sources PSFs, one per observation: every solve of an observation uses its spectrum. */
 int bsgp_set_psf(bsgp_plan* plan, const void* psf_dev, int n_psf, void* stream);
 int bsgp_set_psf_host(bsgp_plan* plan, const void* psf_host, int n_psf);
 /* Second kernel for A^T (sgp.py:157: convolve_fft(x, psf.conj().T, ...)); same n_psf as bsgp_set_psf.  Power-of-two
