@@ -49,7 +49,8 @@ class Outputs(C.Structure):
                 ("times", C.c_void_p), ("stop_value", C.c_void_p), ("err", C.c_void_p), ("beta_final", C.c_void_p),
                 ("proj_evals", C.c_void_p), ("ls_trials", C.c_void_p), ("scalars", C.c_void_p),
                 ("trace_alpha", C.c_void_p), ("trace_lambda", C.c_void_p), ("trace_beta", C.c_void_p),
-                ("trace_trials", C.c_void_p), ("trace_evals", C.c_void_p)]
+                ("trace_trials", C.c_void_p), ("trace_evals", C.c_void_p),
+                ("snap_x", C.c_void_p), ("snap_every", C.c_int), ("snap_count", C.c_void_p)]
 
 
 class PlanInfo(C.Structure):

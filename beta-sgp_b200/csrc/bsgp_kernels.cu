@@ -685,7 +685,10 @@ static int solve_grid(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_in
     a.tr_beta = out->trace_beta; a.tr_trials = out->trace_trials; a.tr_evals = out->trace_evals;
     a.queue = p->queue;
     a.ready = p->frame ? nullptr : ready;
-    const RowArgs ra{kw.rows, kw.trace_stride, in->source};
+    // snapshots of a wrapped plan have the caller's image shape: the kernel stores the valid window (snap_crop)
+    const bool snap = out->snap_every > 0;
+    const RowArgs ra{kw.rows, kw.trace_stride, in->source, snap ? out->snap_x : nullptr, snap ? out->snap_count : nullptr,
+                     out->snap_every, snap ? snapshot_slots(kw.trace_stride, out->snap_every) : 0, p->embedded ? 1 : 0};
     const RowArgs* rows = kw.rows ? &ra : nullptr;                  // no rows: the kernels compiled without them
     if (p->frame) {
         LaunchCfg fc{p->g.G, 512, 1, p->smem_bytes, st, 1};
@@ -852,6 +855,7 @@ static int check_solve(const bsgp_plan* p, const bsgp_params* prm, const bsgp_pa
     int rc = check_batch_params(prm, rows, batch, in, out, &kw->trace_stride, err, sizeof err);
     if (rc) return fail(rc, "%s", err);
     if ((rc = check_sources(in, batch, err, sizeof err))) return fail(rc, "%s", err);
+    if ((rc = check_snapshots(out, err, sizeof err))) return fail(rc, "%s", err);
     if ((rc = check_psf_count(p->n_psf, in, batch, err, sizeof err))) return fail(rc, "%s", err);
     if (!in->gn || !in->bkg || !out->x || !out->iters || !out->status || !out->discr || !out->times) return fail(BSGP_E_ARG, "required pointer is NULL");
     if (p->n_psf < 1) return fail(BSGP_E_STATE, "bsgp_set_psf has not been called");
@@ -871,10 +875,11 @@ static int check_solve(const bsgp_plan* p, const bsgp_params* prm, const bsgp_pa
 
 // launch on device arrays that passed check_solve; `ready` (device, [batch]) makes the kernel wait for queue item i until ready[i] != 0.
 // The host rows of a mixed batch go up to the plan's row buffer on the launch's stream, behind the plan's previous launch,
-// and so does a source map.  A launch with a map runs the mixed-batch kernels: shared keywords become equal rows here.
-// `ready` is then indexed by observation.
+// and so does a source map.  A launch with a map or with snapshots runs the mixed-batch kernels: shared keywords become
+// equal rows here.  With a map, `ready` is indexed by observation.
 static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* stream, const int* ready) {
-    if (!p->embedded && (misaligned(in->gn) || misaligned(out->x) || misaligned(in->x0) || misaligned(in->obj) || (in->bkg_is_image && misaligned(in->bkg))))
+    if (!p->embedded && (misaligned(in->gn) || misaligned(out->x) || misaligned(in->x0) || misaligned(in->obj) || (in->bkg_is_image && misaligned(in->bkg)) ||
+                         (out->snap_every > 0 && misaligned(out->snap_x))))
         return fail(BSGP_E_ARG, "image pointers must be 16-byte aligned (vector loads)");
     CU(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -882,7 +887,7 @@ static int solve_launch(bsgp_plan* p, const Keywords& kw, int batch, const bsgp_
     if (rc) return rc;
     Keywords dk = kw;
     std::vector<bsgp_params> uniform;
-    if (in->source && !kw.rows) { uniform.assign((size_t)batch, *kw.prm); dk.rows = uniform.data(); }
+    if ((in->source || out->snap_every > 0) && !kw.rows) { uniform.assign((size_t)batch, *kw.prm); dk.rows = uniform.data(); }
     if (dk.rows) {
         const size_t bytes = (size_t)batch * sizeof(bsgp_params);
         if ((rc = grow((void**)&p->rows, &p->rows_cap, bytes, "the per-image keywords"))) return rc;
@@ -942,7 +947,7 @@ struct DevBuf {
 struct HostIO {
     enum Slot { GN, BKG, X0, OBJ, FLUX, BETA0, ORDER,                 // inputs, the image-shaped ones first
                 X, ITERS, STATUS, DISCR, TIMES, STOP_VALUE, ERR, BETA_FINAL, PROJ_EVALS, LS_TRIALS, SCALARS,
-                TRACE_ALPHA, TRACE_LAMBDA, TRACE_BETA, TRACE_TRIALS, TRACE_EVALS, NSLOT };
+                TRACE_ALPHA, TRACE_LAMBDA, TRACE_BETA, TRACE_TRIALS, TRACE_EVALS, SNAP_X, SNAP_COUNT, NSLOT };
     const void* host[NSLOT];              // nullptr: not staged
     size_t bytes[NSLOT], off[NSLOT];
     size_t out_begin = 0, size = 0;       // the outputs occupy [out_begin, size)
@@ -950,20 +955,24 @@ struct HostIO {
     int bkg_is_image;
     void* x_mapped;
     const int* source; int n_sources;     // the caller's map (host memory), passed on as it is
+    int snap_every;                       // snapshots: staged like the outputs, but filled from the caller's array first
 
     HostIO(const bsgp_plan* p, int trace_stride, int batch, const bsgp_inputs* in, const bsgp_outputs* out, void* x_mapped_)
         : img((size_t)p->img_ny * p->img_nx * p->elem), bkg_is_image(in->bkg_is_image), x_mapped(x_mapped_), source(in->source),
-          n_sources(in->n_sources) {
+          n_sources(in->n_sources), snap_every(out->snap_every) {
         const size_t B = (size_t)batch, tr = (size_t)trace_stride, imgs = B * img, it8 = B * tr * 8, it4 = B * tr * 4;
+        const bool snap = snap_every > 0;
+        const size_t snaps = snap ? B * (size_t)snapshot_slots(trace_stride, snap_every) * img : 0;
         const size_t O = (size_t)observation_count(in, batch), obs = O * img;
         const void* const h[NSLOT] = {in->gn, in->bkg, in->x0, in->obj, in->flux, in->beta0, in->order,
                                       x_mapped ? nullptr : out->x, out->iters, out->status, out->discr, out->times, out->stop_value,
                                       out->err, out->beta_final, out->proj_evals, out->ls_trials, out->scalars,
-                                      out->trace_alpha, out->trace_lambda, out->trace_beta, out->trace_trials, out->trace_evals};
+                                      out->trace_alpha, out->trace_lambda, out->trace_beta, out->trace_trials, out->trace_evals,
+                                      snap ? out->snap_x : nullptr, snap ? out->snap_count : nullptr};
         const size_t n[NSLOT] = {obs, bkg_is_image ? obs : O * p->elem, obs, obs, B * 8, B * 8, B * 4,
                                  imgs, B * 4, B * 4, it8, it8, it8,
                                  B * (tr + 1) * 8, B * 8, B * 4, B * 4, B * BSGP_NSCALARS * 8,
-                                 it8, it8, it8, it4, it4};
+                                 it8, it8, it8, it4, it4, snaps, B * 4};
         for (int k = 0; k < NSLOT; ++k) {
             if (k == X) out_begin = size;
             host[k] = h[k]; bytes[k] = n[k]; off[k] = size;
@@ -979,7 +988,8 @@ struct HostIO {
         const bsgp_outputs out = {x_mapped ? x_mapped : dev(X), (int*)dev(ITERS), (int*)dev(STATUS), (double*)dev(DISCR), (double*)dev(TIMES),
                                   (double*)dev(STOP_VALUE), (double*)dev(ERR), (double*)dev(BETA_FINAL), (int*)dev(PROJ_EVALS),
                                   (int*)dev(LS_TRIALS), (double*)dev(SCALARS), (double*)dev(TRACE_ALPHA), (double*)dev(TRACE_LAMBDA),
-                                  (double*)dev(TRACE_BETA), (int*)dev(TRACE_TRIALS), (int*)dev(TRACE_EVALS)};
+                                  (double*)dev(TRACE_BETA), (int*)dev(TRACE_TRIALS), (int*)dev(TRACE_EVALS), dev(SNAP_X), snap_every,
+                                  (int*)dev(SNAP_COUNT)};
         return solve_launch(p, kw, batch, &in, &out, stream, ready);
     }
     // the staged outputs to the caller's arrays, queued on `st`
@@ -1002,6 +1012,8 @@ static int solve_host(bsgp_plan* p, const bsgp_params* prm, const bsgp_params* r
     char* base = (char*)area.d;
     for (int k = 0; k < HostIO::X; ++k)
         if (io.host[k]) CU(cudaMemcpy(base + io.off[k], io.host[k], io.bytes[k], cudaMemcpyHostToDevice));
+    // slots a solve does not reach keep the caller's values
+    if (io.host[HostIO::SNAP_X]) CU(cudaMemcpy(base + io.off[HostIO::SNAP_X], io.host[HostIO::SNAP_X], io.bytes[HostIO::SNAP_X], cudaMemcpyHostToDevice));
     TRY(io.launch(p, kw, batch, base, nullptr, nullptr));
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess) return fail(BSGP_E_CUDA, "solve kernel failed: %s", cudaGetErrorString(e));
@@ -1036,6 +1048,7 @@ static int solve_pinned(bsgp_plan* p, const bsgp_params* prm, const bsgp_params*
     int rc;
     Keywords kw;
     TRY(check_solve(p, prm, rows, batch, in, out, true, &kw));
+    if (out->snap_every > 0) return fail(BSGP_E_ARG, "iterate snapshots (snap_every > 0) are not supported by bsgp_solve_batch_pinned; use the device or _host entry point");
     CU(cudaSetDevice(p->device));
     if (!page_locked(in->gn) || !page_locked(out->x) || !page_locked(in->x0) || !page_locked(in->obj) || (in->bkg_is_image && !page_locked(in->bkg)))
         return fail(BSGP_E_ARG, "bsgp_solve_batch_pinned needs page-locked image buffers (cudaHostAlloc / cudaHostRegister / torch pin_memory)");

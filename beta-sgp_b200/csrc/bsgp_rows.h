@@ -83,6 +83,23 @@ inline int check_sources(const bsgp_inputs* in, int batch, char* err, size_t err
 // The number of observations a batch reads: n_sources with a map, else one per image.
 inline int observation_count(const bsgp_inputs* in, int batch) { return in->source ? in->n_sources : batch; }
 
+// Iterate snapshots (bsgp_outputs.snap_x / snap_every / snap_count): an interval >= 0, and a destination when it is > 0.
+inline int check_snapshots(const bsgp_outputs* out, char* err, size_t errlen) {
+    if (out->snap_every < 0) {
+        snprintf(err, errlen, "snap_every must be >= 0 (got %d)", out->snap_every);
+        return BSGP_E_ARG;
+    }
+    if (out->snap_every > 0 && !out->snap_x) {
+        snprintf(err, errlen, "snap_every = %d needs outputs.snap_x", out->snap_every);
+        return BSGP_E_ARG;
+    }
+    return BSGP_OK;
+}
+
+// Snapshot slots per solve for a batch whose trace stride (check_batch_params) is the largest maxit + 1: the iterates
+// after 0, k, 2k, ... <= maxit passes.
+inline int snapshot_slots(int trace_stride, int snap_every) { return (trace_stride - 1) / snap_every + 1; }
+
 // PSF spectra set on the plan: one for all, or one per observation.
 inline int check_psf_count(int n_psf, const bsgp_inputs* in, int batch, char* err, size_t errlen) {
     if (n_psf == 1 || n_psf == observation_count(in, batch)) return BSGP_OK;

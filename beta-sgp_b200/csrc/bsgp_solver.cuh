@@ -71,7 +71,13 @@ template <typename T> struct SolveArgs {
 // runs kernels compiled exactly as before the feature existed.
 // source: [batch] (device) or NULL: the observation each solve reads (bsgp_inputs.source).  A launch with a map always runs
 // the ROWS kernels (the host expands shared keywords into equal rows), so the kernels without rows never see one.
-struct RowArgs { const bsgp_params* rows; int trace_stride; const int* source; };
+// snap: [batch][n_snap][..] (device) or NULL: iterate snapshots (bsgp_outputs.snap_x), every snap_every-th pass; a slot
+// holds the whole grid, or with snap_crop the valid window a.p.region (a wrapped plan: the caller's image shape).
+// snap_count: [batch] or NULL.  Like a source map, snapshots always run the ROWS kernels.
+struct RowArgs {
+    const bsgp_params* rows; int trace_stride; const int* source;
+    void* snap; int* snap_count; int snap_every, n_snap, snap_crop;
+};
 struct NoRow {};
 // the observation solve `img` reads: gn, bkg, x0, obj and the PSF spectra are indexed by it
 BSGP_DEV int source_of(int img) { return img; }
@@ -608,10 +614,32 @@ template <typename T, bool MK, int KIND, class Ctx> BSGP_NOINLINE R3 ph_trial_k(
     return r;
 }
 
+// Iterate snapshots (RowArgs::snap): the slot one phase stores x * scaling into, like ph_store_out.  crop: the slot holds
+// the valid window [reg0, reg1) x [reg2, reg3) row by row (masked kernels only), else the whole grid.
+template <typename T> struct SnapDst { T* dst; int crop; };
+struct NoSnap {};
+template <bool MK, typename T, class Ctx>
+BSGP_DEV void snap_store2(const Ctx& ctx, const ImgState<T>* S, const Region& R, const SnapDst<T>& sn, int i, V2<T> v) {
+    const T scaling = S->scaling;
+    const V2<T> o = mk2(nmul(v.x, scaling), nmul(v.y, scaling));
+    if constexpr (MK) {
+        if (sn.crop) {
+            const size_t w = (size_t)(R.c1 - R.c0);
+            const int row = R.row_off + (i >> R.lg_nx), col = i & R.colmask;      // i is even: both pixels share the row
+            if (inside<MK>(R, i)) sn.dst[(size_t)(row - R.r0) * w + (size_t)(col - R.c0)] = o.x;
+            if (inside<MK>(R, i + 1)) sn.dst[(size_t)(row - R.r0) * w + (size_t)(col + 1 - R.c0)] = o.y;
+            return;
+        }
+    }
+    st2(sn.dst + (size_t)ctx.rank * S->nslab, i, o);
+}
+template <bool MK, typename T, class Ctx> BSGP_DEV void snap_store2(const Ctx&, const ImgState<T>*, const Region&, const NoSnap&, int, V2<T>) {}
+
 // consumer of A^T(.): new gradient, y_k, Barzilai-Borwein sums, stop-rule / error sums   sgp.py:343-365, 394-402
 // The next iterate x + lam*d goes into the d array (d is dead after this pass); the controller swaps the x and d
-// pointers when the loop continues, so x keeps the previous iterate when it stops.
-template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, const ImgState<T>* S, T lam, int kind) {
+// pointers when the loop continues, so x keeps the previous iterate when it stops.  ph_ri_bb_snap (mixed-batch kernels,
+// on the passes that take a snapshot) also stores that iterate into the snapshot slot `sn`.
+template <typename T, bool MK, class Ctx, class Sn> BSGP_DEV R7 ri_bb_body(Ctx& ctx, const ImgState<T>* S, T lam, int kind, const Sn& sn) {
     const T* t1 = S->t1; T* gr = S->g; T* dbuf = S->d; const T* x = S->x; const T* truth = S->truth;
     const T xlo = S->xlo, xhi = S->xhi, scaling = S->scaling, div = S->div_at;
     const bool want_err = S->want_err != 0, stop2 = S->stop2 != 0;
@@ -648,12 +676,39 @@ template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, con
         gnew.y = one(inside<MK>(R, i + 1), in.a.y, in.b.y, in.c.y, in.d.y, in.e.y, w.y, xn.y);
         st2(gr, i, gnew);
         st2(dbuf, i, xn);
+        snap_store2<MK>(ctx, S, R, sn, i, xn);
     };
     conv_rows_inverse<1, MK>(ctx, S->geom, S->ws_off, S->twx, S->twx_off, S->tw_split, S->ppx_off, S->spec, cf, ca);
     R7 r;
 #pragma unroll
     for (int k = 0; k < 7; ++k) r.v[k] = bb[k];
     return r;
+}
+template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb(Ctx ctx, const ImgState<T>* S, T lam, int kind) {
+    return ri_bb_body<T, MK>(ctx, S, lam, kind, NoSnap{});
+}
+template <typename T, bool MK, class Ctx> BSGP_NOINLINE R7 ph_ri_bb_snap(Ctx ctx, const ImgState<T>* S, T lam, int kind, SnapDst<T> sn) {
+    return ri_bb_body<T, MK>(ctx, S, lam, kind, sn);
+}
+
+// snapshot slot 0: the start image after the initial projection (mixed-batch kernels only)
+template <typename T, bool MK, class Ctx> BSGP_NOINLINE void ph_store_snap(Ctx ctx, const ImgState<T>* S, SnapDst<T> sn) {
+    ctx.sync();
+    const T* x = S->x;
+    const Region R = region_of<MK>(ctx, S);
+    auto fetch = [&](int i) { In1<T> r; r.a = ld2(x, i); return r; };
+    auto body = [&](int i, const In1<T>& in) { snap_store2<MK>(ctx, S, R, sn, i, in.a); };
+    pair_loop<4>(ctx, S->nslab, fetch, body);
+}
+
+// where solve `img` keeps snapshot slot j (RowArgs::snap)
+template <typename T> BSGP_DEV SnapDst<T> snap_slot(const SolveArgs<T>& a, const RowArgs& ra, int img, int j) {
+    const int* r = a.p.region;
+    const size_t per = ra.snap_crop ? (size_t)(r[1] - r[0]) * (size_t)(r[3] - r[2]) : (size_t)a.g.ny * a.g.nx;
+    SnapDst<T> sn;
+    sn.dst = (T*)ra.snap + ((size_t)img * ra.n_snap + (size_t)j) * per;
+    sn.crop = ra.snap_crop;
+    return sn;
 }
 
 // x_out = x * scaling                                                        sgp.py:428
@@ -917,6 +972,9 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
             ph_proj_init_store<T, MK>(ctx, S, (T)pr.lambda);
         }
     }
+    if constexpr (ROWS) {
+        if (ra.snap) ph_store_snap<T, MK>(ctx, S, snap_slot(a, ra, img, 0));     // slot 0: what MAXIT = 1 returns
+    }
 
     W->truth_sq = 1.0;
     if (want_err && W->status == BSGP_ST_OK) {                          // :240-244, 255-257
@@ -1061,7 +1119,15 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         // ---- accept: x_tf, new gradient through A^T, BB sums (:337-347, 355-365, 402); the new x goes into the d array
         ph_rf_grad<T, MK>(ctx, S, W->dk.kind, (T)W->lam, 0);
         conv_middle<T, MK>(ctx, S, S->tf_at, mode_at);
-        R7 bbr = ph_ri_bb<T, MK>(ctx, S, (T)W->lam, W->dk.kind);
+        R7 bbr;
+        if constexpr (ROWS) {
+            // pass W->iter forms the iterate after that many passes: a snapshot on every snap_every-th
+            if (ra.snap && W->iter % ra.snap_every == 0)
+                bbr = ph_ri_bb_snap<T, MK>(ctx, S, (T)W->lam, W->dk.kind, snap_slot(a, ra, img, W->iter / ra.snap_every));
+            else bbr = ph_ri_bb<T, MK>(ctx, S, (T)W->lam, W->dk.kind);
+        } else {
+            bbr = ph_ri_bb<T, MK>(ctx, S, (T)W->lam, W->dk.kind);
+        }
         allreduce_fn<0, 7>(ctx, bbr.v);
 
         // ---- Barzilai-Borwein steps, lr schedule, bookkeeping and stop rules (:366-425)
@@ -1090,6 +1156,9 @@ BSGP_DEV void solve_image(Ctx& ctx, const SolveArgs<T>& a, ImgState<T>* S, T* co
         if (a.beta_final) a.beta_final[img] = W->beta_p;
         if (a.proj_evals) a.proj_evals[img] = W->total_evals;
         if (a.ls_trials) a.ls_trials[img] = W->total_trials;
+        if constexpr (ROWS) {
+            if (ra.snap && ra.snap_count) ra.snap_count[img] = 1 + (W->iter - 1) / ra.snap_every;   // W->iter - 1 passes made
+        }
         if (a.scalars) {
             double* sc = a.scalars + (size_t)img * BSGP_NSCALARS;
             sc[0] = (double)S->scaling; sc[1] = W->flux; sc[2] = W->x_low; sc[3] = W->x_upp; sc[4] = W->tol; sc[5] = W->fv; sc[6] = W->alpha; sc[7] = W->tau;

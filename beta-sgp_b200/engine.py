@@ -183,6 +183,8 @@ class BatchResult:
     ls_trials: object         # [B] total line-search evaluations
     scalars: object           # [B,8]
     trace: dict | None = None
+    snapshots: object = None       # [B,n_snap,ny,nx]: slot j is the iterate after j * snapshot_every passes (solve_batch)
+    snapshot_count: object = None  # [B] slots each solve wrote
 
 
 def _queue_order(divergence, beta0, is_beta=None):
@@ -372,7 +374,7 @@ class _Args:
     `vector(a, B, dtype)` (a scalar or [B] array as a contiguous [B] array of a numpy dtype) and `alloc(shape, dtype)`."""
 
     def __init__(self, gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, *, psf_arg, image,
-                 vector, alloc, per_image=None, source=None):
+                 vector, alloc, per_image=None, source=None, snapshot_every=0, snap_alloc=None):
         # B solves of n_obs observations: one each, or solve i of observation source[i] (_source_map)
         n_obs = int(gn.shape[0])
         B = self.B = n_obs if source is None else int(source.size)
@@ -398,6 +400,12 @@ class _Args:
         present = {None: True, "errflag": any(r.errflag for r in rows), "trace": bool(trace)}
         stride = max(r.maxit for r in rows) + 1                 # the library's trace stride (include/bsgp.h, bsgp_outputs)
         self.out = {f: alloc(shape(B, stride), dt) if present[when] else None for f, shape, dt, when in _OUTPUTS}
+        # iterate snapshots: n_snap slots per solve, NaN until the kernel writes them (include/bsgp.h, bsgp_outputs.snap_x)
+        self.snap_every = int(snapshot_every)
+        self.snapshots = self.snap_count = None
+        if self.snap_every:
+            self.snapshots = snap_alloc((B, snapshot_slots(stride - 1, self.snap_every)) + tuple(gn.shape[1:]))
+            self.snap_count = alloc((B,), np.int32)
 
     def structs(self, x, order):
         """_capi.Inputs / _capi.Outputs for restored images `x` and the work-queue order (None: natural order).  The
@@ -405,7 +413,8 @@ class _Args:
         self.order = order
         ci = _capi.Inputs(_ptr(self.gn), _ptr(self.bkg), self.bkg_img, _ptr(self.flux), _ptr(self.beta0), _ptr(self.x0),
                           _ptr(self.obj), _ptr(order), _ptr(self.source), self.n_sources)
-        return ci, _capi.Outputs(_ptr(x), *(_ptr(a) for a in self.out.values()))
+        return ci, _capi.Outputs(_ptr(x), *(_ptr(a) for a in self.out.values()), _ptr(self.snapshots), self.snap_every,
+                                 _ptr(self.snap_count))
 
     def solve(self, plan, entry, ci, co, *stream):
         """bsgp_solve_batch<entry> with the shared keywords, or its bsgp_solve_batch_rows<entry> twin for a mixed batch."""
@@ -419,11 +428,24 @@ class _Args:
     def result(self, x):
         out = dict(self.out)
         trace = {key: out.pop(f) for f, key in _TRACE_KEYS.items()}
-        return BatchResult(x=x, trace=trace if self.trace else None, **out)
+        return BatchResult(x=x, trace=trace if self.trace else None, snapshots=self.snapshots, snapshot_count=self.snap_count, **out)
+
+
+def snapshot_slots(maxit, every):
+    """Snapshot slots per solve: the iterates after 0, every, 2 * every, ... <= maxit passes (maxit: the largest MAXIT of
+    the batch)."""
+    return maxit // every + 1
+
+
+def _check_snapshot_every(k):
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 0:
+        raise ValueError(f"snapshot_every must be an integer >= 0 (0: no snapshots); got {k!r}")
+    return int(k)
 
 
 def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=None, obj=None, dtype="float64",
-                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, per_image=None, source=None, **kw):
+                device=0, trace=False, plan=None, psf_is_set=False, padded=False, x_out=None, per_image=None, source=None,
+                snapshot_every=0, **kw):
     """Restore a batch of independent images in one persistent kernel launch.
 
     gn [B,ny,nx]; psf [ny,nx] (shared) or [B,ny,nx]; bkg scalar, [B] or [B,ny,nx]; flux None or [B];
@@ -445,9 +467,21 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
     several solves of one image (a beta sweep, KL and beta-SGP runs of one sub-frame) carry its pixels and its PSF once.
     gn is then [n_sources, ny, nx]; bkg a scalar, [n_sources] or [n_sources, ny, nx]; psf one image or [n_sources, ...];
     x0 and obj [n_sources, ...].  flux, betaParam and per_image stay per solve, and the result has B entries, each
-    bit-identical to the same solve with its observation replicated (gn[source], ...)."""
+    bit-identical to the same solve with its observation replicated (gn[source], ...).
+
+    ``snapshot_every``: k >= 1 keeps every k-th iterate of each solve, stored by the kernel as it runs, so that picking
+    the iteration to keep (the restored image starts to amplify noise past some iteration) costs one launch.
+    ``BatchResult.snapshots`` is [B, n_snap, ny, nx] in the dtype of x (numpy or tensor like x), n_snap = max MAXIT // k
+    + 1.  Slot j belongs to iteration j * k: it is the image x of the same solve run with MAXIT = j * k + 1 (stop rule
+    1), bit for bit, and slot 0 is the start image after the initial projection.  ``BatchResult.snapshot_count`` [B]
+    says how many slots each solve wrote (1 + passes // k); the slots after them are NaN.  Memory: B * n_snap * ny * nx
+    values.  Not supported with pinned CPU tensors (ValueError)."""
     if divergence not in ("kl", "beta"):
         raise ValueError("divergence must be 'kl' or 'beta'")
+    snapshot_every = _check_snapshot_every(snapshot_every)
+    if snapshot_every and _is_tensor(gn) and not gn.is_cuda and gn.is_pinned() and not padded:
+        raise ValueError("snapshot_every is not supported with pinned CPU tensors (the pipelined host path); pass CUDA "
+                         "tensors or numpy arrays")
     if source is not None:
         source = _source_map(source, gn, psf, bkg, flux, betaParam, x0, obj)
     B = int(gn.shape[0]) if source is None else int(source.size)
@@ -464,22 +498,24 @@ def solve_batch(gn, psf, bkg, divergence="beta", flux=None, betaParam=1.005, x0=
         if per_image is not None and any(k in row for row in per_image for k in _OPERATOR_KEYS):
             raise ValueError("per_image rows of the padded operator share its geometry: region, div_a, div_at and "
                              "adjoint_second_psf are set by padded=True")
-        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source, kw)
+        return _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source,
+                                   snapshot_every, kw)
     if x_out is not None and not (_is_tensor(gn) and not gn.is_cuda and gn.is_pinned()):
         raise ValueError("x_out is only supported with pinned CPU tensor inputs")
     if _is_tensor(gn) and not gn.is_cuda and gn.is_pinned():
         return _solve_batch_pinned(gn, psf, bkg, divergence, flux, betaParam, x0, obj, device, trace, plan, psf_is_set, x_out, per_image,
                                    source, kw)
     if _is_tensor(gn) and gn.is_cuda:
-        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source, kw)
+        return _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source,
+                                   snapshot_every, kw)
     if _is_tensor(gn):                                    # pageable CPU tensor: the plain host path
         gn = gn.numpy()
         psf, bkg, flux, betaParam, x0, obj = (a.numpy() if _is_tensor(a) and not a.is_cuda else a for a in (psf, bkg, flux, betaParam, x0, obj))
     return _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, source,
-                             kw)
+                             snapshot_every, kw)
 
 
-def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source, kw):
+def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, per_image, source, snapshot_every, kw):
     """Embed into the padded grid, solve there with the window mask, crop (see PaddedGeometry).  numpy inputs give
     numpy outputs; CUDA-tensor images stay on the device (the small kernels may be numpy or tensors).  With a source map
     the observations and their kernels are embedded once each."""
@@ -512,13 +548,17 @@ def _solve_batch_padded(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtyp
         res = solve_batch(geo.embed(gn, dt), None, geo.embed(bkg, dt) if _ndim(bkg) == 3 else bkg, divergence=divergence,
                           flux=flux, betaParam=betaParam, x0=None if x0 is None else geo.embed(x0, dt),
                           obj=None if obj is None else geo.embed(obj, dt), dtype=dtype, device=device, trace=trace, plan=plan,
-                          psf_is_set=True, per_image=per_image, source=source, **extra, **kw)
+                          psf_is_set=True, per_image=per_image, source=source, snapshot_every=snapshot_every, **extra, **kw)
     x = res.x[:, geo.rows, geo.cols]
     res.x = x.contiguous() if on_dev else np.ascontiguousarray(x)
+    if res.snapshots is not None:                          # grid-sized like x: cropped the same way
+        sn = res.snapshots[..., geo.rows, geo.cols]
+        res.snapshots = sn.contiguous() if on_dev else np.ascontiguousarray(sn)
     return res
 
 
-def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, source, kw):
+def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype, device, trace, plan, psf_is_set, per_image, source,
+                      snapshot_every, kw):
     """numpy arrays -> numpy arrays; one call of bsgp_solve_batch_host."""
     npdt = _NP[dtype]
     gn = np.ascontiguousarray(gn, dtype=npdt)
@@ -531,14 +571,16 @@ def _solve_batch_host(gn, psf, bkg, divergence, flux, betaParam, x0, obj, dtype,
         return a
 
     args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw,
-                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros, per_image=per_image, source=source)
+                 psf_arg=lambda a: a, image=image, vector=_host_vector, alloc=np.zeros, per_image=per_image, source=source,
+                 snapshot_every=snapshot_every, snap_alloc=lambda shape: np.full(shape, np.nan, npdt))
     x = np.empty((args.B,) + gn.shape[1:], npdt)
     ci, co = args.structs(x, _queue_order(divergence, args.beta0, args.is_beta))
     args.solve(plan, "_host", ci, co)
     return args.result(x)
 
 
-def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source, kw):
+def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, per_image, source, snapshot_every,
+                        kw):
     """CUDA tensors -> CUDA tensors, asynchronous on the current stream: no host synchronisation, no host copies."""
     import torch
     if not gn.is_cuda:
@@ -570,7 +612,8 @@ def _solve_batch_device(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trac
     with torch.cuda.device(dev):
         args = _Args(gn, psf, bkg, divergence, flux, betaParam, x0, obj, trace, plan, psf_is_set, kw, psf_arg=psf_arg,
                      image=image, vector=vector, alloc=lambda shape, dt: torch.zeros(shape, dtype=_torch_dtype(dt), device=dev),
-                     per_image=per_image, source=source)
+                     per_image=per_image, source=source, snapshot_every=snapshot_every,
+                     snap_alloc=lambda shape: torch.full(shape, float("nan"), dtype=gn.dtype, device=dev))
         x = torch.empty((args.B,) + tuple(gn.shape[1:]), dtype=gn.dtype, device=dev)
         order = None
         if args.is_beta is not None and args.is_beta.any() and args.B > 1:

@@ -147,7 +147,10 @@ def solve_batch_sharded(gn, psf, bkg, flux=None, betaParam=1.005, x0=None, obj=N
     cost_rank: optional precomputed expected_cost_rank(...) (a host array); give it when betaParam is a device tensor, so
     that the dealing does not have to copy betaParam back to the host (a synchronisation) on every call.
     timing: optional dict; with CUDA tensors it receives timing["solve"] = (start, end) CUDA events around the local solve
-    (what bench.py divides the algorithmic bytes by) and timing["plan"] = the plan's info."""
+    (what bench.py divides the algorithmic bytes by) and timing["plan"] = the plan's info.
+    Iterate snapshots (engine.solve_batch(snapshot_every=...)) are not gathered across ranks: call engine.solve_batch."""
+    if "snapshot_every" in kw:
+        raise ValueError("solve_batch_sharded does not support snapshot_every; call solve_batch on one GPU")
     import torch
     import torch.distributed as dist
     from . import engine

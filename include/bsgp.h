@@ -134,6 +134,24 @@ typedef struct bsgp_outputs {
     double* trace_beta;
     int* trace_trials;
     int* trace_evals;
+    /* Iterate snapshots: every snap_every-th iterate of each solve, stored from inside the kernel, so that "which
+     * iteration to keep" needs one launch instead of one solve per candidate MAXIT.  snap_every = 0: none (the behaviour
+     * without these fields); < 0 is BSGP_E_ARG, and so is snap_every > 0 with snap_x NULL.
+     *   snap_x: [batch][n_snap][ny][nx] in the plan's dtype, n_snap = maxit / snap_every + 1 (a mixed batch: the largest
+     *           maxit of its rows, as for the traces).  Slot j holds the iterate after j * snap_every passes of the main
+     *           loop (sgp.py:302-425 / 748-882), un-scaled like x: slot 0 is the start image after the initial
+     *           projection.  A pass that stops the solve still stores the iterate it formed (the one the reference then
+     *           discards, x = prev_x) if its number is a multiple of snap_every.  So slot j is bit-identical to x of the
+     *           same solve run with MAXIT = j * snap_every + 1 and stop rule 1.  Slots past the last one a solve writes
+     *           are left as the caller allocated them.  The shape is the caller's image shape on every plan, including
+     *           plans whose grid differs from the image (sides that are not powers of two).
+     *   snap_count: [batch] or NULL: the number of slots each solve wrote, 1 + (passes made) / snap_every.
+     * A launch with snapshots runs the mixed-batch kernels (shared keywords become equal rows).  The device and _host
+     * entry points, plain and _rows, support them; bsgp_solve_batch_pinned and _rows_pinned refuse snap_every > 0 with
+     * BSGP_E_ARG.  Memory: batch * n_snap * ny * nx * sizeof(dtype) bytes. */
+    void* snap_x;
+    int snap_every;
+    int* snap_count;
 } bsgp_outputs;
 
 typedef struct bsgp_plan_info {
